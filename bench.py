@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the CSMPN hot path on B200: one EGCL layer forward+backward over a batch of synthetic complexes.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload md17|motion|nba|hulls]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload md17|motion|nba|hulls] [--dump-outputs DIR]
 
 Metric (BASELINE.json): simplices/sec fwd+bwd per CSMPN layer.  A step = one pass (forward + backward, all
 parameter and input gradients) of one shared simplicial message layer (EGCL) over one batch of 100 complexes.
@@ -29,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree, which may be read-only
 
 import numpy as np
 import torch
@@ -202,6 +203,11 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        try:  # reaped here: the sampler must not outlive the benchmark
+            self.proc.wait(timeout=5)
+        except subprocess.TimeoutExpired:
+            self.proc.kill()
+            self.proc.wait()
         sm, mx, reasons = [], None, set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for l in self.lines:
@@ -488,9 +494,29 @@ def _traffic_for_build():
         return None
 
 
+def dump_outputs(out_dir, per_simplex, whole, budget=64 << 20, seed=0):
+    """Write every array as <out_dir>/<name>.npy in float32.  If they exceed `budget` bytes in all, the per-simplex arrays
+    ([N, ...], same N) keep only a fixed, seeded sample of their rows -- the same rows in each -- so that two builds
+    run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu() for k, v in whole.items()}
+    rows = {k: v.detach().float().cpu() for k, v in per_simplex.items()}
+    n = next(iter(rows.values())).shape[0]
+    row_bytes = sum(v[0].numel() * 4 for v in rows.values())
+    headers = 256 * (len(arrays) + len(rows))  # an .npy header takes at most a few hundred bytes
+    keep = max(0, budget - headers - sum(v.numel() * 4 for v in arrays.values())) // max(row_bytes, 1)
+    if keep < n:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+        rows = {k: v[idx] for k, v in rows.items()}
+    arrays.update(rows)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.numpy())
+
+
 def layer_leg(workload, ncx, C, dev, world, rank, steps, warmup, lib, use_graph=True, with_e2e=True, with_roofline=True,
-              hbm_peak=6553.0, peak_src=""):
-    """One workload: the layer step with resident inputs (`value`), from host buffers (`e2e`), its kernel roofline."""
+              hbm_peak=6553.0, peak_src="", dump_dir=None):
+    """One workload: the layer step with resident inputs (`value`), from host buffers (`e2e`), its kernel roofline.
+    `dump_dir`: write what the last timed step returned (dump_outputs)."""
     import torch.distributed as dist
 
     from csmpn_b200.algebra.cliffordalgebra import CliffordAlgebra
@@ -519,16 +545,18 @@ def layer_leg(workload, ncx, C, dev, world, rank, steps, warmup, lib, use_graph=
     flat = torch.empty(n_par, device=dev)
 
     def step(h, graph_, node_attr, pack=True):
-        """one EAGER layer step (forward + backward through autograd); the graphed runs replay GraphedLayerStep instead"""
+        """one EAGER layer step (forward + backward through autograd); the graphed runs replay GraphedLayerStep instead.
+        Returns the layer output, grad_h and the parameter gradients (packed into `flat` when it was packed)."""
         hh = h.detach().requires_grad_()
         y = layer(hh, graph_, PairedNodeAttr(node_attr), node_attr)
         grads = torch.autograd.grad(y, [hh] + params, d["cot"])
-        if pack or world > 1:  # one flat gradient buffer: the all-reduce bucket / the D2H payload of the e2e leg
+        packed = pack or world > 1
+        if packed:  # one flat gradient buffer: the all-reduce bucket / the D2H payload of the e2e leg
             torch._foreach_copy_(list(flat.split([p.numel() for p in params])), [g.reshape(-1) for g in grads[1:]])
         if world > 1:
             dist.all_reduce(flat)
             flat.div_(world)
-        return y, grads[0]
+        return y, grads[0], flat if packed else grads[1:]
 
     # host-resident inputs (pinned) for the end-to-end leg
     # ONE pinned staging buffer holding h | edge_index | node_attr back to back: one H2D copy per step instead of three.
@@ -609,7 +637,7 @@ def layer_leg(workload, ncx, C, dev, world, rank, steps, warmup, lib, use_graph=
                     dist.all_reduce(gflat)
                     gflat.div_(world)
             else:
-                y, gh = step(x["h"], CSRGraph(ei_dev[k], N), na_dev[k])
+                y, gh, _ = step(x["h"], CSRGraph(ei_dev[k], N), na_dev[k])
                 gflat = flat
             feeder.drain(y, y_host)
             if d2h_grad_h:
@@ -638,14 +666,18 @@ def layer_leg(workload, ncx, C, dev, world, rank, steps, warmup, lib, use_graph=
         gstep = GraphedLayerStep(layer, d["edge_index"], d["h"], d["node_attr"], d["cot"], pack=world > 1)
 
     def resident_step():
+        """one step; returns the layer output, grad_h and the parameter gradients (one flat tensor or one per parameter)"""
         if gstep is None:
             return step(d["h"], graph, d["node_attr"], pack=False)
-        _, _, gflat = gstep()
+        y, gh, gflat = gstep()
         if world > 1:
             dist.all_reduce(gflat)
             gflat.div_(world)
+            return y, gh, gflat
+        return y, gh, gstep.param_grads
 
     def timed(steps, warmup):
+        """(summed ms of `steps` timed steps, the outputs of the last one; None unless they are dumped)"""
         for _ in range(warmup):
             resident_step()
         torch.cuda.synchronize()
@@ -657,16 +689,18 @@ def layer_leg(workload, ncx, C, dev, world, rank, steps, warmup, lib, use_graph=
             flush.fill_(1.0)  # L2 flush (256 MiB > 126 MB L2), outside the timed events
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            resident_step()
+            last = resident_step()
             e1.record()
             evs.append((e0, e1))
+            if dump_dir is None:
+                last = None
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
         t = torch.tensor([sum(a.elapsed_time(bb) for a, bb in evs)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item())
+        return float(t.item()), last
 
     if use_graph:
         glayer = gstep  # (flag for the host-fed leg below: graphed)
@@ -692,7 +726,13 @@ def layer_leg(workload, ncx, C, dev, world, rank, steps, warmup, lib, use_graph=
         res["e2e_regions_ms_per_step"] = [r / steps for r in regions]
         res["e2e_host_enqueue_ms_per_step"] = timed_e2e.host_ms_per_step
         res["h2d_bytes_per_step"], res["d2h_bytes_per_step"] = h2d_bytes, d2h_bytes
-    total_ms = timed(steps, warmup)
+    total_ms, last = timed(steps, warmup)
+    if dump_dir is not None:
+        y, gh, pgrads = last
+        if torch.is_tensor(pgrads):
+            pgrads = pgrads.split([p.numel() for p in params])
+        names = [n for n, _ in layer.named_parameters()]
+        dump_outputs(dump_dir, {"y": y, "grad_h": gh}, {f"grad.{n}": g.reshape(p.shape) for n, g, p in zip(names, pgrads, params)})
     res["ms_per_step"] = total_ms / steps
     nt = torch.tensor([N], device=dev, dtype=torch.float64)
     if world > 1:
@@ -787,7 +827,8 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     main = layer_leg(args.workload, ncx, C, dev, world, rank, args.steps, args.warmup, lib, use_graph=not args.no_graph,
-                     with_e2e=not args.no_e2e, with_roofline=not args.no_roofline, hbm_peak=hbm_peak, peak_src=peak_src)
+                     with_e2e=not args.no_e2e, with_roofline=not args.no_roofline, hbm_peak=hbm_peak, peak_src=peak_src,
+                     dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None  # sampled over the e2e and layer-step timed regions of the headline workload
     _release_cached(dev)
     others = {}
@@ -864,7 +905,14 @@ def main():
     ap.add_argument("--no-roofline", action="store_true", help="skip the per-kernel timing table")
     ap.add_argument("--train-only", action="store_true", help="only the full-model train-step leg")
     ap.add_argument("--only", action="store_true", help="only the named workload's layer legs (no motion/NBA side runs, no lifting leg)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (layer output, grad_h, every parameter gradient) "
+                         "as DIR/<name>.npy, float32, at most 64 MB in all (a fixed, seeded sample of rows beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.train_only):
+        ap.error("--dump-outputs writes what the layer step of --impl ours computed (not with --train-only)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -351,36 +351,27 @@ def test_equivariance_with_correct_inverse():
 
 def test_versor_utilities_match_the_reference():
     """the off-path helpers of CliffordAlgebra (alpha_w, inverse, rho, sandwich, output_blades, parity, eta,
-    reduce_geometric_product, random_vector / versor shapes) against the reference's own class on the same inputs
-    (oracle/_ref, CPU).  Skipped where the reference copy is absent."""
-    from oracle import refshim
-
-    if not refshim.reference_available():
-        pytest.skip("no copy of the reference (oracle/_ref)")
-    refshim.install()
-    from csmpn.algebra.cliffordalgebra import CliffordAlgebra as RefAlgebra
-
+    reduce_geometric_product, random_vector / versor shapes) against the reference's definitions on the same inputs
+    (tests/golden/versor.pt, made by tests/golden/make_golden_versor.py)."""
     CliffordAlgebra, _ = _mods()
-    gen = torch.Generator().manual_seed(11)
+    gold = load_golden("versor.pt")
     for metric in ((1, 1), (1, 1, 1)):
-        ref = RefAlgebra(metric)
+        ref = gold[metric]
         alg = CliffordAlgebra(metric).to(DEV)
         Bn = 2 ** len(metric)
-        mv = torch.randn(5, Bn, generator=gen)
-        vec = torch.zeros(1, Bn); vec[0, 1:1 + len(metric)] = torch.randn(len(metric), generator=gen)          # odd element
-        rot = ref.geometric_product(vec, torch.roll(vec, 1, dims=1) * (ref.bbo_grades == 1))                         # even element
-        for w in (vec, rot):
-            assert bool(alg.parity(w.to(DEV))) == bool(ref.parity(w)) and int(alg.eta(w.to(DEV))) == int(ref.eta(w))
-            assert_close(alg.alpha_w(w.to(DEV), mv.to(DEV)), ref.alpha_w(w, mv), 1e-6, "alpha_w")
-            assert_close(alg.inverse(w.to(DEV)), ref.inverse(w), 1e-5, "inverse")
-            assert_close(alg.rho(w.to(DEV), mv.to(DEV)), ref.rho(w, mv), 1e-5, "rho")
-        assert_close(alg.sandwich(mv.to(DEV), vec.to(DEV), mv.to(DEV)), ref.sandwich(mv, vec, mv), 1e-5, "sandwich")
+        mv, vec, rot = ref["mv"], ref["vec"], ref["rot"]   # rot: an even element, vec: an odd one
+        for w, r in zip((vec, rot), ref["elements"]):
+            assert bool(alg.parity(w.to(DEV))) == r["parity"] and int(alg.eta(w.to(DEV))) == r["eta"]
+            assert_close(alg.alpha_w(w.to(DEV), mv.to(DEV)), r["alpha_w"], 1e-6, "alpha_w")
+            assert_close(alg.inverse(w.to(DEV)), r["inverse"], 1e-5, "inverse")
+            assert_close(alg.rho(w.to(DEV), mv.to(DEV)), r["rho"], 1e-5, "rho")
+        assert_close(alg.sandwich(mv.to(DEV), vec.to(DEV), mv.to(DEV)), ref["sandwich"], 1e-5, "sandwich")
         with pytest.raises(ValueError):
             alg.parity((vec + rot).to(DEV))
-        left, right = [1, 2], list(range(Bn))
-        assert torch.equal(alg.output_blades(left, right), ref.output_blades(left, right))
-        chain = [torch.randn(3, Bn, generator=gen) for _ in range(3)]
-        assert_close(alg.reduce_geometric_product([c.to(DEV) for c in chain]), ref.reduce_geometric_product(chain), 1e-5, "reduce")
+        ob = ref["output_blades"]
+        assert torch.equal(alg.output_blades(ob["left"], ob["right"]), ob["blades"])
+        chain = ref["chain"]
+        assert_close(alg.reduce_geometric_product([c.to(DEV) for c in chain]), ref["reduce_geometric_product"], 1e-5, "reduce")
         rv = alg.random_vector(4)
         assert rv.shape == (4, Bn) and bool((rv[:, alg.bbo_grades.to(rv.device) != 1] == 0).all())
         v = alg.versor()

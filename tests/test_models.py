@@ -124,7 +124,9 @@ def test_md17_model_at_benched_size_matches_reference():
     """The md17 model at the size `bench.py`'s train leg runs (100 complexes: ~8.6 k simplices, ~52 k pairs, so the layers'
     per-pair blocks run on the tensor-core engine with 3 tiles per persistent CTA) against the UNMODIFIED reference
     model's loss and parameter gradients (tests/golden/md17_bench.pt, made by tests/golden/make_golden_md17_bench.py).
-    The batch is regenerated from the seed and lifted on the GPU; checksums tie it to the one the reference saw."""
+    The batch is regenerated from the seed and lifted on the GPU, the parameters from the seed of the reference's
+    initialisation; checksums tie both to what the reference saw.  The gradients are compared on a fixed sample of their
+    entries, against the largest magnitude of the whole reference gradient (the scale of rel_err)."""
     import hashlib
     import os
     import sys
@@ -144,9 +146,14 @@ def test_md17_model_at_benched_size_matches_reference():
     sha = lambda t: hashlib.sha256(t.contiguous().cpu().numpy().tobytes()).hexdigest()
     assert sha(batch.edge_index) == fx["edge_index_sha256"] and sha(batch.x_ind) == fx["x_ind_sha256"]
     assert int(batch.edge_index.shape[1]) == fx["n_pairs"] >= 8192
-    m = model_class("md17")().to(dev)
-    missing, unexpected = m.load_state_dict(fx["state_dict"], strict=False)
-    assert not unexpected and all("algebra" in k for k in missing), (missing, unexpected)
+    torch.manual_seed(fx["init_seed"])
+    m = model_class("md17")()
+    sd = hashlib.sha256()
+    for k, v in m.state_dict().items():
+        if "algebra" not in k:
+            sd.update(k.encode() + b"\0" + v.contiguous().numpy().tobytes())
+    assert sd.hexdigest() == fx["state_dict_sha256"], "the seeded initialisation no longer gives the reference's parameters"
+    m = m.to(dev)
     n0 = _lib.lib().csmpn_launch_count()
     loss, out = m(batch, 0, "train")
     named = list(m.named_parameters())
@@ -160,7 +167,14 @@ def test_md17_model_at_benched_size_matches_reference():
         if ref is None:
             assert gr is None or float(gr.abs().max()) == 0.0, n
             continue
-        assert_close(gr, ref, GRAD_TOL, f"md17@100 grad {n}")
+        assert gr is not None and tuple(gr.shape) == ref["shape"], n
+        flat = gr.detach().double().cpu().reshape(-1)
+        scale = ref["absmax"] + 1e-30
+        e = float((flat[ref["index"].long()] - ref["value"].double()).abs().max()) / scale
+        assert e <= GRAD_TOL, f"md17@100 grad {n}: rel err {e:.3e} > {GRAD_TOL:.1e}"
+        # the largest magnitude of the whole gradient: within the same bound if every entry is
+        e = abs(float(flat.abs().max()) - ref["absmax"]) / scale
+        assert e <= GRAD_TOL, f"md17@100 grad {n}: max |g| rel err {e:.3e} > {GRAD_TOL:.1e}"
 
 
 @pytest.mark.gpu
