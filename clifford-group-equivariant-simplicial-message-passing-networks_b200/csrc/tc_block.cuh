@@ -241,6 +241,44 @@ struct Pipe {
   }
 };
 
+// ---- overlapped epilogue (tc_f1db_kernel, tc_bgemmdb_kernel) ---------------------------------------------------------
+// Accumulators alternate between two TMEM buffers by tile.  The epilogue of tile t-1 stays pending on each epilogue warp
+// (warps 4-15: lane quadrant warp & 3, channel groups (warp >> 2) - 1, + 3, ...) while the K loop of tile t runs; the
+// warp runs one channel-group unit of it, unit(tile, c4, tb), between two of its chunks.
+struct PendingEpilogue {
+  int64_t tile = -1;  // nothing pending
+  int c4 = 0;         // next channel group
+  int q = 0;          // last chunk of the pending tile
+  uint32_t tb = 0;    // its accumulator buffer
+  bool ready = false;
+  // after the K loop of `t` (last chunk last_q, accumulators at buf); warps 0-3 never run the epilogue
+  __device__ __forceinline__ void start(int warp, int64_t t, int last_q, uint32_t buf) {
+    if (warp >= 4) { tile = t; c4 = (warp >> 2) - 1; q = last_q; tb = buf; ready = false; }
+  }
+  // at most one unit
+  template <class Unit>
+  __device__ __forceinline__ void step(const Pipe& p, int n_c4, Unit&& unit) {
+    if (tile < 0) return;
+    if (!ready) {  // the MMAs of the pending tile have completed (its last chunk released its slot)
+      mbar_wait(&p.slot_bar[q % kRing], (q / kRing) & 1);
+      fence_after_sync();
+      ready = true;
+    }
+    if (c4 < n_c4) {
+      unit(tile, c4, tb);
+      c4 += 3;
+    }
+    if (c4 >= n_c4) { tile = -1; fence_before_sync(); }
+  }
+  // Called at the end of each K loop: the previous tile's epilogue must be finished before this warp signals the next
+  // tile's first chunk (conv_done).  The issuer waits for that full_bar before the first MMA of the next tile, which
+  // overwrites the buffer this epilogue reads.
+  template <class Unit>
+  __device__ __forceinline__ void drain(const Pipe& p, int n_c4, Unit&& unit) {
+    while (tile >= 0) step(p, n_c4, unit);
+  }
+};
+
 // ---- streamed weights (wide blocks) --------------------------------------------------------------------------------
 // When the weight images of a GEMM do not fit shared memory next to the chunk ring (Cl(3,0) with C >= 64), the weights
 // are streamed WITH the activations: a raw slot holds the activation chunk followed by the "weight unit" of the same K

@@ -355,6 +355,8 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b3_kernel(EwArgs 
 
 // =====================================================================================================================
 // transposed-weight GEMM:  out[r, n] = addend[r, n] + sum_s sum_k src_s[r, k] * W_s[k, n]     (W_s global [K_s, N_s, G])
+// The kernels index src / cp / w / wk with runtime values, so they take the arguments as __grid_constant__: without it
+// nvcc copies the whole struct to a local-memory stack frame first.
 struct GemmArgs {
   int64_t rows;
   int tiles;
@@ -367,42 +369,52 @@ struct GemmArgs {
   const float* addend;  // BPT [n16] or NULL
   float* out;
   int out_bpt;          // 1: BPT [n16]; 0: reference layout [rows, wn, B]
-  // SILU epilogue (the MVSiLU adjoint folded into the dy2 GEMM, so dy2 never leaves the SM): out = dy1
-  const float *y1, *sa, *sb;  // pre-activation (BPT [n16]), gate parameters [C, G]
-  float* partial;             // [grid][C][2G + 1] per-CTA partials of the gradients of sa, sb, b1
-  int C;
   // streamed-weights mode (wide blocks): pre-split images in global memory, np = output channels per pass
   const float* wimg;
   int np;
 };
 
-// Sum n <= 16 register values over the 32 lanes of a warp with n shuffles (instead of 5 n): in round `step` a lane keeps
-// the half of the values selected by its lane bit and receives the partner's copy of the same half.  Afterwards lane l
-// holds the warp total of value (l & 15), in v[0].
-__device__ __forceinline__ float warp_transpose_reduce16(float (&v)[16], int lane) {
+// Store channel group gc4 of row r of `tile` to a.out: BPT (rows past the end as zeros) or the reference layout, one
+// 32-byte store per (row, channel) when B == 8 and the output is 32-byte aligned (wide_ok).
+template <int DIM>
+__device__ __forceinline__ void store_gemm_group(const GemmArgs& a, const float (&v)[Alg<DIM>::B][4], int64_t tile, int gc4, int r,
+                                                 bool wide_ok) {
+  constexpr int B = Alg<DIM>::B;
+  const int64_t row0 = tile * kTile;
+  const bool row_ok = row0 + r < a.rows;
+  if (a.out_bpt) {
 #pragma unroll
-  for (int step = 8; step >= 1; step >>= 1) {
-    const bool up = (lane & step) != 0;
+    for (int b = 0; b < B; ++b) {
+      float4 x = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
+      if (!row_ok) x = make_float4(0.f, 0.f, 0.f, 0.f);
+      *reinterpret_cast<float4*>(a.out + bpt_off(B, a.n16, tile, b, gc4, r)) = x;
+    }
+  } else if (row_ok) {
 #pragma unroll
-    for (int i = 0; i < step; ++i) {
-      const float send = up ? v[i] : v[i + step];
-      const float keep = up ? v[i + step] : v[i];
-      v[i] = keep + __shfl_xor_sync(0xffffffffu, send, step);
+    for (int jj = 0; jj < 4; ++jj) {
+      const int n = gc4 * 4 + jj;
+      if (n >= a.wn) continue;
+      float* dst = a.out + ((size_t)(row0 + r) * a.wn + n) * B;
+      if constexpr (B == 8) {
+        if (wide_ok) {
+          float w8[8];
+#pragma unroll
+          for (int b = 0; b < 8; ++b) w8[b] = v[b][jj];
+          st_global_v8(dst, w8);
+          continue;
+        }
+      }
+#pragma unroll
+      for (int h = 0; h < B / 4; ++h)
+        *reinterpret_cast<float4*>(dst + 4 * h) = make_float4(v[4 * h][jj], v[4 * h + 1][jj], v[4 * h + 2][jj], v[4 * h + 3][jj]);
     }
   }
-  return v[0] + __shfl_xor_sync(0xffffffffu, v[0], 16);
-}
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
 }
 
-template <int DIM, bool SILU, bool ST>
-__global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
+template <int DIM, bool ST>
+__global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_constant__ GemmArgs a) {
   using A = Alg<DIM>;
-  constexpr int B = A::B, G = A::G, NPS = 2 * G + 1;  // NPS: per-channel SiLU parameter gradients (sa[G], sb[G], b1)
-  static_assert(2 * NPS <= 18, "two channels' SiLU gradients are reduced as 16 + 2 values");
+  constexpr int B = A::B, G = A::G;
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int nmax = ST ? a.np : (512 / B) / 16 * 16;            // output channels per pass (TMEM columns / blades)
@@ -414,25 +426,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
   const int nsets = a.src[1] ? 2 : 1;
   uint64_t* bars = reinterpret_cast<uint64_t*>(wimg + (size_t)nsets * set_bytes);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kPipeBars);
-  float* sa_s = reinterpret_cast<float*>(tmem_slot + 4);  // SILU: [n16][G] gate parameters
-  float* sb_s = sa_s + a.n16 * G;
   Pipe p;
   p.init(smem, bars, half);
-  if (SILU) {
-    for (int i = tid; i < a.n16 * G; i += kThreads) {
-      sa_s[i] = (i < a.C * G) ? a.sa[i] : 0.f;
-      sb_s[i] = (i < a.C * G) ? a.sb[i] : 0.f;
-    }
-  }
-  // SILU: per-lane accumulators of the parameter gradients of this warp's channel groups (iteration it of the epilogue
-  // loop = channel group (warp >> 2) + 4 it; two channel pairs per group): lane l holds value (l & 15) of the pair's 18
-  // values (index = 9 * (channel & 1) + k) for l < 16, lanes 16 and 17 hold values 16 and 17
-  float acc[4][2];
-#pragma unroll
-  for (int it = 0; it < 4; ++it) {
-#pragma unroll
-    for (int pr = 0; pr < 2; ++pr) acc[it][pr] = 0.f;
-  }
   const int npass = (a.n16 + nmax - 1) / nmax;
   const int nk = a.nk[0] + a.nk[1];
   const int per_tile = npass * nk;
@@ -455,10 +450,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
   const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   if (!ST) {
-    {
     const WJob wj[2] = {{wimg, a.w[0], a.wk[0], a.wn, 0}, {wimg + set_bytes, a.w[nsets - 1], a.wk[nsets - 1], a.wn, 0}};
     stage_weight_jobs<DIM, true, 2>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
-  }
   }
   fence_async_smem();
   fence_before_sync();
@@ -469,7 +462,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
   const bool wide_ok = aligned32(a.out);
   for (int t = 0; t < my_tiles; ++t) {
     const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
-    const int64_t row0 = tile * kTile;
     for (int ps = 0; ps < npass; ++ps) {
       const int n0 = ps * nmax;
       const int Np = (a.n16 - n0) < nmax ? (a.n16 - n0) : nmax;
@@ -497,7 +489,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
       // ---- epilogue of this pass: output channels [n0, n0 + Np).  The addend rows of the first channel group are
       // requested before waiting for the MMAs, those of the next group while the current one is processed.
       const int r = lane_base + lane;
-      const bool row_ok = row0 + r < a.rows;
       float4 ad[B];
       if (a.addend && (warp >> 2) < (Np >> 2)) {
 #pragma unroll
@@ -522,94 +513,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
             for (int b = 0; b < B; ++b) ad[b] = *reinterpret_cast<const float4*>(a.addend + bpt_off(B, a.n16, tile, b, gc4 + 4, r));
           }
         }
-        if constexpr (SILU) {
-          // MVSiLU adjoint on the dy2 values in registers (cegnn_utils.py:73-83): dy1 replaces dy2 in v; the gate
-          // parameter gradients are summed over the warp's 32 rows here and over tiles / lane quadrants at the end
-          const int it = c4 >> 2;  // (c4 - (warp >> 2)) / 4
-#pragma unroll
-          for (int pr = 0; pr < 2; ++pr) {
-            float2 y1v[B];  // the two channels of this pair (8-byte loads: half the live registers of a float4 per blade)
-#pragma unroll
-            for (int b = 0; b < B; ++b)
-              y1v[b] = *reinterpret_cast<const float2*>(a.y1 + bpt_off(B, a.n16, tile, b, gc4, r) + 2 * pr);
-            float vals[16], t0 = 0.f, t1 = 0.f;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) vals[i] = 0.f;
-#pragma unroll
-            for (int jj = 0; jj < 2; ++jj) {
-              const int j = 2 * pr + jj, ch = gc4 * 4 + j;
-              float y1[B], dy[B], sg[G], inv[G], tg[G], ds[G];
-#pragma unroll
-              for (int b = 0; b < B; ++b) {
-                y1[b] = jj == 0 ? y1v[b].x : y1v[b].y;
-                dy[b] = v[b][j];
-              }
-              const float* sa = sa_s + ch * G;
-              silu_gates<DIM>(y1, sa, sb_s + ch * G, sg, inv);
-#pragma unroll
-              for (int g = 0; g < G; ++g) tg[g] = 0.f;
-#pragma unroll
-              for (int b = 0; b < B; ++b) tg[A::grade_of(b)] = fmaf(dy[b], y1[b], tg[A::grade_of(b)]);
-              const bool ok = row_ok && ch < a.C;
-              float gv[NPS];
-#pragma unroll
-              for (int g = 0; g < G; ++g) {
-                ds[g] = ok ? tg[g] * sg[g] * (1.f - sg[g]) : 0.f;
-                gv[g] = ds[g] * inv[g];
-                gv[G + g] = ds[g];
-              }
-#pragma unroll
-              for (int b = 0; b < B; ++b) {
-                const int g = A::grade_of(b);
-                const float dinv = (g == 0) ? 1.f : 2.f * y1[b];
-                v[b][j] = ok ? fmaf(sg[g], dy[b], ds[g] * sa[g] * dinv) : 0.f;
-              }
-              gv[2 * G] = v[0][j];
-#pragma unroll
-              for (int k = 0; k < NPS; ++k) {
-                const int idx = jj * NPS + k;  // compile-time after unrolling
-                if (idx < 16) vals[idx] = gv[k];
-                else if (idx == 16) t0 = gv[k];
-                else t1 = gv[k];
-              }
-            }
-            const float s16 = warp_transpose_reduce16(vals, lane);
-            t0 = warp_sum(t0);
-            t1 = warp_sum(t1);
-            const float mine = lane < 16 ? s16 : lane == 16 ? t0 : lane == 17 ? t1 : 0.f;
-#pragma unroll
-            for (int q4 = 0; q4 < 4; ++q4) {
-              if (q4 == it) acc[q4][pr] += mine;
-            }
-          }
-        }
-        if (a.out_bpt) {
-#pragma unroll
-          for (int b = 0; b < B; ++b) {
-            float4 x = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
-            if (!row_ok) x = make_float4(0.f, 0.f, 0.f, 0.f);
-            *reinterpret_cast<float4*>(a.out + bpt_off(B, a.n16, tile, b, gc4, r)) = x;
-          }
-        } else if (row_ok) {
-#pragma unroll
-          for (int jj = 0; jj < 4; ++jj) {
-            const int n = gc4 * 4 + jj;
-            if (n >= a.wn) continue;
-            float* dst = a.out + ((size_t)(row0 + r) * a.wn + n) * B;
-            if constexpr (B == 8) {
-              if (wide_ok) {
-                float w8[8];
-#pragma unroll
-                for (int b = 0; b < 8; ++b) w8[b] = v[b][jj];
-                st_global_v8(dst, w8);
-                continue;
-              }
-            }
-#pragma unroll
-            for (int h = 0; h < B / 4; ++h)
-              *reinterpret_cast<float4*>(dst + 4 * h) = make_float4(v[4 * h][jj], v[4 * h + 1][jj], v[4 * h + 2][jj], v[4 * h + 3][jj]);
-          }
-        }
+        store_gemm_group<DIM>(a, v, tile, gc4, r, wide_ok);
       }
       fence_before_sync();
     }
@@ -617,41 +521,17 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(GemmArgs a) {
   fence_before_sync();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tbase, tcols);
-  if constexpr (SILU) {
-    // combine the four lane-quadrant warps of every channel group in a fixed order -> one partial per CTA, in the layout
-    // the MVSiLU-adjoint kernel writes ([C][2G + 1]); the chunk ring is free now (every MMA of this CTA has completed)
-    float* red = reinterpret_cast<float*>(p.lo);  // [16 warps][4 it][2 pairs][18]
-#pragma unroll
-    for (int it = 0; it < 4; ++it) {
-#pragma unroll
-      for (int pr = 0; pr < 2; ++pr) {
-        float* dst = red + ((warp * 4 + it) * 2 + pr) * 18;
-        if (lane < 18) dst[lane] = acc[it][pr];
-      }
-    }
-    __syncthreads();
-    for (int e = tid; e < a.C * NPS; e += kThreads) {
-      const int ch = e / NPS, k = e - ch * NPS;
-      const int c4 = ch >> 2, j = ch & 3, cg = c4 & 3, it = c4 >> 2, pr = j >> 1, idx = (j & 1) * NPS + k;
-      float sum = 0.f;
-#pragma unroll
-      for (int q4 = 0; q4 < 4; ++q4) sum += red[(((cg * 4 + q4) * 4 + it) * 2 + pr) * 18 + idx];
-      a.partial[((size_t)blockIdx.x * a.C + ch) * NPS + k] = sum;
-    }
-  }
 }
 
 // =====================================================================================================================
 // The same GEMM with an OVERLAPPED epilogue (resident weights, one pass, B * n16 <= 256 TMEM columns): accumulators
 // alternate between two TMEM buffers by tile and the epilogue of tile t-1 runs as channel-group units between the chunks
-// of tile t's K loop (see tc_f1db_kernel).  Warp 0 issues; warps 1-15 convert; warps 4-15 own the epilogue (lane quadrant
-// warp & 3, channel groups (warp >> 2) - 1, + 3, ...).  Bit-identical outputs; the SILU parameter-gradient partials are
-// summed in a different (still fixed) order than in tc_bgemm_kernel.
-template <int DIM, bool SILU>
-__global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(GemmArgs a) {
+// of tile t's K loop (PendingEpilogue, see tc_f1db_kernel).  Warp 0 issues; warps 1-15 convert; warps 4-15 own the
+// epilogue.  Bit-identical outputs.
+template <int DIM>
+__global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_constant__ GemmArgs a) {
   using A = Alg<DIM>;
-  constexpr int B = A::B, G = A::G, NPS = 2 * G + 1;
-  constexpr int kUnits = 6;  // channel groups per epilogue warp: n16 / 4 / 3 <= 6 (n16 <= 64)
+  constexpr int B = A::B, G = A::G;
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const uint32_t img = (uint32_t)a.n16 * a.kmax * 4;
@@ -660,19 +540,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(GemmArgs a) {
   const int nsets = a.src[1] ? 2 : 1;
   uint64_t* bars = reinterpret_cast<uint64_t*>(wimg + (size_t)nsets * set_bytes);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kPipeBars);
-  float* sa_s = reinterpret_cast<float*>(tmem_slot + 4);
-  float* sb_s = sa_s + a.n16 * G;
   Pipe p;
   p.init(smem, bars, B * kPS);
-  if (SILU) {
-    for (int i = tid; i < a.n16 * G; i += kThreads) {
-      sa_s[i] = (i < a.C * G) ? a.sa[i] : 0.f;
-      sb_s[i] = (i < a.C * G) ? a.sb[i] : 0.f;
-    }
-  }
-  float acc[kUnits][2];
-#pragma unroll
-  for (int u = 0; u < kUnits; ++u) { acc[u][0] = 0.f; acc[u][1] = 0.f; }
   const int nk = a.nk[0] + a.nk[1];
   const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
   const int total_chunks = my_tiles * nk;
@@ -705,8 +574,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(GemmArgs a) {
   const int n_c4 = Np >> 2;
 
   auto epilogue_unit = [&](int64_t tile, int c4, uint32_t tb) {
-    const int64_t row0 = tile * kTile;
-    const bool row_ok = row0 + r < a.rows;
     float v[B][4];
 #pragma unroll
     for (int b = 0; b < B; ++b) tmem_ld4(tmem_at(tb, lane_base, b * Np + c4 * 4), v[b]);
@@ -722,110 +589,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(GemmArgs a) {
     } else {
       tmem_wait_ld();
     }
-    if constexpr (SILU) {
-      const int u = c4 / 3;
-#pragma unroll
-      for (int pr = 0; pr < 2; ++pr) {
-        float2 y1v[B];
-#pragma unroll
-        for (int b = 0; b < B; ++b)
-          y1v[b] = *reinterpret_cast<const float2*>(a.y1 + bpt_off(B, a.n16, tile, b, c4, r) + 2 * pr);
-        float vals[16], t0 = 0.f, t1 = 0.f;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) vals[i] = 0.f;
-#pragma unroll
-        for (int jj = 0; jj < 2; ++jj) {
-          const int j = 2 * pr + jj, ch = c4 * 4 + j;
-          float y1[B], dy[B], sg[G], inv[G], tg[G], ds[G];
-#pragma unroll
-          for (int b = 0; b < B; ++b) {
-            y1[b] = jj == 0 ? y1v[b].x : y1v[b].y;
-            dy[b] = v[b][j];
-          }
-          const float* sa = sa_s + ch * G;
-          silu_gates<DIM>(y1, sa, sb_s + ch * G, sg, inv);
-#pragma unroll
-          for (int g = 0; g < G; ++g) tg[g] = 0.f;
-#pragma unroll
-          for (int b = 0; b < B; ++b) tg[A::grade_of(b)] = fmaf(dy[b], y1[b], tg[A::grade_of(b)]);
-          const bool ok = row_ok && ch < a.C;
-          float gv[NPS];
-#pragma unroll
-          for (int g = 0; g < G; ++g) {
-            ds[g] = ok ? tg[g] * sg[g] * (1.f - sg[g]) : 0.f;
-            gv[g] = ds[g] * inv[g];
-            gv[G + g] = ds[g];
-          }
-#pragma unroll
-          for (int b = 0; b < B; ++b) {
-            const int g = A::grade_of(b);
-            const float dinv = (g == 0) ? 1.f : 2.f * y1[b];
-            v[b][j] = ok ? fmaf(sg[g], dy[b], ds[g] * sa[g] * dinv) : 0.f;
-          }
-          gv[2 * G] = v[0][j];
-#pragma unroll
-          for (int k = 0; k < NPS; ++k) {
-            const int idx = jj * NPS + k;
-            if (idx < 16) vals[idx] = gv[k];
-            else if (idx == 16) t0 = gv[k];
-            else t1 = gv[k];
-          }
-        }
-        const float s16 = warp_transpose_reduce16(vals, lane);
-        t0 = warp_sum(t0);
-        t1 = warp_sum(t1);
-        const float mine = lane < 16 ? s16 : lane == 16 ? t0 : lane == 17 ? t1 : 0.f;
-#pragma unroll
-        for (int k = 0; k < kUnits; ++k) {
-          if (k == u) acc[k][pr] += mine;
-        }
-      }
-    }
-    if (a.out_bpt) {
-#pragma unroll
-      for (int b = 0; b < B; ++b) {
-        float4 x = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
-        if (!row_ok) x = make_float4(0.f, 0.f, 0.f, 0.f);
-        *reinterpret_cast<float4*>(a.out + bpt_off(B, a.n16, tile, b, c4, r)) = x;
-      }
-    } else if (row_ok) {
-#pragma unroll
-      for (int jj = 0; jj < 4; ++jj) {
-        const int n = c4 * 4 + jj;
-        if (n >= a.wn) continue;
-        float* dst = a.out + ((size_t)(row0 + r) * a.wn + n) * B;
-        if constexpr (B == 8) {
-          if (wide_ok) {
-            float w8[8];
-#pragma unroll
-            for (int b = 0; b < 8; ++b) w8[b] = v[b][jj];
-            st_global_v8(dst, w8);
-            continue;
-          }
-        }
-#pragma unroll
-        for (int h = 0; h < B / 4; ++h)
-          *reinterpret_cast<float4*>(dst + 4 * h) = make_float4(v[4 * h][jj], v[4 * h + 1][jj], v[4 * h + 2][jj], v[4 * h + 3][jj]);
-      }
-    }
+    store_gemm_group<DIM>(a, v, tile, c4, r, wide_ok);
   };
-  int64_t pend_tile = -1;
-  int pend_c4 = 0, pend_q = 0;
-  uint32_t pend_tb = 0;
-  bool pend_ready = false;
-  auto epilogue_step = [&]() {
-    if (warp < 4 || pend_tile < 0) return;
-    if (!pend_ready) {
-      mbar_wait(&p.slot_bar[pend_q % kRing], (pend_q / kRing) & 1);
-      fence_after_sync();
-      pend_ready = true;
-    }
-    if (pend_c4 < n_c4) {
-      epilogue_unit(pend_tile, pend_c4, pend_tb);
-      pend_c4 += 3;
-    }
-    if (pend_c4 >= n_c4) { pend_tile = -1; fence_before_sync(); }
-  };
+  PendingEpilogue pend;
 
   for (int t = 0; t < my_tiles; ++t) {
     const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
@@ -843,36 +609,16 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(GemmArgs a) {
       } else {
         mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);
         split_chunk<B>(p, q);
-        epilogue_step();
+        pend.step(p, n_c4, epilogue_unit);
       }
     }
-    while (warp >= 4 && pend_tile >= 0) epilogue_step();
-    pend_tile = tile; pend_c4 = (warp >> 2) - 1; pend_q = q - 1; pend_tb = tb; pend_ready = false;
+    pend.drain(p, n_c4, epilogue_unit);
+    pend.start(warp, tile, q - 1, tb);
   }
-  while (warp >= 4 && pend_tile >= 0) epilogue_step();
+  pend.drain(p, n_c4, epilogue_unit);
   fence_before_sync();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tbase, tcols);
-  if constexpr (SILU) {
-    float* red = reinterpret_cast<float*>(p.lo);  // [16 warps][kUnits][2 pairs][18]; 16 * 6 * 2 * 18 * 4 B = 13.8 KB <= the lo slot
-#pragma unroll
-    for (int u = 0; u < kUnits; ++u) {
-#pragma unroll
-      for (int pr = 0; pr < 2; ++pr) {
-        float* dst = red + ((warp * kUnits + u) * 2 + pr) * 18;
-        if (lane < 18) dst[lane] = acc[u][pr];
-      }
-    }
-    __syncthreads();
-    for (int e = tid; e < a.C * NPS; e += kThreads) {
-      const int ch = e / NPS, k = e - ch * NPS;
-      const int c4 = ch >> 2, j = ch & 3, g3 = c4 % 3, u = c4 / 3, pr = j >> 1, idx = (j & 1) * NPS + k;
-      float sum = 0.f;
-#pragma unroll
-      for (int q4 = 0; q4 < 4; ++q4) sum += red[((((g3 + 1) * 4 + q4) * kUnits + u) * 2 + pr) * 18 + idx];
-      a.partial[((size_t)blockIdx.x * a.C + ch) * NPS + k] = sum;
-    }
-  }
 }
 
 // =====================================================================================================================
@@ -1150,17 +896,9 @@ __global__ void __launch_bounds__(256) tc_final_kernel(FinalJobs jobs) {
 // =====================================================================================================================
 // host side
 template <int DIM>
-size_t gemm_smem(int nsets, int n16, int kmax, bool silu = false) {
+size_t gemm_smem(int nsets, int n16, int kmax) {
   constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G;
-  return (size_t)(kRing + 1) * B * kPS + (size_t)nsets * G * 2 * n16 * kmax * 4 + 128 + (silu ? (size_t)2 * n16 * G * 4 : 0);
-}
-// CSMPN_TC_FUSE_SILU=1 folds the MVSiLU adjoint into the epilogue of the dy2 GEMM (tests compare the two paths).  Default
-// since the prologue rework: its own kernel.  The fused epilogue saves two tensor passes, but it runs in the GEMM kernel's
-// one 16-warp CTA per SM, whose per-SM chain bounds the kernel; the streaming elementwise kernel (two 8-warp CTAs per SM,
-// cp.async stages) does the same work at 0.7 of the HBM roof: layer 1.130 -> 1.111 ms, motion 0.774 -> 0.739, NBA 3.14 -> 3.10.
-inline bool fuse_silu_adjoint() {
-  const char* e = getenv("CSMPN_TC_FUSE_SILU");  // read per call: a test toggles it within one process
-  return e && e[0] == '1';
+  return (size_t)(kRing + 1) * B * kPS + (size_t)nsets * G * 2 * n16 * kmax * 4 + 128;
 }
 template <int DIM>
 size_t dw_smem(int M, int na4, int cpb) {
@@ -1314,21 +1052,13 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   ga.w[0] = d.wl; ga.w[1] = d.wr; ga.wk[0] = ga.wk[1] = C; ga.wn = C;
   ga.n16 = Cp; ga.kmax = Cp;
   ga.addend = ws + p.o_dy2p; ga.out = ws + p.o_dy2; ga.out_bpt = 1;
-  // the MVSiLU adjoint runs in the epilogue of this GEMM (dy2 stays in registers, the kernel writes dy1) unless disabled
-  const bool fuse_silu = !p.wide && fuse_silu_adjoint() && Cp <= 64 && gemm_smem<DIM>(2, Cp, Cp, true) <= kSmemMax;
-  if (fuse_silu) {
-    ga.out = ws + p.o_dy1;
-    ga.y1 = d.save_y1; ga.sa = d.sa; ga.sb = d.sb; ga.partial = ws + p.o_p3; ga.C = C;
-  }
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemmdb_kernel<DIM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemmdb_kernel<DIM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  // the overlapped-epilogue GEMM needs two accumulator buffers in TMEM and at most 6 channel groups per epilogue warp
+  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemmdb_kernel<DIM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  // the overlapped-epilogue GEMM needs two accumulator buffers in TMEM
   auto overlap_ok = [&](int n16) {
     const char* e = getenv("CSMPN_TC_OVERLAP");
-    return !(e && e[0] == '0') && 2 * B * n16 <= 512 && n16 <= 64;
+    return !(e && e[0] == '0') && 2 * B * n16 <= 512;
   };
   auto prep = [&](const WPrepArgs& w, int64_t floats) -> int {
     int64_t blocks = (floats + 255) / 256;
@@ -1343,23 +1073,17 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
       int rc = prep(w, p.img_dy2);
       if (rc) return rc;
       ga.wimg = img_dy2; ga.np = p.np;
-      tc_bgemm_kernel<DIM, false, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
+      tc_bgemm_kernel<DIM, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
+    } else if (overlap_ok(ga.n16)) {  // two accumulator buffers fit: epilogue overlapped with the next tile's K loop
+      tc_bgemmdb_kernel<DIM><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax), stream>>>(ga);
     } else {
-      const size_t sm = gemm_smem<DIM>(2, ga.n16, ga.kmax, fuse_silu);
-      if (overlap_ok(ga.n16)) {  // two accumulator buffers fit: epilogue overlapped with the next tile's K loop
-        if (fuse_silu) tc_bgemmdb_kernel<DIM, true><<<grid, kThreads, sm, stream>>>(ga);
-        else tc_bgemmdb_kernel<DIM, false><<<grid, kThreads, sm, stream>>>(ga);
-      } else if (fuse_silu) {
-        tc_bgemm_kernel<DIM, true, false><<<grid, kThreads, sm, stream>>>(ga);
-      } else {
-        tc_bgemm_kernel<DIM, false, false><<<grid, kThreads, sm, stream>>>(ga);
-      }
+      tc_bgemm_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax), stream>>>(ga);
     }
     CSMPN_LAUNCH_CHECK("tc_bgemm_kernel(dy2)");
   }
   // ---- B3
   e.partial = ws + p.o_p3;
-  if ((mask & 4) && !fuse_silu) {
+  if (mask & 4) {
     const size_t sm3 = (size_t)2 * 2 * B * ew_threads * 4;
     auto run = [&](auto kern) -> int {
       CSMPN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm3));
@@ -1385,11 +1109,11 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
       int rc = prep(w, p.img_gx);
       if (rc) return rc;
       ga.wimg = img_gx; ga.np = p.np;
-      tc_bgemm_kernel<DIM, false, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
+      tc_bgemm_kernel<DIM, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
     } else if (overlap_ok(ga.n16)) {
-      tc_bgemmdb_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
+      tc_bgemmdb_kernel<DIM><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
     } else {
-      tc_bgemm_kernel<DIM, false, false><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
+      tc_bgemm_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
     }
     CSMPN_LAUNCH_CHECK("tc_bgemm_kernel(grad_x)");
   }
@@ -1504,10 +1228,9 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   cjob(ws + p.o_p1, g.g_na, p.grid_ew, NP1, P, G);
   cjob(ws + p.o_p1, g.g_la, p.grid_ew, NP1, P + G, 1);
   cjob(ws + p.o_p1, g.g_bl, p.grid_ew, NP1, P + G + 1, 1);
-  const int parts3 = fuse_silu ? grid : p.grid_ew;  // per-CTA partials of the kernel that ran the MVSiLU adjoint
-  cjob(ws + p.o_p3, g.g_sa, parts3, NP3, 0, G);
-  cjob(ws + p.o_p3, g.g_sb, parts3, NP3, G, G);
-  cjob(ws + p.o_p3, d.has_b1 ? g.g_b1 : nullptr, parts3, NP3, 2 * G, 1);
+  cjob(ws + p.o_p3, g.g_sa, p.grid_ew, NP3, 0, G);
+  cjob(ws + p.o_p3, g.g_sb, p.grid_ew, NP3, G, G);
+  cjob(ws + p.o_p3, d.has_b1 ? g.g_b1 : nullptr, p.grid_ew, NP3, 2 * G, 1);
   if (mask & 64) {
     for (size_t j0 = 0; j0 < jobs.size(); j0 += kFinalJobs) {  // wide blocks have more jobs than one launch takes
       FinalJobs fj;

@@ -209,6 +209,45 @@ __device__ __forceinline__ void zero_chunk_bpt(float* dst, int cp, int64_t tile,
   }
 }
 
+// F1 epilogue of channel group gc4 of row r of `tile`, from the accumulators already loaded from TMEM (v): bias -> y1
+// (saved when requested), MVSiLU -> y2.  b1_s / sa_s / sb_s: the bias and gate parameters staged in shared memory.
+template <int DIM>
+__device__ __forceinline__ void f1_epilogue_group(const FwdArgs& a, float (&v)[Alg<DIM>::B][4], int64_t tile, int gc4, int r,
+                                                  const float* b1_s, const float* sa_s, const float* sb_s) {
+  using A = Alg<DIM>;
+  constexpr int B = A::B, G = A::G;
+  const bool row_ok = tile * kTile + r < a.rows;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int ch = gc4 * 4 + j;
+    float y1[B];
+    const bool ok = row_ok && ch < a.C;
+#pragma unroll
+    for (int b = 0; b < B; ++b) y1[b] = ok ? v[b][j] : 0.f;
+    if (ok) y1[0] += b1_s[ch];
+#pragma unroll
+    for (int b = 0; b < B; ++b) v[b][j] = y1[b];
+  }
+  if (a.save_y1) {
+#pragma unroll
+    for (int b = 0; b < B; ++b)
+      *reinterpret_cast<float4*>(a.save_y1 + bpt_off(B, a.Cp, tile, b, gc4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
+  }
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int ch = gc4 * 4 + j;
+    float y1[B], sg[G], inv[G];
+#pragma unroll
+    for (int b = 0; b < B; ++b) y1[b] = v[b][j];
+    silu_gates<DIM>(y1, sa_s + ch * G, sb_s + ch * G, sg, inv);
+#pragma unroll
+    for (int b = 0; b < B; ++b) v[b][j] = y1[b] * sg[A::grade_of(b)];
+  }
+#pragma unroll
+  for (int b = 0; b < B; ++b)
+    *reinterpret_cast<float4*>(a.y2 + bpt_off(B, a.Cp, tile, b, gc4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
+}
+
 // =====================================================================================================================
 // F1: MVLinear (W1) + bias + MVSiLU.  ST (streamed weights, wide blocks): the output channels are produced in passes of
 // a.ns1 channels (accumulators = B * ns1 TMEM columns), the K chunks of the input are walked once per pass and every chunk
@@ -284,7 +323,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
   const uint32_t idesc = idesc_tf32(kTile, NS, false, false);
   for (int t = 0; t < my_tiles; ++t) {
     const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
-    const int64_t row0 = tile * kTile;
     for (int ps = 0; ps < npass; ++ps) {
       const int n0 = ps * NS;
       for (int kc = 0; kc < nk; ++kc, ++q) {
@@ -325,42 +363,12 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
         for (; loaded < q + kRing && loaded < total_chunks; ++loaded) load(loaded);
       }
       const int r = (warp & 3) * 32 + lane;
-      const bool row_ok = row0 + r < a.rows;
       for (int c4 = warp >> 2; c4 < (NS >> 2); c4 += 4) {
-        const int gc4 = (n0 >> 2) + c4;
         float v[B][4];
 #pragma unroll
         for (int b = 0; b < B; ++b) tmem_ld4(tmem_at(tbase, (warp & 3) * 32, b * NS + c4 * 4), v[b]);
         tmem_wait_ld();
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int ch = gc4 * 4 + j;
-          float y1[B];
-          const bool ok = row_ok && ch < C;
-#pragma unroll
-          for (int b = 0; b < B; ++b) y1[b] = ok ? v[b][j] : 0.f;
-          if (ok) y1[0] += b1_s[ch];
-#pragma unroll
-          for (int b = 0; b < B; ++b) v[b][j] = y1[b];
-        }
-        if (a.save_y1) {
-#pragma unroll
-          for (int b = 0; b < B; ++b)
-            *reinterpret_cast<float4*>(a.save_y1 + bpt_off(B, Cp, tile, b, gc4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
-        }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int ch = gc4 * 4 + j;
-          float y1[B], sg[G], inv[G];
-#pragma unroll
-          for (int b = 0; b < B; ++b) y1[b] = v[b][j];
-          silu_gates<DIM>(y1, sa_s + ch * G, sb_s + ch * G, sg, inv);
-#pragma unroll
-          for (int b = 0; b < B; ++b) v[b][j] = y1[b] * sg[A::grade_of(b)];
-        }
-#pragma unroll
-        for (int b = 0; b < B; ++b)
-          *reinterpret_cast<float4*>(a.y2 + bpt_off(B, Cp, tile, b, gc4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
+        f1_epilogue_group<DIM>(a, v, tile, (n0 >> 2) + c4, r, b1_s, sa_s, sb_s);
       }
       // The next pass's first MMA overwrites these accumulators.  It is issued only after full_bar of the next chunk has
       // collected an arrival from EVERY converter warp (conv_done), and each warp arrives after its own epilogue loads
@@ -380,7 +388,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
 // neighbouring tiles then overlap instead of running back to back (the plain kernel above spends two thirds of a tile in
 // the epilogue and its drain with the tensor pipe and the copy engine idle).
 // Roles: warp 0 issues copies and MMAs only; warps 1-15 convert / gather; warps 4-15 also own the epilogue: lane quadrant
-// warp & 3, channel groups (warp >> 2) - 1, + 3, ...  Same arithmetic as tc_f1_kernel: results are bit-identical.
+// warp & 3, channel groups (warp >> 2) - 1, + 3, ... (PendingEpilogue).  Same epilogue body as tc_f1_kernel
+// (f1_epilogue_group): results are bit-identical.
 template <int DIM, bool BPT_IN>
 __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
   using A = Alg<DIM>;
@@ -442,59 +451,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
 
   // one epilogue unit: channel group c4 of `tile`, accumulators at tb
   auto epilogue_unit = [&](int64_t tile, int c4, uint32_t tb) {
-    const bool row_ok = tile * kTile + r < a.rows;
     float v[B][4];
 #pragma unroll
     for (int b = 0; b < B; ++b) tmem_ld4(tmem_at(tb, (warp & 3) * 32, b * Cp + c4 * 4), v[b]);
     tmem_wait_ld();
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int ch = c4 * 4 + j;
-      float y1[B];
-      const bool ok = row_ok && ch < C;
-#pragma unroll
-      for (int b = 0; b < B; ++b) y1[b] = ok ? v[b][j] : 0.f;
-      if (ok) y1[0] += b1_s[ch];
-#pragma unroll
-      for (int b = 0; b < B; ++b) v[b][j] = y1[b];
-    }
-    if (a.save_y1) {
-#pragma unroll
-      for (int b = 0; b < B; ++b)
-        *reinterpret_cast<float4*>(a.save_y1 + bpt_off(B, Cp, tile, b, c4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int ch = c4 * 4 + j;
-      float y1[B], sg[G], inv[G];
-#pragma unroll
-      for (int b = 0; b < B; ++b) y1[b] = v[b][j];
-      silu_gates<DIM>(y1, sa_s + ch * G, sb_s + ch * G, sg, inv);
-#pragma unroll
-      for (int b = 0; b < B; ++b) v[b][j] = y1[b] * sg[A::grade_of(b)];
-    }
-#pragma unroll
-    for (int b = 0; b < B; ++b)
-      *reinterpret_cast<float4*>(a.y2 + bpt_off(B, Cp, tile, b, c4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
+    f1_epilogue_group<DIM>(a, v, tile, c4, r, b1_s, sa_s, sb_s);
   };
-  // pending epilogue of this warp: tile, next channel group, accumulator buffer, last chunk of that tile
-  int64_t pend_tile = -1;
-  int pend_c4 = 0, pend_q = 0;
-  uint32_t pend_tb = 0;
-  bool pend_ready = false;
-  auto epilogue_step = [&]() {  // at most one unit
-    if (warp < 4 || pend_tile < 0) return;
-    if (!pend_ready) {  // the MMAs of the pending tile have completed (its last chunk released its slot)
-      mbar_wait(&p.slot_bar[pend_q % kRing], (pend_q / kRing) & 1);
-      fence_after_sync();
-      pend_ready = true;
-    }
-    if (pend_c4 < n_c4) {
-      epilogue_unit(pend_tile, pend_c4, pend_tb);
-      pend_c4 += 3;
-    }
-    if (pend_c4 >= n_c4) { pend_tile = -1; fence_before_sync(); }
-  };
+  PendingEpilogue pend;
 
   for (int t = 0; t < my_tiles; ++t) {
     const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
@@ -532,15 +495,14 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
           if (a.save_x0 && kc == nk - 1 && (a.kin8 & 8)) zero_chunk_bpt<B>(a.save_x0, round_up(a.kin8, 16), tile, nk);
           TSTAMP(34);
         }
-        epilogue_step();  // one unit of the previous tile between two chunks of this one
+        pend.step(p, n_c4, epilogue_unit);  // one unit of the previous tile between two chunks of this one
         TSTAMP(35);
       }
     }
-    // the previous tile's epilogue must be finished before this warp signals the next tile's first chunk
-    while (warp >= 4 && pend_tile >= 0) epilogue_step();
-    pend_tile = tile; pend_c4 = (warp >> 2) - 1; pend_q = q - 1; pend_tb = tb; pend_ready = false;
+    pend.drain(p, n_c4, epilogue_unit);
+    pend.start(warp, tile, q - 1, tb);
   }
-  while (warp >= 4 && pend_tile >= 0) epilogue_step();
+  pend.drain(p, n_c4, epilogue_unit);
   fence_before_sync();
   __syncthreads();
   if (warp == 0) tmem_dealloc(tbase, tcols);

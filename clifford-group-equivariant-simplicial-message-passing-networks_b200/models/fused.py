@@ -411,7 +411,7 @@ def _tc_block_backward(ctx, gy):
         raise _lib.CsmpnError("tensor-core block backward: unsupported configuration")
     ws = workspace(nbytes, dev)
     _record("bwd", dim, d, g, ws, keep=[srcs, params, y1, xr, o, y2, x0, gy, gx, pg])
-    if _fork_enabled() and rows <= fork_max_rows():
+    if _fork_enabled():
         _tc_backward_forked(dim, d, g, ws, dev)
     else:
         check(lib().csmpn_block_bwd(dim, ctypes.byref(d), ctypes.byref(g), ptr(ws), ws.numel(), stream_ptr(dev)),
@@ -451,18 +451,13 @@ def _fork_enabled() -> bool:
     return os.environ.get("CSMPN_TC_FORK", "1") != "0"
 
 
-def fork_max_rows() -> int:
-    """Blocks with at most this many rows run their weight-gradient kernels on a side stream next to the dy2 / dy1 / grad_x
-    chain.  Default: always.  Measured on B200 (layer step, CUDA-graph replay): md17 1.63 -> 1.50 ms with the node blocks
-    (69 tiles, each kernel fills half the GPU) on the tensor-core engine, and still 1.51 -> 1.48 ms from forking the
-    per-pair blocks alone, whose persistent kernels leave SMs idle in their last wave (2.85 tiles per SM)."""
-    return int(os.environ.get("CSMPN_TC_FORK_MAX_ROWS", str(1 << 40)))
-
-
 def _tc_backward_forked(dim, d, g, ws, dev):
     """csmpn_block_bwd (engine 1) as two concurrent chains, joined before returning:
          main:  b1 -> gemm(dy2) -> b3 -> gemm(grad_x)
-         side:        dW(wl, wr) [after b1] -> dW(w1) [after b3] -> final reduce"""
+         side:        dW(wl, wr) [after b1] -> dW(w1) [after b3] -> final reduce
+    Every block forks, whatever its row count.  Measured on B200 (layer step, CUDA-graph replay): md17 1.63 -> 1.50 ms with
+    the node blocks (69 tiles, each kernel fills half the GPU) on the tensor-core engine, and still 1.51 -> 1.48 ms from
+    forking the per-pair blocks alone, whose persistent kernels leave SMs idle in their last wave (2.85 tiles per SM)."""
     main = torch.cuda.current_stream(dev)
     side = _SIDE_STREAMS.get(dev)
     if side is None:
@@ -544,9 +539,6 @@ def _need_grad(*tensors_and_params):
     return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors_and_params)
 
 
-TC_BACKWARD_READY = True
-
-
 def tc_min_rows() -> int:
     """Rows below which a block stays on the FP32 SIMT engine: the tensor-core engine runs a block as several
     persistent kernels over 128-row tiles, each paying its prologue once per CTA.  With the batched weight staging
@@ -557,7 +549,7 @@ def tc_min_rows() -> int:
 
 def _block_uses_tc(algebra, layer, need_grad, rows=None) -> bool:
     lin = layer[0]
-    if algebra.dim not in (2, 3) or (need_grad and not TC_BACKWARD_READY):
+    if algebra.dim not in (2, 3):
         return False
     if not tc_supported(algebra.dim, lin.in_features, lin.out_features):
         return False
@@ -708,12 +700,9 @@ def _kernel_stages(d: BlockDesc, g, B: int):
                 ("tc_f2", "linear_right/left + normalisation + weighted GP + MVLayerNorm (+residual)", 2, 4 * T + y_out, 3 * rows * 4 * B * C * C)]
     gy = T if g.gy_bpt else ref(C)
     gx = 0 if not g.grad_x else (Tin if g.gx_bpt else ref(cin))
-    wide = bool(lib().csmpn_block_tc_plan(B.bit_length() - 1, cin, C) & 8)
-    fused_silu = os.environ.get("CSMPN_TC_FUSE_SILU", "0") == "1" and cp <= 64 and not wide
-    mid = ([("tc_bgemm", "dy2 = dy2p + d WL + dxr WR, MVSiLU adjoint in the epilogue -> dy1", 2, 5 * T, 3 * rows * 4 * B * C * C)]
-           if fused_silu else
-           [("tc_bgemm", "dy2 = dy2p + d WL + dxr WR", 2, 4 * T, 3 * rows * 4 * B * C * C), ("tc_b3", "MVSiLU adjoint", 4, 3 * T, 0)])
-    return [("tc_b1", "MVLayerNorm / weighted GP / normalisation adjoints", 1, 6 * T + gy, 0)] + mid + [
+    return [("tc_b1", "MVLayerNorm / weighted GP / normalisation adjoints", 1, 6 * T + gy, 0),
+            ("tc_bgemm", "dy2 = dy2p + d WL + dxr WR", 2, 4 * T, 3 * rows * 4 * B * C * C),
+            ("tc_b3", "MVSiLU adjoint", 4, 3 * T, 0),
             ("tc_bgemm", "grad_x = dy1 W1", 8, T + gx, 3 * rows * 2 * B * C * cin),
             ("tc_dw", "dWL, dWR = [d|dxr]^T y2", 16, 3 * T, 3 * rows * 4 * B * C * C),
             ("tc_dw", "dW1 = dy1^T x0", 32, T + Tin, 3 * rows * 2 * B * C * cin),

@@ -335,34 +335,6 @@ def test_graphed_layer_with_paired_node_attr():
         assert torch.equal(a, b)
 
 
-@pytest.mark.parametrize("case", [CASES[1], CASES[2], CASES[3]], ids=["md17", "nba", "odd_c"])
-def test_silu_adjoint_folded_into_gemm_matches_separate_kernel(case, monkeypatch):
-    """The MVSiLU adjoint runs in the epilogue of the dy2 GEMM (dy2 never leaves the SM; warp-transposed reduction of the
-    gate-parameter gradients); CSMPN_TC_FUSE_SILU=0 keeps it as its own kernel.  Same gradients either way."""
-    name, metric, C, T, ncx, n, e, aggr = case
-    CliffordAlgebra, M = _mods()
-    ralg, params, h, ei, ea, na, cot = _inputs(case)
-    alg = CliffordAlgebra(metric).to(DEV)
-    m = M.EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=aggr).to(DEV)
-    _load(m, params)
-    names = [k for k, _ in m.named_parameters()]
-    plist = [p for _, p in m.named_parameters()]
-    out = {}
-    from csmpn_b200 import _lib
-
-    for fuse in ("1", "0"):
-        monkeypatch.setenv("CSMPN_TC_FUSE_SILU", fuse)
-        hd = h.to(DEV).requires_grad_()
-        n0 = _lib.lib().csmpn_launch_count()
-        y = m(hd, ei.to(DEV), ea.to(DEV), na.to(DEV))
-        out[fuse] = torch.autograd.grad(y, [hd] + plist, cot.to(DEV))
-        torch.cuda.synchronize()
-        out["launches" + fuse] = _lib.lib().csmpn_launch_count() - n0
-    assert out["launches0"] == out["launches1"] + 4  # one kernel less per block
-    for what, a, b in zip(["gh"] + names, out["1"], out["0"]):
-        assert_close(a, b, 2e-6, f"{name} {what} fused vs separate MVSiLU adjoint")
-
-
 # ---------------------------------------------------------------------------------------------------------------------
 # wide blocks: weights streamed with the K chunks (csmpn_block_tc_plan bits 1-3), hidden widths 64 / 128 / 256
 WIDE = [
@@ -424,8 +396,7 @@ def test_wide_block_forward_backward_vs_oracle(case):
 @pytest.mark.parametrize("case", [CASES[0], CASES[1], CASES[2], CASES[3], CASES[4]], ids=["motion", "md17", "nba", "odd_c", "tiny"])
 def test_overlapped_epilogue_kernels_match_plain_kernels(case, monkeypatch):
     """tc_f1db / tc_bgemmdb (two TMEM accumulator buffers, epilogue of tile t-1 interleaved with the K loop of tile t) against
-    the plain kernels (CSMPN_TC_OVERLAP=0): same arithmetic, so the layer output is bit-identical; the MVSiLU parameter
-    gradients are summed in another fixed order"""
+    the plain kernels (CSMPN_TC_OVERLAP=0): same arithmetic, so the layer output and every gradient are bit-identical"""
     name, metric, C, T, ncx, n, e, aggr = case
     CliffordAlgebra, M = _mods()
     ralg, params, h, ei, ea, na, cot = _inputs(case)
@@ -443,4 +414,4 @@ def test_overlapped_epilogue_kernels_match_plain_kernels(case, monkeypatch):
         torch.cuda.synchronize()
     assert torch.equal(out["1"][0], out["0"][0])
     for what, a, b in zip(["gh"] + names, out["1"][1], out["0"][1]):
-        assert_close(a, b, 2e-6, f"{name} {what} overlapped vs plain")
+        assert torch.equal(a, b), f"{name} {what} overlapped vs plain"

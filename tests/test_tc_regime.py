@@ -143,7 +143,7 @@ def test_step_is_deterministic_in_bench_regime(bench_mod):
 
 def test_overlapped_epilogue_bitwise_in_bench_regime(bench_mod, monkeypatch):
     """three tiles per CTA, alternating TMEM buffers: the overlapped-epilogue kernels reproduce the plain kernels' layer
-    output bit for bit on the bench batch"""
+    output and every gradient bit for bit on the bench batch"""
     b = bench_mod.make_batch("md17", 100, 1000)
     params = R.init_egcl_params(R.RefAlgebra(b["metric"]), b["C"], T, torch.Generator().manual_seed(7))
     monkeypatch.setenv("CSMPN_TC_OVERLAP", "1")
@@ -151,6 +151,5 @@ def test_overlapped_epilogue_bitwise_in_bench_regime(bench_mod, monkeypatch):
     monkeypatch.setenv("CSMPN_TC_OVERLAP", "0")
     y0, g0 = _ours(b, params)
     assert torch.equal(y1, y0)
-    assert torch.equal(g1["h"], g0["h"])
     for k in g1:
-        assert rel_err(g1[k], g0[k]) <= 2e-6, k
+        assert torch.equal(g1[k], g0[k]), k
