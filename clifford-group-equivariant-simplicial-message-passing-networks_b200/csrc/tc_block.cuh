@@ -193,7 +193,32 @@ __device__ __forceinline__ uint64_t chunk_desc(uint32_t half_saddr, int b) {
   return smem_desc(half_saddr + (uint32_t)b * kPS, kKH, 128u);
 }
 
-// ---- K-chunk pipeline shared by the GEMM kernels ------------------------------------------------------------------
+// ---- persistent CTAs, TMEM, prologue and teardown (every tcgen05 kernel) -----------------------------------------------
+// One CTA per SM; this CTA runs tiles blockIdx.x, blockIdx.x + gridDim.x, ...
+__device__ __forceinline__ int cta_tiles(int tiles) { return (tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x; }
+__device__ __forceinline__ int64_t cta_tile(int t) { return (int64_t)blockIdx.x + (int64_t)t * gridDim.x; }
+// tcgen05.alloc takes a power of two >= 32 columns
+__host__ __device__ constexpr uint32_t tmem_cols(uint32_t need) {
+  return need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+}
+// End of the prologue: the barrier inits, the TMEM address written by tcgen05.alloc and the generic-proxy stores of the
+// staged weights are visible to every thread and to the tensor cores.
+__device__ __forceinline__ void prologue_sync() {
+  fence_async_smem();
+  fence_before_sync();
+  __syncthreads();
+  fence_after_sync();
+}
+// End of the kernel: every warp's TMEM accesses are complete before the allocating warp 0 frees the columns.
+__device__ __forceinline__ void tmem_teardown(int warp, uint32_t tbase, uint32_t tcols) {
+  fence_before_sync();
+  __syncthreads();
+  if (warp == 0) tmem_dealloc(tbase, tcols);
+}
+
+constexpr size_t kSmemMax = 227 * 1024;  // dynamic shared memory of one CTA
+
+// ---- K-chunk pipeline of the ring-fed kernels (tc_f1, tc_f1db, tc_f2, tc_bgemm, tc_bgemmdb) ----------------------------
 // A chunk = 8 channels of all blades of a 128-row tile.  Chunk q lands (bulk copies) in raw slot q % kRing; the split
 // pass turns the slot into the TF32-exact high parts in place and writes the remainders to the single `lo` buffer;
 // the MMAs of the chunk read both.  Loads run kRing-1 chunks ahead of the MMAs (two chunks = 64 KB per SM in flight).
@@ -205,6 +230,16 @@ __device__ __forceinline__ uint64_t chunk_desc(uint32_t half_saddr, int b) {
 // tcgen05.mma kind::tf32 reads fp32 operands and ignores the low 13 mantissa bits (truncation, verified on B200 by the
 // 1e-5 parity tests, which a round-to-nearest read would fail by 2^-11): the raw chunk already IS the high operand, so the
 // split pass only has to produce the remainders.
+//
+// Reuse rules (nothing but these mbarriers orders the K loop):
+// * Raw slot q % kRing is overwritten by chunk q + kRing only once slot_bar has seen the MMAs of chunk q complete:
+//   ChunkFeed::refill / refill_all for bulk copies, Pipe::wait_free(q - kRing) for the gathering producer's stores.
+// * `lo` is rewritten for chunk q once lo_bar has seen the MMAs of chunk q-1 complete (split_chunk, store_chunk_api).
+// * An accumulator is read (tcgen05.ld) only after wait_mmas of the last chunk that wrote it.  It is overwritten by the
+//   first MMA of a later pass or tile, which the issuer issues only after wait_full of that chunk; every converter warp
+//   arrives on full_bar (conv_done) after its own epilogue loads (tcgen05.wait::ld), and the issuer warp runs its part
+//   of a plain epilogue itself, so the mbarrier orders the reuse.  The overlapped kernels alternate two accumulator
+//   buffers by tile (PendingEpilogue).
 constexpr bool kTf32Truncates = true;
 constexpr int kRing = 3;
 constexpr int kPipeBars = 3 * kRing + 1;
@@ -239,6 +274,48 @@ struct Pipe {
     mbar_wait(&full_bar[q % kRing], (q / kRing) & 1);
     fence_after_sync();
   }
+  // the bulk copies of chunk q (activation planes and / or weight unit) have landed in its slot
+  __device__ __forceinline__ void wait_landed(int q) const { mbar_wait(&load_bar[q % kRing], (q / kRing) & 1); }
+  // the MMAs of chunk q have completed: its slot may be overwritten
+  __device__ __forceinline__ void wait_free(int q) const { mbar_wait(&slot_bar[q % kRing], (q / kRing) & 1); }
+  // ... and, with those of every earlier chunk, written their accumulators: tcgen05.ld may read them
+  __device__ __forceinline__ void wait_mmas(int q) const {
+    wait_free(q);
+    fence_after_sync();
+  }
+};
+
+// Copy-ahead of the issuer warp (all lanes of warp 0): chunk loads run kRing - 1 chunks ahead of the MMAs.  `load(q)`
+// issues the bulk copies of the CTA's chunk q; `total` = chunks of this CTA.  ON == false (no bulk copies: gathered
+// input with resident weights) compiles every call away.  The loader is an argument of each call rather than a member:
+// a struct holding the lambda (or a reference to it) made nvcc widen shared-memory address arithmetic to 64 bits and
+// cost the streamed-weight kernels 3 to 7 registers.
+template <bool ON = true>
+struct ChunkFeed {
+  const Pipe& p;
+  int total;
+  int loaded = 0;  // chunks whose copies have been issued
+  // The first kRing - 1 chunks, requested BEFORE the weights are staged: with one to three tiles per CTA the prologue is
+  // a visible part of the kernel and these latencies overlap it.
+  template <class Load>
+  __device__ __forceinline__ void prime(Load&& load) {
+    if (ON) for (; loaded < kRing - 1 && loaded < total; ++loaded) load(loaded);
+  }
+  // After wait_full(q): slot (q-1) % kRing was read by the MMAs of chunk q-1, issued a whole chunk period ago; reload it
+  // before issuing the MMAs of chunk q, so that the copy has their issue time as extra lead.
+  template <class Load>
+  __device__ __forceinline__ void refill(int q, Load&& load) {
+    if (ON && loaded == q + kRing - 1 && loaded < total) {
+      if (q >= 1) p.wait_free(q - 1);
+      load(loaded);
+      ++loaded;
+    }
+  }
+  // After wait_mmas(q - 1) at the end of a pass: every slot is free; prefetch the next chunks under the epilogue.
+  template <class Load>
+  __device__ __forceinline__ void refill_all(int q, Load&& load) {
+    if (ON) for (; loaded < q + kRing && loaded < total; ++loaded) load(loaded);
+  }
 };
 
 // ---- overlapped epilogue (tc_f1db_kernel, tc_bgemmdb_kernel) ---------------------------------------------------------
@@ -260,8 +337,7 @@ struct PendingEpilogue {
   __device__ __forceinline__ void step(const Pipe& p, int n_c4, Unit&& unit) {
     if (tile < 0) return;
     if (!ready) {  // the MMAs of the pending tile have completed (its last chunk released its slot)
-      mbar_wait(&p.slot_bar[q % kRing], (q / kRing) & 1);
-      fence_after_sync();
+      p.wait_mmas(q);
       ready = true;
     }
     if (c4 < n_c4) {
@@ -334,6 +410,22 @@ __global__ void tc_weight_images_kernel(WPrepArgs a) {
 template <int DIM>
 __host__ inline int64_t weight_image_floats(int stack, int np, int npass, int nk_total) {
   return (int64_t)npass * nk_total * Alg<DIM>::G * 2 * (stack ? 2 * np : np) * 8;
+}
+template <int DIM>
+__host__ int launch_weight_images(const WPrepArgs& w, int64_t floats, cudaStream_t stream) {
+  int64_t blocks = (floats + 255) / 256;
+  if (blocks > 4096) blocks = 4096;
+  tc_weight_images_kernel<DIM><<<(unsigned)blocks, 256, 0, stream>>>(w);
+  CSMPN_LAUNCH_CHECK("tc_weight_images_kernel");
+  return CSMPN_OK;
+}
+
+// The overlapped-epilogue kernels (tc_f1db, tc_bgemmdb) need two accumulator buffers of B * ncols columns in TMEM.
+// CSMPN_TC_OVERLAP=0 selects the plain kernels (epilogue after the K loop); read per call so a test can compare both.
+__host__ inline bool use_overlapped_epilogue(int B, int ncols) {
+  if (2 * B * ncols > 512) return false;
+  const char* e = getenv("CSMPN_TC_OVERLAP");
+  return !(e && e[0] == '0');
 }
 
 // bulk copies of chunk q (8 channels kc of a BPT tensor) into its raw slot: called by ALL lanes of one warp

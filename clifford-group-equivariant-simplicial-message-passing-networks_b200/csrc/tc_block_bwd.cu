@@ -431,9 +431,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
   const int npass = (a.n16 + nmax - 1) / nmax;
   const int nk = a.nk[0] + a.nk[1];
   const int per_tile = npass * nk;
-  const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  const int total_chunks = my_tiles * per_tile;
-  auto issue = [&](int qq) {  // chunk qq of this CTA (all lanes of warp 0)
+  const int my_tiles = cta_tiles(a.tiles);
+  auto load = [&](int qq) {
+    // = cta_tile(qq / per_tile); called through the helper, nvcc gives tc_bgemm_kernel<3, true> 4 more registers
     const int64_t tile = (int64_t)blockIdx.x + (int64_t)(qq / per_tile) * gridDim.x;
     const int kc = (qq % per_tile) % nk;
     const int s = kc < a.nk[0] ? 0 : 1;
@@ -444,24 +444,21 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
       issue_chunk_load<B>(p, qq, a.src[s], a.cp[s], tile, s ? kc - a.nk[0] : kc);
     }
   };
-  int q = 0, loaded = 0;
-  if (warp == 0) for (; loaded < kRing - 1 && loaded < total_chunks; ++loaded) issue(loaded);  // before the weights are staged
-  const uint32_t need = (uint32_t)B * (a.n16 < nmax ? a.n16 : nmax);
-  const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+  ChunkFeed<> feed{p, my_tiles * per_tile};
+  int q = 0;
+  if (warp == 0) feed.prime(load);
+  const uint32_t tcols = tmem_cols((uint32_t)B * (a.n16 < nmax ? a.n16 : nmax));
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   if (!ST) {
     const WJob wj[2] = {{wimg, a.w[0], a.wk[0], a.wn, 0}, {wimg + set_bytes, a.w[nsets - 1], a.wk[nsets - 1], a.wn, 0}};
     stage_weight_jobs<DIM, true, 2>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
   }
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
+  prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t lane_base = (warp & 3) * 32;
   const bool wide_ok = aligned32(a.out);
   for (int t = 0; t < my_tiles; ++t) {
-    const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
+    const int64_t tile = cta_tile(t);
     for (int ps = 0; ps < npass; ++ps) {
       const int n0 = ps * nmax;
       const int Np = (a.n16 - n0) < nmax ? (a.n16 - n0) : nmax;
@@ -469,20 +466,16 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
       for (int kc = 0; kc < nk; ++kc, ++q) {
         if (warp == 0) {  // issuer
           p.wait_full(q);
-          if (loaded == q + kRing - 1 && loaded < total_chunks) {  // reload the slot of chunk q-1 before issuing the MMAs
-            if (q >= 1) mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-            issue(loaded);
-            ++loaded;
-          }
+          feed.refill(q, load);
           if constexpr (ST) {
-            mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);  // the weight unit of this chunk has landed
+            p.wait_landed(q);  // the weight unit of this chunk
             issue_chunk_mma<DIM>(p, q, tbase, Np, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, nmax, 0, 0, idesc);
           } else {
             const int s = kc < a.nk[0] ? 0 : 1;
             issue_chunk_mma<DIM>(p, q, tbase, Np, kc > 0, wimg, img, s, 1, set_bytes, a.n16, s ? kc - a.nk[0] : kc, n0, idesc);
           }
         } else {          // converters
-          mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);
+          p.wait_landed(q);
           split_chunk<B>(p, q);
         }
       }
@@ -494,9 +487,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
 #pragma unroll
         for (int b = 0; b < B; ++b) ad[b] = *reinterpret_cast<const float4*>(a.addend + bpt_off(B, a.n16, tile, b, (n0 >> 2) + (warp >> 2), r));
       }
-      mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-      fence_after_sync();
-      if (warp == 0) for (; loaded < q + kRing && loaded < total_chunks; ++loaded) issue(loaded);
+      p.wait_mmas(q - 1);
+      if (warp == 0) feed.refill_all(q, load);
       for (int c4 = warp >> 2; c4 < (Np >> 2); c4 += 4) {
         float v[B][4];
 #pragma unroll
@@ -518,9 +510,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
       fence_before_sync();
     }
   }
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, tcols);
+  tmem_teardown(warp, tbase, tcols);
 }
 
 // =====================================================================================================================
@@ -543,29 +533,24 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_co
   Pipe p;
   p.init(smem, bars, B * kPS);
   const int nk = a.nk[0] + a.nk[1];
-  const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  const int total_chunks = my_tiles * nk;
-  auto issue = [&](int qq) {
-    const int64_t tile = (int64_t)blockIdx.x + (int64_t)(qq / nk) * gridDim.x;
+  const int my_tiles = cta_tiles(a.tiles);
+  auto load = [&](int qq) {
     const int kc = qq % nk;
     const int s = kc < a.nk[0] ? 0 : 1;
-    issue_chunk_load<B>(p, qq, a.src[s], a.cp[s], tile, s ? kc - a.nk[0] : kc);
+    issue_chunk_load<B>(p, qq, a.src[s], a.cp[s], cta_tile(qq / nk), s ? kc - a.nk[0] : kc);
   };
-  int q = 0, loaded = 0;
-  if (warp == 0) for (; loaded < kRing - 1 && loaded < total_chunks; ++loaded) issue(loaded);  // before the weights are staged
+  ChunkFeed<> feed{p, my_tiles * nk};
+  int q = 0;
+  if (warp == 0) feed.prime(load);
   const int Np = a.n16;
   const uint32_t bufcols = (uint32_t)B * Np;  // <= 256 (host)
-  const uint32_t need = 2 * bufcols;
-  const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+  const uint32_t tcols = tmem_cols(2 * bufcols);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   {
     const WJob wj[2] = {{wimg, a.w[0], a.wk[0], a.wn, 0}, {wimg + set_bytes, a.w[nsets - 1], a.wk[nsets - 1], a.wn, 0}};
     stage_weight_jobs<DIM, true, 2>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
   }
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
+  prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t idesc = idesc_tf32(kTile, Np, false, false);
   const uint32_t lane_base = (warp & 3) * 32;
@@ -594,20 +579,16 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_co
   PendingEpilogue pend;
 
   for (int t = 0; t < my_tiles; ++t) {
-    const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
+    const int64_t tile = cta_tile(t);
     const uint32_t tb = tbase + (uint32_t)(t & 1) * bufcols;
     for (int kc = 0; kc < nk; ++kc, ++q) {
       if (warp == 0) {  // issuer
         p.wait_full(q);
-        if (loaded == q + kRing - 1 && loaded < total_chunks) {
-          if (q >= 1) mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-          issue(loaded);
-          ++loaded;
-        }
+        feed.refill(q, load);
         const int s = kc < a.nk[0] ? 0 : 1;
         issue_chunk_mma<DIM>(p, q, tb, Np, kc > 0, wimg, img, s, 1, set_bytes, a.n16, s ? kc - a.nk[0] : kc, 0, idesc);
       } else {
-        mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);
+        p.wait_landed(q);
         split_chunk<B>(p, q);
         pend.step(p, n_c4, epilogue_unit);
       }
@@ -616,9 +597,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_co
     pend.start(warp, tile, q - 1, tb);
   }
   pend.drain(p, n_c4, epilogue_unit);
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, tcols);
+  tmem_teardown(warp, tbase, tcols);
 }
 
 // =====================================================================================================================
@@ -699,23 +678,18 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
   // instructions.  The epilogue adds the two column halves and writes the two lane halves as two partials.
   const bool merged = a.M == 64;
   const uint32_t ncol = merged ? 2u * gb * 32u : (uint32_t)a.cpb;  // accumulator columns per grade
-  const uint32_t need = (uint32_t)G * ncol;
-  const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+  const uint32_t tcols = tmem_cols((uint32_t)G * ncol);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
+  prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t idesc = merged ? idesc_tf32(128, (int)ncol, true, true) : idesc_tf32(a.M, a.cpb, true, true);
-  const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  const int steps = my_tiles * B * 2;  // step = (tile, blade, row half)
+  const int steps = cta_tiles(a.tiles) * B * 2;  // step = (tile, blade, row half)
   // The producer/issuer warp and the converter warps are decoupled by mbarriers (no CTA-wide barrier in the loop): the
   // conversion of step st+1 runs while warp 0 issues the MMAs of step st and the copies of step st+kDwLand.
   if (warp == 0) {
     const int units = steps >> 1;        // landing units = (tile, blade)
     auto issue = [&](int lu) {           // all lanes of warp 0
-      const int64_t tile = (int64_t)blockIdx.x + (int64_t)(lu / B) * gridDim.x;
+      const int64_t tile = cta_tile(lu / B);
       const int b = lu % B;
       uint8_t* dst = land + (size_t)(lu % kDwLand) * land_bytes;
       uint64_t* bar = &load_bar[lu % kDwLand];
@@ -833,9 +807,7 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
       }
     }
   }
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, tcols);
+  tmem_teardown(warp, tbase, tcols);
 }
 
 // =====================================================================================================================
@@ -905,7 +877,6 @@ size_t dw_smem(int M, int na4, int cpb) {
   const int ga = M / 32, gb = (cpb + 31) / 32;
   return (size_t)2 * 2 * (ga + gb) * kDwRows * 128 + (size_t)kDwLand * (na4 + cpb / 4) * kLand + 128;  // kLand = 2 KB
 }
-constexpr size_t kSmemMax = 227 * 1024;
 
 struct BwdPlan {
   int Cp, cin, n16, tiles;
@@ -1055,26 +1026,14 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemmdb_kernel<DIM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  // the overlapped-epilogue GEMM needs two accumulator buffers in TMEM
-  auto overlap_ok = [&](int n16) {
-    const char* e = getenv("CSMPN_TC_OVERLAP");
-    return !(e && e[0] == '0') && 2 * B * n16 <= 512;
-  };
-  auto prep = [&](const WPrepArgs& w, int64_t floats) -> int {
-    int64_t blocks = (floats + 255) / 256;
-    if (blocks > 4096) blocks = 4096;
-    tc_weight_images_kernel<DIM><<<(unsigned)blocks, 256, 0, stream>>>(w);
-    CSMPN_LAUNCH_CHECK("tc_weight_images_kernel");
-    return CSMPN_OK;
-  };
   if (mask & 2) {
     if (p.wide) {
       WPrepArgs w{d.wl, d.wr, 0, 1, C, C, C, p.np, (Cp + p.np - 1) / p.np, Cp / 8, Cp / 8, img_dy2};
-      int rc = prep(w, p.img_dy2);
+      int rc = launch_weight_images<DIM>(w, p.img_dy2, stream);
       if (rc) return rc;
       ga.wimg = img_dy2; ga.np = p.np;
       tc_bgemm_kernel<DIM, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
-    } else if (overlap_ok(ga.n16)) {  // two accumulator buffers fit: epilogue overlapped with the next tile's K loop
+    } else if (use_overlapped_epilogue(B, ga.n16)) {
       tc_bgemmdb_kernel<DIM><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax), stream>>>(ga);
     } else {
       tc_bgemm_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax), stream>>>(ga);
@@ -1106,11 +1065,11 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
     ga.out = g.grad_x; ga.out_bpt = g.gx_bpt;
     if (p.wide) {
       WPrepArgs w{d.w1, nullptr, 0, 1, p.cin, C, 0, p.np, (p.n16 + p.np - 1) / p.np, Cp / 8, 0, img_gx};
-      int rc = prep(w, p.img_gx);
+      int rc = launch_weight_images<DIM>(w, p.img_gx, stream);
       if (rc) return rc;
       ga.wimg = img_gx; ga.np = p.np;
       tc_bgemm_kernel<DIM, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
-    } else if (overlap_ok(ga.n16)) {
+    } else if (use_overlapped_epilogue(B, ga.n16)) {
       tc_bgemmdb_kernel<DIM><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
     } else {
       tc_bgemm_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);

@@ -248,6 +248,26 @@ __device__ __forceinline__ void f1_epilogue_group(const FwdArgs& a, float (&v)[A
     *reinterpret_cast<float4*>(a.y2 + bpt_off(B, a.Cp, tile, b, gc4, r)) = make_float4(v[b][0], v[b][1], v[b][2], v[b][3]);
 }
 
+// The bias and gate parameters of f1 into shared memory: b1_s [Cp], sa_s / sb_s [Cp][G], zero beyond the real channels.
+// Each thread's first elements are requested before stage_weights() runs (one exposed latency for the whole prologue
+// instead of one per loop), the rest after it.
+template <int DIM, class StageWeights>
+__device__ __forceinline__ void stage_f1_params(const FwdArgs& a, float* b1_s, float* sa_s, float* sb_s, StageWeights&& stage_weights) {
+  constexpr int G = Alg<DIM>::G;
+  const int tid = threadIdx.x, C = a.C, Cp = a.Cp;
+  const float pf_b1 = (tid < C && a.has_b1) ? __ldg(a.b1 + tid) : 0.f;
+  const float pf_sa = tid < C * G ? __ldg(a.sa + tid) : 0.f;
+  const float pf_sb = tid < C * G ? __ldg(a.sb + tid) : 0.f;
+  stage_weights();
+  if (tid < Cp) b1_s[tid] = pf_b1;
+  for (int i = tid + kThreads; i < Cp; i += kThreads) b1_s[i] = (i < C && a.has_b1) ? a.b1[i] : 0.f;
+  if (tid < Cp * G) { sa_s[tid] = pf_sa; sb_s[tid] = pf_sb; }
+  for (int i = tid + kThreads; i < Cp * G; i += kThreads) {
+    sa_s[i] = (i < C * G) ? a.sa[i] : 0.f;
+    sb_s[i] = (i < C * G) ? a.sb[i] : 0.f;
+  }
+}
+
 // =====================================================================================================================
 // F1: MVLinear (W1) + bias + MVSiLU.  ST (streamed weights, wide blocks): the output channels are produced in passes of
 // a.ns1 channels (accumulators = B * ns1 TMEM columns), the K chunks of the input are walked once per pass and every chunk
@@ -256,7 +276,6 @@ template <int DIM, bool BPT_IN, bool ST>
 __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G;
-  constexpr bool LOADS = BPT_IN || ST;  // the issuer warp runs the copy-ahead logic (activation planes and / or weight units)
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int C = a.C, Cp = a.Cp, nk = a.kin8 / 8;
@@ -273,11 +292,12 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kPipeBars);
   Pipe p;
   p.init(smem, bars, half);
-  const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
+  const int my_tiles = cta_tiles(a.tiles);
   const int per_tile = npass * nk;
   const int total_chunks = my_tiles * per_tile;
-  auto tile_of = [&](int q) { return (int64_t)blockIdx.x + (int64_t)(q / per_tile) * gridDim.x; };
-  auto load = [&](int qq) {  // copies of chunk qq of this CTA (all lanes of warp 0)
+  auto tile_of = [&](int q) { return cta_tile(q / per_tile); };
+  // the issuer's bulk copies: activation planes (BPT input) and / or weight units (ST)
+  auto load = [&](int qq) {
     if constexpr (ST) {
       const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(a.wimg1) + (size_t)(qq % per_tile) * wunit;
       issue_chunk_load_w<B>(p, qq, BPT_IN ? a.p0 : nullptr, a.in_cp, tile_of(qq), qq % nk, wsrc, wunit);
@@ -285,67 +305,44 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
       issue_chunk_load<B>(p, qq, a.p0, a.in_cp, tile_of(qq), qq % nk);
     }
   };
-  // The first chunks are requested BEFORE the weights are staged (bulk copies by the thread that initialised the
-  // barriers; register gathers by the converters): with one to three tiles per CTA the prologue is a visible part of
-  // the kernel and these latencies overlap it.
-  int q = 0;       // chunk sequence number of this CTA; chunk q lives in raw slot q % kRing
-  int loaded = 0;  // warp 0: chunks whose bulk copies have been issued
+  ChunkFeed<BPT_IN || ST> feed{p, total_chunks};
+  // the gathering converters request their first chunk before the prologue as well (see ChunkFeed::prime)
+  int q = 0;  // chunk sequence number of this CTA; chunk q lives in raw slot q % kRing
   float4 gv[BPT_IN ? 1 : ApiItems<DIM>::N];  // gathered items of the NEXT chunk to stage (API-layout input)
   GatherIdx<DIM> gi;
   if (!BPT_IN && warp != 0 && total_chunks > 0) {
     load_gather_idx<DIM>(a, tile_of(0) * kTile, gi);
     gather_chunk_api<DIM>(a, tile_of(0) * kTile, 0, gv, gi);
   }
-  if (LOADS && warp == 0) {
-    for (; loaded < kRing - 1 && loaded < total_chunks; ++loaded) load(loaded);
-  }
+  if (warp == 0) feed.prime(load);
 
-  const uint32_t need = (uint32_t)B * NS;
-  const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+  const uint32_t tcols = tmem_cols((uint32_t)B * NS);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
-  // small parameters requested before the weights are staged (see tc_f2_kernel)
-  const float pf_b1 = (tid < C && a.has_b1) ? __ldg(a.b1 + tid) : 0.f;
-  const float pf_sa = tid < C * G ? __ldg(a.sa + tid) : 0.f;
-  const float pf_sb = tid < C * G ? __ldg(a.sb + tid) : 0.f;
-  if (!ST) stage_weight_images<DIM, false>(wimg, img, a.w1, C, a.cin, Cp, a.kin8);
-  if (tid < Cp) b1_s[tid] = pf_b1;
-  for (int i = tid + kThreads; i < Cp; i += kThreads) b1_s[i] = (i < C && a.has_b1) ? a.b1[i] : 0.f;
-  if (tid < Cp * G) { sa_s[tid] = pf_sa; sb_s[tid] = pf_sb; }
-  for (int i = tid + kThreads; i < Cp * G; i += kThreads) {
-    sa_s[i] = (i < C * G) ? a.sa[i] : 0.f;
-    sb_s[i] = (i < C * G) ? a.sb[i] : 0.f;
-  }
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
+  stage_f1_params<DIM>(a, b1_s, sa_s, sb_s, [&] {
+    if (!ST) stage_weight_images<DIM, false>(wimg, img, a.w1, C, a.cin, Cp, a.kin8);
+  });
+  prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t idesc = idesc_tf32(kTile, NS, false, false);
   for (int t = 0; t < my_tiles; ++t) {
-    const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
+    const int64_t tile = cta_tile(t);
     for (int ps = 0; ps < npass; ++ps) {
       const int n0 = ps * NS;
       for (int kc = 0; kc < nk; ++kc, ++q) {
         if (warp == 0) {  // issuer
           p.wait_full(q);
-          if (LOADS && loaded == q + kRing - 1 && loaded < total_chunks) {
-            // slot (q-1) % kRing was read by the MMAs of chunk q-1, issued a whole chunk period ago: reload it first, so
-            // that the copy has the issue time of this chunk's MMAs as extra lead
-            if (q >= 1) mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-            load(loaded);
-            ++loaded;
-          }
+          feed.refill(q, load);
           if constexpr (ST) {
-            mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);  // the weight unit of this chunk has landed
+            p.wait_landed(q);  // the weight unit of this chunk
             issue_chunk_mma<DIM>(p, q, tbase, NS, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, NS, 0, 0, idesc);
           } else {
             issue_chunk_mma<DIM>(p, q, tbase, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
           }
         } else if (BPT_IN) {  // converters: split the landed chunk
-          mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);
+          p.wait_landed(q);
           split_chunk<B>(p, q);
         } else {              // converters: gathering producer (wide blocks gather the input rows once per pass)
-          if (q >= kRing) mbar_wait(&p.slot_bar[q % kRing], ((q - kRing) / kRing) & 1);  // MMAs of chunk q-kRing released the slot
+          if (q >= kRing) p.wait_free(q - kRing);
           float* x0 = ps == 0 ? a.save_x0 : nullptr;
           store_chunk_api<DIM>(p, q, gv, x0, round_up(a.kin8, 16), tile, kc);
           p.conv_done(q);
@@ -356,12 +353,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
           if (x0 && kc == nk - 1 && (a.kin8 & 8)) zero_chunk_bpt<B>(x0, round_up(a.kin8, 16), tile, nk);
         }
       }
-      // ---- epilogue of this pass: all its MMAs have completed
-      mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-      fence_after_sync();
-      if (LOADS && warp == 0) {  // every slot is free: prefetch the next chunks under the epilogue
-        for (; loaded < q + kRing && loaded < total_chunks; ++loaded) load(loaded);
-      }
+      // ---- epilogue of this pass
+      p.wait_mmas(q - 1);
+      if (warp == 0) feed.refill_all(q, load);
       const int r = (warp & 3) * 32 + lane;
       for (int c4 = warp >> 2; c4 < (NS >> 2); c4 += 4) {
         float v[B][4];
@@ -370,15 +364,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
         tmem_wait_ld();
         f1_epilogue_group<DIM>(a, v, tile, (n0 >> 2) + c4, r, b1_s, sa_s, sb_s);
       }
-      // The next pass's first MMA overwrites these accumulators.  It is issued only after full_bar of the next chunk has
-      // collected an arrival from EVERY converter warp (conv_done), and each warp arrives after its own epilogue loads
-      // (tcgen05.wait::ld above) -- the issuer warp runs its epilogue part itself -- so the mbarrier orders the reuse.
-      fence_before_sync();
+      fence_before_sync();  // the next pass's first MMA overwrites these accumulators (tc_block.cuh: reuse rules)
     }
   }
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, tcols);
+  tmem_teardown(warp, tbase, tcols);
 }
 
 // =====================================================================================================================
@@ -408,42 +397,26 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kPipeBars);
   Pipe p;
   p.init(smem, bars, B * kPS);
-  const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
+  const int my_tiles = cta_tiles(a.tiles);
   const int total_chunks = my_tiles * nk;
-  auto tile_of = [&](int q) { return (int64_t)blockIdx.x + (int64_t)(q / nk) * gridDim.x; };
+  auto tile_of = [&](int q) { return cta_tile(q / nk); };
+  auto load = [&](int qq) { issue_chunk_load<B>(p, qq, a.p0, a.in_cp, tile_of(qq), qq % nk); };
+  ChunkFeed<BPT_IN> feed{p, total_chunks};
   // first chunks requested before the weights are staged (see tc_f1_kernel)
-  int q = 0, loaded = 0;
+  int q = 0;
   float4 gv[BPT_IN ? 1 : ApiItems<DIM>::N];
   GatherIdx<DIM> gi;
   if (!BPT_IN && warp != 0 && total_chunks > 0) {
     load_gather_idx<DIM>(a, tile_of(0) * kTile, gi);
     gather_chunk_api<DIM>(a, tile_of(0) * kTile, 0, gv, gi);
   }
-  if (BPT_IN && warp == 0) {
-    for (; loaded < kRing - 1 && loaded < total_chunks; ++loaded)
-      issue_chunk_load<B>(p, loaded, a.p0, a.in_cp, tile_of(loaded), loaded % nk);
-  }
+  if (warp == 0) feed.prime(load);
 
   const uint32_t bufcols = (uint32_t)B * Cp;  // <= 256 (host)
-  const uint32_t need = 2 * bufcols;
-  const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+  const uint32_t tcols = tmem_cols(2 * bufcols);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
-  // small parameters requested before the weights are staged (see tc_f2_kernel)
-  const float pf_b1 = (tid < C && a.has_b1) ? __ldg(a.b1 + tid) : 0.f;
-  const float pf_sa = tid < C * G ? __ldg(a.sa + tid) : 0.f;
-  const float pf_sb = tid < C * G ? __ldg(a.sb + tid) : 0.f;
-  stage_weight_images<DIM, false>(wimg, img, a.w1, C, a.cin, Cp, a.kin8);
-  if (tid < Cp) b1_s[tid] = pf_b1;
-  for (int i = tid + kThreads; i < Cp; i += kThreads) b1_s[i] = (i < C && a.has_b1) ? a.b1[i] : 0.f;
-  if (tid < Cp * G) { sa_s[tid] = pf_sa; sb_s[tid] = pf_sb; }
-  for (int i = tid + kThreads; i < Cp * G; i += kThreads) {
-    sa_s[i] = (i < C * G) ? a.sa[i] : 0.f;
-    sb_s[i] = (i < C * G) ? a.sb[i] : 0.f;
-  }
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
+  stage_f1_params<DIM>(a, b1_s, sa_s, sb_s, [&] { stage_weight_images<DIM, false>(wimg, img, a.w1, C, a.cin, Cp, a.kin8); });
+  prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t idesc = idesc_tf32(kTile, Cp, false, false);
   const int r = (warp & 3) * 32 + lane;
@@ -460,29 +433,25 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
   PendingEpilogue pend;
 
   for (int t = 0; t < my_tiles; ++t) {
-    const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
+    const int64_t tile = cta_tile(t);
     const uint32_t tb = tbase + (uint32_t)(t & 1) * bufcols;
     for (int kc = 0; kc < nk; ++kc, ++q) {
       if (warp == 0) {  // issuer
         TSTAMP(36);
         p.wait_full(q);
         TSTAMP(37);
-        if (BPT_IN && loaded == q + kRing - 1 && loaded < total_chunks) {
-          if (q >= 1) mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-          issue_chunk_load<B>(p, loaded, a.p0, a.in_cp, tile_of(loaded), loaded % nk);
-          ++loaded;
-        }
+        feed.refill(q, load);
         // buffer t & 1 was read by the epilogue of tile t-2: every epilogue warp finished it before its conv_done of
         // this tile's first chunk (full_bar observed above), so the first MMA may overwrite it
         issue_chunk_mma<DIM>(p, q, tb, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
         TSTAMP(38);
       } else {
         if (BPT_IN) {
-          mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);
+          p.wait_landed(q);
           split_chunk<B>(p, q);
         } else {
           TSTAMP(30);
-          if (q >= kRing) mbar_wait(&p.slot_bar[q % kRing], ((q - kRing) / kRing) & 1);
+          if (q >= kRing) p.wait_free(q - kRing);
           TSTAMP(31);
           store_chunk_api<DIM>(p, q, gv, a.save_x0, round_up(a.kin8, 16), tile, kc);
           TSTAMP(32);
@@ -503,9 +472,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
     pend.start(warp, tile, q - 1, tb);
   }
   pend.drain(p, n_c4, epilogue_unit);
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, tcols);
+  tmem_teardown(warp, tbase, tcols);
 }
 
 // =====================================================================================================================
@@ -542,26 +509,23 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kPipeBars);
   Pipe p;
   p.init(smem, bars, half);
-  const int my_tiles = (a.tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
+  const int my_tiles = cta_tiles(a.tiles);
   const int per_tile = npass * nk;
-  const int total_chunks = my_tiles * per_tile;
-  auto tile_of = [&](int q) { return (int64_t)blockIdx.x + (int64_t)(q / per_tile) * gridDim.x; };
   auto load = [&](int qq) {
+    const int64_t tile = cta_tile(qq / per_tile);
     if constexpr (ST) {
       const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(a.wimg2) + (size_t)(qq % per_tile) * wunit;
-      issue_chunk_load_w<B>(p, qq, a.y2, Cp, tile_of(qq), qq % nk, wsrc, wunit);
+      issue_chunk_load_w<B>(p, qq, a.y2, Cp, tile, qq % nk, wsrc, wunit);
     } else {
-      issue_chunk_load<B>(p, qq, a.y2, Cp, tile_of(qq), qq % nk);
+      issue_chunk_load<B>(p, qq, a.y2, Cp, tile, qq % nk);
     }
   };
-  int q = 0, loaded = 0;
-  if (warp == 0) {  // first chunks requested before the weights are staged (see tc_f1_kernel)
-    for (; loaded < kRing - 1 && loaded < total_chunks; ++loaded) load(loaded);
-  }
+  ChunkFeed<> feed{p, my_tiles * per_tile};
+  int q = 0;
+  if (warp == 0) feed.prime(load);
 
   TSTAMP(3);
-  const uint32_t need = 2 * B * NS;
-  const uint32_t tcols = need <= 32 ? 32 : need <= 64 ? 64 : need <= 128 ? 128 : need <= 256 ? 256 : 512;
+  const uint32_t tcols = tmem_cols(2 * B * NS);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   // the first elements of the small per-channel parameters are requested before the weights are staged (one exposed
   // latency for the whole prologue instead of one per loop)
@@ -585,10 +549,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
     bl_s[i] = (i < C) ? a.bl[i] : 0.f;
     la_s[i] = (i < C) ? a.la[i] : 0.f;
   }
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
+  prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t idesc = idesc_tf32(kTile, 2 * NS, false, false);
   const uint32_t col_r = 0, col_l = NS, bcols = 2 * NS;  // column of (blade b, channel c of the pass): b * bcols + col_{r,l} + c
@@ -597,7 +558,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
 
   TSTAMP(1);
   for (int t = 0; t < my_tiles; ++t) {
-    const int64_t tile = (int64_t)blockIdx.x + (int64_t)t * gridDim.x;
+    const int64_t tile = cta_tile(t);
     const int64_t row0 = tile * kTile;
     const int r = lane_base + lane;
     const bool row_ok = row0 + r < a.rows;
@@ -609,17 +570,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
         if (warp == 0) {  // issuer
           p.wait_full(q);
           TSTAMP(14);
-          if (loaded == q + kRing - 1 && loaded < total_chunks) {
-            if (q >= 1) mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-            load(loaded);
-            ++loaded;
-          }
+          feed.refill(q, load);
           TSTAMP(16);
           if constexpr (ST) issue_chunk_mma<DIM>(p, q, tbase, bcols, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, bcols, 0, 0, idesc);
           else issue_chunk_mma<DIM>(p, q, tbase, bcols, kc > 0, wimg, img, 0, 1, 0, bcols, kc, 0, idesc);
           TSTAMP(15);
         } else {          // converters
-          mbar_wait(&p.load_bar[q % kRing], (q / kRing) & 1);
+          p.wait_landed(q);
           TSTAMP(11);
           split_chunk<B>(p, q);
           TSTAMP(13);
@@ -632,12 +589,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
 #pragma unroll
         for (int b = 0; b < B; ++b) y2v[b] = *reinterpret_cast<const float4*>(a.y2 + bpt_off(B, Cp, tile, b, (n0 >> 2) + (warp >> 2), r));
       }
-      mbar_wait(&p.slot_bar[(q - 1) % kRing], ((q - 1) / kRing) & 1);
-      fence_after_sync();
+      p.wait_mmas(q - 1);
       TSTAMP(21);
-      if (warp == 0) {
-        for (; loaded < q + kRing && loaded < total_chunks; ++loaded) load(loaded);
-      }
+      if (warp == 0) feed.refill_all(q, load);
       // ---- pass 1: per channel normalisation + weighted geometric product; o -> TMEM over xl (ST: -> save_o only)
       for (int c4 = warp >> 2; c4 < (NS >> 2); c4 += 4) {
         const int gc4 = (n0 >> 2) + c4;
@@ -762,9 +716,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
     fence_before_sync();
     TSTAMP(24);
   }
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, tcols);
+  tmem_teardown(warp, tbase, tcols);
   TSTAMP(5);
 }
 
@@ -773,8 +725,6 @@ long long*& debug_buffer() {
   static long long* p = nullptr;
   return p;
 }
-
-constexpr size_t kSmemMax = 227 * 1024;
 
 // How the two forward kernels of a block of this shape run: weights resident in shared memory, or -- wide blocks --
 // streamed with the K chunks in passes of ns1 / ns2 output channels (tc_block.cuh).
@@ -828,27 +778,12 @@ template <int DIM>
 bool fwd_supported(int cin, int c) { return fwd_plan<DIM>(cin, c).ok; }
 
 inline int64_t align32f(int64_t floats) { return (floats + 31) / 32 * 32; }
-// CSMPN_TC_OVERLAP=0 selects the plain kernels (epilogue after the K loop); read per call so a test can compare both
-inline bool overlap_enabled() {
-  const char* e = getenv("CSMPN_TC_OVERLAP");
-  return !(e && e[0] == '0');
-}
 
 template <int DIM>
 int64_t fwd_ws_bytes(const csmpn_block_desc& d) {
   const FwdPlan p = fwd_plan<DIM>(d.c0 + d.c1 + d.c2, d.c);
   if (!p.ok) return -1;
   return (align32f(p.w1_floats) + align32f(p.w2_floats)) * 4;
-}
-
-template <int DIM>
-int launch_weight_images(const WPrepArgs& w, int64_t floats, cudaStream_t stream) {
-  const int threads = 256;
-  int64_t blocks = (floats + threads - 1) / threads;
-  if (blocks > 4096) blocks = 4096;
-  tc_weight_images_kernel<DIM><<<(unsigned)blocks, threads, 0, stream>>>(w);
-  CSMPN_LAUNCH_CHECK("tc_weight_images_kernel");
-  return CSMPN_OK;
 }
 
 template <int DIM>
@@ -910,8 +845,7 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   const bool dbg_f1 = dbg_k && dbg_k[0] == 'f' && dbg_k[1] == '1';
   a.dbg = dbg_f1 ? dbg_buf : nullptr;
   if (mask & 1) {
-    // resident weights and accumulators of at most half of TMEM: the overlapped-epilogue kernel (CSMPN_TC_OVERLAP=0: plain)
-    const bool overlap = !p.st1 && 2 * B * a.Cp <= 512 && overlap_enabled();
+    const bool overlap = !p.st1 && use_overlapped_epilogue(B, a.Cp);
     int rc = overlap ? (a.in_bpt ? run(tc_f1db_kernel<DIM, true>, p.s1) : run(tc_f1db_kernel<DIM, false>, p.s1))
              : a.in_bpt ? (p.st1 ? run(tc_f1_kernel<DIM, true, true>, p.s1) : run(tc_f1_kernel<DIM, true, false>, p.s1))
                         : (p.st1 ? run(tc_f1_kernel<DIM, false, true>, p.s1) : run(tc_f1_kernel<DIM, false, false>, p.s1));
