@@ -1050,6 +1050,7 @@ inline int check_desc(int dim, const csmpn_block_desc* d) {
   if (d->pair_attr && (d->mode != 1 || (d->c1 & 1))) return CSMPN_ERR_BAD_ARG;
   if (!d->w1 || !d->sa || !d->sb || !d->wr || !d->na || !d->wl || !d->bl || !d->wp || !d->la) return CSMPN_ERR_BAD_ARG;
   if (d->has_b1 && !d->b1) return CSMPN_ERR_BAD_ARG;
+  if (d->tf32 != 0 && d->tf32 != 1) return CSMPN_ERR_BAD_ARG;
   return CSMPN_OK;
 }
 

@@ -80,10 +80,17 @@ __device__ __forceinline__ float mv_sumsq(const float* x) {
   return Q;
 }
 
-// Stage [c_out, c_in, G] weights (global, reference layout) as 2*G operand images each in shared memory:
+// Numeric mode of the GEMM kernels: TERMS = 3 is the error-compensated split (hi*hi + hi*lo + lo*hi, fp32 accuracy, the
+// default); TERMS = 1 is single-pass TF32 (csmpn_block_desc.tf32): every operand rounded to nearest TF32 once, one MMA
+// per product, no `lo` operands.  Weight images per grade: hi and lo, or the rounded weight alone.
+__host__ __device__ constexpr int n_images(int terms) { return terms == 1 ? 1 : 2; }
+
+// Stage [c_out, c_in, G] weights (global, reference layout) as NI*G operand images each in shared memory (NI =
+// n_images(TERMS)):
 //   image (g, hl) = plane with R = rows_p rows;  TRANS == false: row = output channel, column = input channel
 //                                                TRANS == true : row = input channel,  column = output channel
-// hl = 0: TF32-exact high part, hl = 1: remainder.  Rows/columns beyond the real sizes are zero.
+// TERMS = 3: hl = 0: TF32-exact high part, hl = 1: remainder.  TERMS = 1: the weight rounded to nearest TF32.
+// Rows/columns beyond the real sizes are zero.
 // A job = one weight: its image set (img0), its first plane row (two weights can share one image set: rows [0, n) and
 // [n, 2n)).  [zero_base, zero_base + zero_bytes) -- all image sets of the call, contiguous -- is cleared first.
 // The prologue of every GEMM kernel runs this once per CTA, and a one-tile-per-CTA launch (every per-simplex block) pays
@@ -99,10 +106,11 @@ struct WJob {
 // so the 32 stores of one (grade, hi/lo) image are 128 contiguous bytes (conflict-free) and a lane's G grades of one
 // (output, input) pair are one 16-byte load when G == 4.  Units of up to two weights are walked in one flat index space,
 // four units per warp in flight.
-template <int DIM, bool TRANS, int NJ>
+template <int DIM, bool TRANS, int NJ, int TERMS = 3>
 __device__ __forceinline__ void stage_weight_jobs(const WJob (&j)[NJ], int njobs, uint32_t img_bytes, int rows_p, int cols_p,
                                                   uint8_t* zero_base, uint32_t zero_bytes) {
   static_assert(NJ == 1 || NJ == 2, "one or two weights per call");
+  static_assert(TERMS == 1 || TERMS == 3, "split or single-pass products");
   constexpr int G = Alg<DIM>::G, U = 4;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   const int rl = lane >> 2, cl = lane & 3;
@@ -151,9 +159,13 @@ __device__ __forceinline__ void stage_weight_jobs(const WJob (&j)[NJ], int njobs
     uint8_t* dst = (sj ? j1.img0 : j0.img0) + plane_off(rows_p, r, col);
 #pragma unroll
     for (int g = 0; g < G; ++g) {
-      const float hi = tf32_hi(v[g]);
-      *reinterpret_cast<float*>(dst + (size_t)(g * 2 + 0) * img_bytes) = hi;
-      *reinterpret_cast<float*>(dst + (size_t)(g * 2 + 1) * img_bytes) = v[g] - hi;
+      if constexpr (TERMS == 1) {
+        *reinterpret_cast<float*>(dst + (size_t)g * img_bytes) = tf32_rna(v[g]);
+      } else {
+        const float hi = tf32_hi(v[g]);
+        *reinterpret_cast<float*>(dst + (size_t)(g * 2 + 0) * img_bytes) = hi;
+        *reinterpret_cast<float*>(dst + (size_t)(g * 2 + 1) * img_bytes) = v[g] - hi;
+      }
     }
   };
   float x[U][G];
@@ -181,11 +193,12 @@ __device__ __forceinline__ void stage_weight_jobs(const WJob (&j)[NJ], int njobs
   }
 }
 // one weight into its own image set (cleared first)
-template <int DIM, bool TRANS>
+template <int DIM, bool TRANS, int TERMS = 3>
 __device__ __forceinline__ void stage_weight_images(uint8_t* img0, uint32_t img_bytes, const float* __restrict__ w, int c_out,
                                                     int c_in, int rows_p, int cols_p) {
   const WJob j[1] = {{img0, w, c_out, c_in, 0}};
-  stage_weight_jobs<DIM, TRANS, 1>(j, 1, img_bytes, rows_p, cols_p, img0, (uint32_t)Alg<DIM>::G * 2u * img_bytes);
+  stage_weight_jobs<DIM, TRANS, 1, TERMS>(j, 1, img_bytes, rows_p, cols_p, img0,
+                                          (uint32_t)Alg<DIM>::G * (uint32_t)n_images(TERMS) * img_bytes);
 }
 
 // A-operand descriptors of blade b in a chunk buffer half
@@ -217,11 +230,19 @@ __device__ __forceinline__ void tmem_teardown(int warp, uint32_t tbase, uint32_t
 }
 
 constexpr size_t kSmemMax = 227 * 1024;  // dynamic shared memory of one CTA
+// The ring-fed kernels are persistent with one CTA per SM (grid = min(tiles, SMs)) and size their TMEM allocation for an SM
+// of their own.  Several single-pass TF32 instantiations use <= 64 registers, so registers alone would let two 512-thread
+// CTAs share an SM (and wait on each other's TMEM) while other SMs idle: their smaller shared-memory requests are raised
+// to more than half of the SM's 228 KB (1 KB reserved per CTA), which keeps a second CTA off the SM.
+constexpr size_t kOneCtaPerSm = 116 * 1024;
+__host__ inline size_t one_cta_per_sm(size_t smem) { return smem < kOneCtaPerSm ? kOneCtaPerSm : smem; }
 
 // ---- K-chunk pipeline of the ring-fed kernels (tc_f1, tc_f1db, tc_f2, tc_bgemm, tc_bgemmdb) ----------------------------
 // A chunk = 8 channels of all blades of a 128-row tile.  Chunk q lands (bulk copies) in raw slot q % kRing; the split
 // pass turns the slot into the TF32-exact high parts in place and writes the remainders to the single `lo` buffer;
 // the MMAs of the chunk read both.  Loads run kRing-1 chunks ahead of the MMAs (two chunks = 64 KB per SM in flight).
+// Single-pass TF32 (TERMS = 1): the conversion pass rounds the slot to nearest TF32 in place and the MMAs read the slot
+// alone; `lo` and lo_bar are left unused.
 //
 // Roles during the K loop: warp 0 is the ISSUER (bulk copies + MMAs, nothing else); warps 1..15 are CONVERTERS (split
 // pass / gathering producer).  They are decoupled by mbarriers only -- no CTA-wide barrier inside the K loop -- so the
@@ -229,12 +250,14 @@ constexpr size_t kSmemMax = 227 * 1024;  // dynamic shared memory of one CTA
 // epilogue.
 // tcgen05.mma kind::tf32 reads fp32 operands and ignores the low 13 mantissa bits (truncation, verified on B200 by the
 // 1e-5 parity tests, which a round-to-nearest read would fail by 2^-11): the raw chunk already IS the high operand, so the
-// split pass only has to produce the remainders.
+// split pass only has to produce the remainders.  For the same reason single-pass TF32 rounds (cvt.rna) explicitly: raw
+// fp32 operands would bias every product toward zero.
 //
 // Reuse rules (nothing but these mbarriers orders the K loop):
 // * Raw slot q % kRing is overwritten by chunk q + kRing only once slot_bar has seen the MMAs of chunk q complete:
 //   ChunkFeed::refill / refill_all for bulk copies, Pipe::wait_free(q - kRing) for the gathering producer's stores.
 // * `lo` is rewritten for chunk q once lo_bar has seen the MMAs of chunk q-1 complete (split_chunk, store_chunk_api).
+//   TERMS = 1 has no `lo`: the rounding pass writes only the raw slot, which the first rule already protects.
 // * An accumulator is read (tcgen05.ld) only after wait_mmas of the last chunk that wrote it.  It is overwritten by the
 //   first MMA of a later pass or tile, which the issuer issues only after wait_full of that chunk; every converter warp
 //   arrives on full_bar (conv_done) after its own epilogue loads (tcgen05.wait::ld), and the issuer warp runs its part
@@ -360,9 +383,12 @@ struct PendingEpilogue {
 // are streamed WITH the activations: a raw slot holds the activation chunk followed by the "weight unit" of the same K
 // chunk -- for every grade the hi and lo images of [R output rows x 8 input channels] (plane layout with R rows) --
 // brought in by ONE more bulk copy from a pre-split image buffer in global memory (tc_weight_images_kernel), laid out
-// unit after unit in the order the kernel walks them: [pass][K chunk][grade][hi | lo][2][R][4] floats.
+// unit after unit in the order the kernel walks them: [pass][K chunk][grade][hi | lo][2][R][4] floats.  Single-pass
+// TF32: [pass][K chunk][grade][2][R][4], the rounded weight alone (nimg = 1), half the bytes.
 template <int DIM>
-__host__ __device__ constexpr uint32_t wunit_bytes(int rows) { return (uint32_t)Alg<DIM>::G * 2u * (uint32_t)rows * 32u; }
+__host__ __device__ constexpr uint32_t wunit_bytes(int rows, int nimg = 2) {
+  return (uint32_t)Alg<DIM>::G * (uint32_t)nimg * (uint32_t)rows * 32u;
+}
 
 // bulk copies of chunk q: the activation planes (bpt != nullptr) and the weight unit; called by ALL lanes of one warp
 template <int B>
@@ -386,16 +412,16 @@ struct WPrepArgs {
   int stack, trans, n_real, k_real0, k_real1, np, npass, nk0, nk1;
   float* out;
 };
-template <int DIM>
+template <int DIM, int TERMS = 3>
 __global__ void tc_weight_images_kernel(WPrepArgs a) {
-  constexpr int G = Alg<DIM>::G;
+  constexpr int G = Alg<DIM>::G, NI = n_images(TERMS);
   const int R = a.stack ? 2 * a.np : a.np;
   const int nk = a.nk0 + (a.stack ? 0 : a.nk1);
-  const int64_t total = (int64_t)a.npass * nk * G * 2 * R * 8;
+  const int64_t total = (int64_t)a.npass * nk * G * NI * R * 8;
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
-    const int c = (int)(e & 3), r = (int)((e >> 2) % R), cu = (int)((e / (4 * R)) & 1), hl = (int)((e / (8 * R)) & 1);
-    const int g = (int)((e / (16 * R)) % G);
-    const int u = (int)(e / ((int64_t)16 * R * G)), ps = u / nk, kc = u % nk;
+    const int c = (int)(e & 3), r = (int)((e >> 2) % R), cu = (int)((e / (4 * R)) & 1), hl = NI == 2 ? (int)((e / (8 * R)) & 1) : 0;
+    const int g = (int)((e / (8 * NI * R)) % G);
+    const int u = (int)(e / ((int64_t)8 * NI * R * G)), ps = u / nk, kc = u % nk;
     const int second_k = (!a.stack && kc >= a.nk0) ? 1 : 0;
     const int k = (second_k ? kc - a.nk0 : kc) * 8 + cu * 4 + c;
     const int k_real = second_k ? a.k_real1 : a.k_real0;
@@ -403,19 +429,23 @@ __global__ void tc_weight_images_kernel(WPrepArgs a) {
     const int n = ps * a.np + (a.stack ? r % a.np : r);
     float x = 0.f;
     if (w && n < a.n_real && k < k_real) x = a.trans ? w[((size_t)k * a.n_real + n) * G + g] : w[((size_t)n * k_real + k) * G + g];
-    const float hi = tf32_hi(x);
-    a.out[e] = hl ? x - hi : hi;
+    if constexpr (TERMS == 1) {
+      a.out[e] = tf32_rna(x);
+    } else {
+      const float hi = tf32_hi(x);
+      a.out[e] = hl ? x - hi : hi;
+    }
   }
 }
 template <int DIM>
-__host__ inline int64_t weight_image_floats(int stack, int np, int npass, int nk_total) {
-  return (int64_t)npass * nk_total * Alg<DIM>::G * 2 * (stack ? 2 * np : np) * 8;
+__host__ inline int64_t weight_image_floats(int stack, int np, int npass, int nk_total, int nimg = 2) {
+  return (int64_t)npass * nk_total * Alg<DIM>::G * nimg * (stack ? 2 * np : np) * 8;
 }
-template <int DIM>
+template <int DIM, int TERMS = 3>
 __host__ int launch_weight_images(const WPrepArgs& w, int64_t floats, cudaStream_t stream) {
   int64_t blocks = (floats + 255) / 256;
   if (blocks > 4096) blocks = 4096;
-  tc_weight_images_kernel<DIM><<<(unsigned)blocks, 256, 0, stream>>>(w);
+  tc_weight_images_kernel<DIM, TERMS><<<(unsigned)blocks, 256, 0, stream>>>(w);
   CSMPN_LAUNCH_CHECK("tc_weight_images_kernel");
   return CSMPN_OK;
 }
@@ -440,12 +470,26 @@ __device__ __forceinline__ void issue_chunk_load(const Pipe& p, int q, const flo
 // split pass over the landed chunk q (CONVERTER warps only): high parts in place, remainders to `lo`.  The remainders
 // wait in registers until the MMAs of chunk q-1 (the previous readers of `lo`) have completed, so reading the chunk,
 // splitting it and storing the high parts overlap those MMAs.  Ends with conv_done(q).
-template <int B>
+// TERMS = 1: rounds the chunk to nearest TF32 in place; no `lo`, no lo_bar wait.
+template <int B, int TERMS = 3>
 __device__ __forceinline__ void split_chunk(const Pipe& p, int q) {
   uint8_t* hi = p.slot(q);
   constexpr int TOT = B * 2 * kTile;
   constexpr int N = (TOT + kConv - 1) / kConv;
   const int ct = (int)threadIdx.x - 32;
+  if constexpr (TERMS == 1) {
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+      const int it = ct + i * kConv;
+      if (it < TOT) {
+        const int r = it & (kTile - 1), kh = (it >> 7) & 1, b = it >> 8;
+        float4* x = reinterpret_cast<float4*>(hi + b * kPS + kh * kKH + r * 16);
+        *x = tf32_rna4(*x);
+      }
+    }
+    p.conv_done(q);
+    return;
+  }
   float4 l[N];
 #pragma unroll
   for (int i = 0; i < N; ++i) {
@@ -472,9 +516,10 @@ __device__ __forceinline__ void split_chunk(const Pipe& p, int q) {
 }
 // the MMAs of chunk q (called by every lane of one converged warp; an elected lane issues).  Weight set s: images at wimg0 + s*set_bytes, image (g, hi/lo) = 2g / 2g+1, plane
 // rows = w_rows, K step ks, first output row n0; accumulator of (set s, blade b) at column (s*B + b)*ncols.
+// TERMS = 1: image g = the rounded weight of grade g; one MMA per (set, blade) on the rounded chunk, one commit.
 // The issuing thread's instruction stream is serial, so descriptors are formed by adding small 16-byte-unit offsets to
 // bases computed once per chunk, and the loops are fully unrolled.
-template <int DIM>
+template <int DIM, int TERMS = 3>
 __device__ __forceinline__ void issue_chunk_mma(const Pipe& p, int q, uint32_t tbase, uint32_t ncols, bool accumulate,
                                                 const uint8_t* wimg0, uint32_t img_bytes, int s0, int nsets, uint32_t set_bytes,
                                                 uint32_t w_rows, int ks, int n0, uint32_t idesc) {
@@ -485,6 +530,19 @@ __device__ __forceinline__ void issue_chunk_mma(const Pipe& p, int q, uint32_t t
                                 w_rows * 16u, 128u);
   const uint64_t img16 = img_bytes >> 4, set16 = set_bytes >> 4;
   constexpr uint64_t ps16 = kPS >> 4;
+  if constexpr (TERMS == 1) {
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      if (s < nsets) {
+#pragma unroll
+        for (int b = 0; b < B; ++b)
+          mma_tf32_w(tbase + (uint32_t)(s * B + b) * ncols, a_hi + b * ps16, w0 + s * set16 + A::grade_of(b) * img16, idesc,
+                     accumulate);
+      }
+    }
+    mma_commit_w(&p.slot_bar[q % kRing]);
+    return;
+  }
 #pragma unroll
   for (int s = 0; s < 2; ++s) {
     if (s < nsets) {

@@ -411,17 +411,18 @@ __device__ __forceinline__ void store_gemm_group(const GemmArgs& a, const float 
   }
 }
 
-template <int DIM, bool ST>
+// TERMS: numeric mode (tc_block.cuh, n_images)
+template <int DIM, bool ST, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_constant__ GemmArgs a) {
   using A = Alg<DIM>;
-  constexpr int B = A::B, G = A::G;
+  constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int nmax = ST ? a.np : (512 / B) / 16 * 16;            // output channels per pass (TMEM columns / blades)
-  const uint32_t wunit = ST ? wunit_bytes<DIM>(nmax) : 0u;
+  const uint32_t wunit = ST ? wunit_bytes<DIM>(nmax, NI) : 0u;
   const uint32_t half = B * kPS + wunit;
   const uint32_t img = ST ? (uint32_t)nmax * 32u : (uint32_t)a.n16 * a.kmax * 4;
-  const uint32_t set_bytes = ST ? 0u : G * 2 * img;
+  const uint32_t set_bytes = ST ? 0u : G * NI * img;
   uint8_t* wimg = smem + (size_t)kRing * half + B * kPS;
   const int nsets = a.src[1] ? 2 : 1;
   uint64_t* bars = reinterpret_cast<uint64_t*>(wimg + (size_t)nsets * set_bytes);
@@ -451,7 +452,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   if (!ST) {
     const WJob wj[2] = {{wimg, a.w[0], a.wk[0], a.wn, 0}, {wimg + set_bytes, a.w[nsets - 1], a.wk[nsets - 1], a.wn, 0}};
-    stage_weight_jobs<DIM, true, 2>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
+    stage_weight_jobs<DIM, true, 2, TERMS>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
   }
   prologue_sync();
   const uint32_t tbase = *tmem_slot;
@@ -469,14 +470,14 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
           feed.refill(q, load);
           if constexpr (ST) {
             p.wait_landed(q);  // the weight unit of this chunk
-            issue_chunk_mma<DIM>(p, q, tbase, Np, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, nmax, 0, 0, idesc);
+            issue_chunk_mma<DIM, TERMS>(p, q, tbase, Np, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, nmax, 0, 0, idesc);
           } else {
             const int s = kc < a.nk[0] ? 0 : 1;
-            issue_chunk_mma<DIM>(p, q, tbase, Np, kc > 0, wimg, img, s, 1, set_bytes, a.n16, s ? kc - a.nk[0] : kc, n0, idesc);
+            issue_chunk_mma<DIM, TERMS>(p, q, tbase, Np, kc > 0, wimg, img, s, 1, set_bytes, a.n16, s ? kc - a.nk[0] : kc, n0, idesc);
           }
         } else {          // converters
           p.wait_landed(q);
-          split_chunk<B>(p, q);
+          split_chunk<B, TERMS>(p, q);
         }
       }
       // ---- epilogue of this pass: output channels [n0, n0 + Np).  The addend rows of the first channel group are
@@ -518,14 +519,14 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemm_kernel(const __grid_cons
 // alternate between two TMEM buffers by tile and the epilogue of tile t-1 runs as channel-group units between the chunks
 // of tile t's K loop (PendingEpilogue, see tc_f1db_kernel).  Warp 0 issues; warps 1-15 convert; warps 4-15 own the
 // epilogue.  Bit-identical outputs.
-template <int DIM>
+template <int DIM, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_constant__ GemmArgs a) {
   using A = Alg<DIM>;
-  constexpr int B = A::B, G = A::G;
+  constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const uint32_t img = (uint32_t)a.n16 * a.kmax * 4;
-  const uint32_t set_bytes = G * 2 * img;
+  const uint32_t set_bytes = G * NI * img;
   uint8_t* wimg = smem + (kRing + 1) * B * kPS;
   const int nsets = a.src[1] ? 2 : 1;
   uint64_t* bars = reinterpret_cast<uint64_t*>(wimg + (size_t)nsets * set_bytes);
@@ -548,7 +549,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_co
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   {
     const WJob wj[2] = {{wimg, a.w[0], a.wk[0], a.wn, 0}, {wimg + set_bytes, a.w[nsets - 1], a.wk[nsets - 1], a.wn, 0}};
-    stage_weight_jobs<DIM, true, 2>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
+    stage_weight_jobs<DIM, true, 2, TERMS>(wj, nsets, img, a.n16, a.kmax, wimg, (uint32_t)nsets * set_bytes);
   }
   prologue_sync();
   const uint32_t tbase = *tmem_slot;
@@ -586,10 +587,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bgemmdb_kernel(const __grid_co
         p.wait_full(q);
         feed.refill(q, load);
         const int s = kc < a.nk[0] ? 0 : 1;
-        issue_chunk_mma<DIM>(p, q, tb, Np, kc > 0, wimg, img, s, 1, set_bytes, a.n16, s ? kc - a.nk[0] : kc, 0, idesc);
+        issue_chunk_mma<DIM, TERMS>(p, q, tb, Np, kc > 0, wimg, img, s, 1, set_bytes, a.n16, s ? kc - a.nk[0] : kc, 0, idesc);
       } else {
         p.wait_landed(q);
-        split_chunk<B>(p, q);
+        split_chunk<B, TERMS>(p, q);
         pend.step(p, n_c4, epilogue_unit);
       }
     }
@@ -635,11 +636,13 @@ long long*& debug_buffer();  // tc_block_fwd.cu
 // copies into one of kDwLand landing slots (the next unit loads while the current one is converted); a conversion pass
 // splits a step into hi / lo and re-lays it out as [row][32 channels] operand groups (SWIZZLE_128B_BASE32B),
 // double-buffered so that the conversion of step s+1 overlaps the MMAs of step s.
+// TERMS = 1 (single-pass TF32): the conversion writes only the operands rounded to nearest TF32 (the hi groups; the lo
+// groups keep the zeros of the prologue) and the issuer runs one MMA per K step (see `merged` for M = 64).
 constexpr int kDwRows = 64;
 constexpr int kDwLand = 2;                 // landing slots; a slot holds one (tile, blade) = both row halves = two steps
 constexpr uint32_t kLand = kTile * 16;     // landing stride of one 4-channel column: [128 rows][4 channels], as in global memory
 
-template <int DIM, bool TL>
+template <int DIM, bool TL, int TERMS = 3>
 __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G;
@@ -676,8 +679,11 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
   // shape 128 x (2 * 32 gb) x 8 multiplies [A_hi; A_lo] by [B_hi | B_lo] and yields all four split products at once
   // (lanes 0-63: A_hi rows, lanes 64-127: A_lo rows; first column half: B_hi, second: B_lo) instead of three M = 64
   // instructions.  The epilogue adds the two column halves and writes the two lane halves as two partials.
+  // TERMS = 1 keeps the M = 128 instruction, now 128 x (32 gb) x 8 on [A; 0] x B: lanes 64-127 multiply the zero lo
+  // groups and their partial is zero.  The M = 64 shape would read half the A rows, but its TMEM accumulator layout
+  // differs from the M = 128 one every other kernel here uses; one instruction per K step either way.
   const bool merged = a.M == 64;
-  const uint32_t ncol = merged ? 2u * gb * 32u : (uint32_t)a.cpb;  // accumulator columns per grade
+  const uint32_t ncol = merged ? (TERMS == 1 ? 1u : 2u) * gb * 32u : (uint32_t)a.cpb;  // accumulator columns per grade
   const uint32_t tcols = tmem_cols((uint32_t)G * ncol);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   prologue_sync();
@@ -716,7 +722,7 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
       const uint64_t b_hi = desc_mn32b(smem_addr(op_b), grp, 0), b_lo = b_hi + ((uint64_t)gb * grp >> 4);
       const uint32_t dcol = tbase + (uint32_t)g * ncol;
       const uint32_t acc = (grade_used >> g) & 1;
-      if (merged) {
+      if (merged || TERMS == 1) {
 #pragma unroll
         for (int ks = 0; ks < kDwRows / 8; ++ks) mma_tf32_w(dcol, a_hi + ks * 64, b_hi + ks * 64, idesc, ks == 0 ? acc : 1u);
       } else {
@@ -755,15 +761,19 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
         const int swap = g8 >> 3, r = ((g8 & 7) << 3) + q;
         const int u = 2 * pr + ((q >> 2) ^ swap);
         const float4 x = *reinterpret_cast<const float4*>(src + (uint32_t)u * kLand + r * 16);
-        float4 h, l;
-        split4(x, h, l);
         const bool isb = u >= na4;
         const int cc = (isb ? u - na4 : u) * 4;  // channel inside its operand
         uint8_t* base = isb ? op_b : op_a;
         const int ng = isb ? gb : ga;
         const uint32_t off = (uint32_t)(cc >> 5) * grp + mn32b_off(r, cc & 31);
-        *reinterpret_cast<float4*>(base + off) = h;
-        *reinterpret_cast<float4*>(base + (size_t)ng * grp + off) = l;
+        if constexpr (TERMS == 1) {
+          *reinterpret_cast<float4*>(base + off) = tf32_rna4(x);
+        } else {
+          float4 h, l;
+          split4(x, h, l);
+          *reinterpret_cast<float4*>(base + off) = h;
+          *reinterpret_cast<float4*>(base + (size_t)ng * grp + off) = l;
+        }
       }
       fence_async_smem();
       __syncwarp();
@@ -786,7 +796,7 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
         float v[4] = {0.f, 0.f, 0.f, 0.f}, w[4] = {0.f, 0.f, 0.f, 0.f};
         if (used) {
           tmem_ld4(tmem_at(tbase, warp * 32, g * ncol + n), v);
-          tmem_ld4(tmem_at(tbase, warp * 32, g * ncol + gb * 32 + n), w);
+          if (TERMS == 3) tmem_ld4(tmem_at(tbase, warp * 32, g * ncol + gb * 32 + n), w);
           tmem_wait_ld();
         }
         *reinterpret_cast<float4*>(out + ((size_t)g * 64 + m) * a.cpb + n) = make_float4(v[0] + w[0], v[1] + w[1], v[2] + w[2], v[3] + w[3]);
@@ -868,9 +878,10 @@ __global__ void __launch_bounds__(256) tc_final_kernel(FinalJobs jobs) {
 // =====================================================================================================================
 // host side
 template <int DIM>
-size_t gemm_smem(int nsets, int n16, int kmax) {
+size_t gemm_smem(int nsets, int n16, int kmax, int nimg = 2) {
   constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G;
-  return (size_t)(kRing + 1) * B * kPS + (size_t)nsets * G * 2 * n16 * kmax * 4 + 128;
+  const size_t s = (size_t)(kRing + 1) * B * kPS + (size_t)nsets * G * nimg * n16 * kmax * 4 + 128;
+  return nimg == 2 ? s : one_cta_per_sm(s);
 }
 template <int DIM>
 size_t dw_smem(int M, int na4, int cpb) {
@@ -894,11 +905,14 @@ struct BwdPlan {
 };
 constexpr int kSlabA = 64, kSlabB = 32;  // wide weight-gradient launches: A rows (merged M = 64) x B columns
 template <int DIM>
-size_t gemm_smem_streamed(int np) {
+size_t gemm_smem_streamed(int np, int nimg = 2) {
   constexpr int B = Alg<DIM>::B;
-  return (size_t)kRing * (B * kPS + wunit_bytes<DIM>(np)) + (size_t)B * kPS + 128;
+  const size_t s = (size_t)kRing * (B * kPS + wunit_bytes<DIM>(np, nimg)) + (size_t)B * kPS + 128;
+  return nimg == 2 ? s : one_cta_per_sm(s);
 }
 
+// The plan is chosen for the default (split) weight images, so both numeric modes run a shape the same way;
+// single-pass TF32 (d.tf32) only halves the streamed image buffers.
 template <int DIM>
 int make_bwd_plan(const csmpn_block_desc& d, BwdPlan* p) {
   constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G, P = Alg<DIM>::P;
@@ -936,8 +950,9 @@ int make_bwd_plan(const csmpn_block_desc& d, BwdPlan* p) {
     p->n_dwa = 2 * sa * ((p->Cp + kSlabB - 1) / kSlabB);
     p->n_dwb = sa * ((p->n16 + kSlabB - 1) / kSlabB);
     p->dw_part = (size_t)p->grid_dw * 2 * G * kSlabA * kSlabB;
-    p->img_dy2 = weight_image_floats<DIM>(0, p->np, (p->Cp + p->np - 1) / p->np, 2 * (p->Cp / 8));
-    p->img_gx = weight_image_floats<DIM>(0, p->np, (p->n16 + p->np - 1) / p->np, p->Cp / 8);
+    const int nimg = d.tf32 ? 1 : 2;
+    p->img_dy2 = weight_image_floats<DIM>(0, p->np, (p->Cp + p->np - 1) / p->np, 2 * (p->Cp / 8), nimg);
+    p->img_gx = weight_image_floats<DIM>(0, p->np, (p->n16 + p->np - 1) / p->np, p->Cp / 8, nimg);
   }
   const size_t t = (size_t)bpt_floats(B, d.rows, p->Cp);
   size_t o = 0;
@@ -963,9 +978,10 @@ int make_bwd_plan(const csmpn_block_desc& d, BwdPlan* p) {
   return CSMPN_OK;
 }
 
-template <int DIM>
+// TERMS: numeric mode (csmpn_block_desc.tf32 = 1 -> 1, else 3); the elementwise kernels do not depend on it
+template <int DIM, int TERMS>
 int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* workspace, int64_t bytes, cudaStream_t stream) {
-  constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G, P = Alg<DIM>::P;
+  constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G, P = Alg<DIM>::P, NI = n_images(TERMS);
   BwdPlan p;
   int st = make_bwd_plan<DIM>(d, &p);
   if (st) return st;
@@ -1023,20 +1039,20 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   ga.w[0] = d.wl; ga.w[1] = d.wr; ga.wk[0] = ga.wk[1] = C; ga.wn = C;
   ga.n16 = Cp; ga.kmax = Cp;
   ga.addend = ws + p.o_dy2p; ga.out = ws + p.o_dy2; ga.out_bpt = 1;
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
-  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemmdb_kernel<DIM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, false, TERMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemm_kernel<DIM, true, TERMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
+  CSMPN_CUDA_TRY(cudaFuncSetAttribute(tc_bgemmdb_kernel<DIM, TERMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   if (mask & 2) {
     if (p.wide) {
       WPrepArgs w{d.wl, d.wr, 0, 1, C, C, C, p.np, (Cp + p.np - 1) / p.np, Cp / 8, Cp / 8, img_dy2};
-      int rc = launch_weight_images<DIM>(w, p.img_dy2, stream);
+      int rc = launch_weight_images<DIM, TERMS>(w, p.img_dy2, stream);
       if (rc) return rc;
       ga.wimg = img_dy2; ga.np = p.np;
-      tc_bgemm_kernel<DIM, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
+      tc_bgemm_kernel<DIM, true, TERMS><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np, NI), stream>>>(ga);
     } else if (use_overlapped_epilogue(B, ga.n16)) {
-      tc_bgemmdb_kernel<DIM><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax), stream>>>(ga);
+      tc_bgemmdb_kernel<DIM, TERMS><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax, NI), stream>>>(ga);
     } else {
-      tc_bgemm_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax), stream>>>(ga);
+      tc_bgemm_kernel<DIM, false, TERMS><<<grid, kThreads, gemm_smem<DIM>(2, ga.n16, ga.kmax, NI), stream>>>(ga);
     }
     CSMPN_LAUNCH_CHECK("tc_bgemm_kernel(dy2)");
   }
@@ -1065,14 +1081,14 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
     ga.out = g.grad_x; ga.out_bpt = g.gx_bpt;
     if (p.wide) {
       WPrepArgs w{d.w1, nullptr, 0, 1, p.cin, C, 0, p.np, (p.n16 + p.np - 1) / p.np, Cp / 8, 0, img_gx};
-      int rc = launch_weight_images<DIM>(w, p.img_gx, stream);
+      int rc = launch_weight_images<DIM, TERMS>(w, p.img_gx, stream);
       if (rc) return rc;
       ga.wimg = img_gx; ga.np = p.np;
-      tc_bgemm_kernel<DIM, true><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np), stream>>>(ga);
+      tc_bgemm_kernel<DIM, true, TERMS><<<grid, kThreads, gemm_smem_streamed<DIM>(p.np, NI), stream>>>(ga);
     } else if (use_overlapped_epilogue(B, ga.n16)) {
-      tc_bgemmdb_kernel<DIM><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
+      tc_bgemmdb_kernel<DIM, TERMS><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax, NI), stream>>>(ga);
     } else {
-      tc_bgemm_kernel<DIM, false><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax), stream>>>(ga);
+      tc_bgemm_kernel<DIM, false, TERMS><<<grid, kThreads, gemm_smem<DIM>(1, ga.n16, ga.kmax, NI), stream>>>(ga);
     }
     CSMPN_LAUNCH_CHECK("tc_bgemm_kernel(grad_x)");
   }
@@ -1081,9 +1097,9 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   memset(&da, 0, sizeof(da));
   da.dbg = debug_buffer();
 #ifdef CSMPN_DEBUG_TOOLS
-  auto dw_kernel = da.dbg ? tc_dw_kernel<DIM, true> : tc_dw_kernel<DIM, false>;
+  auto dw_kernel = da.dbg ? tc_dw_kernel<DIM, true, TERMS> : tc_dw_kernel<DIM, false, TERMS>;
 #else
-  auto dw_kernel = tc_dw_kernel<DIM, false>;
+  auto dw_kernel = tc_dw_kernel<DIM, false, TERMS>;
 #endif
   CSMPN_CUDA_TRY(cudaFuncSetAttribute(dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   da.rows = d.rows; da.tiles = p.tiles;
@@ -1216,8 +1232,8 @@ int64_t bwd_ws_bytes(const csmpn_block_desc& d) {
 }  // namespace tcb
 
 int tc_block_bwd(int dim, const csmpn_block_desc* d, const csmpn_block_grads* g, void* ws, int64_t bytes, cudaStream_t stream) {
-  if (dim == 2) return tcb::launch_bwd<2>(*d, *g, ws, bytes, stream);
-  if (dim == 3) return tcb::launch_bwd<3>(*d, *g, ws, bytes, stream);
+  if (dim == 2) return d->tf32 ? tcb::launch_bwd<2, 1>(*d, *g, ws, bytes, stream) : tcb::launch_bwd<2, 3>(*d, *g, ws, bytes, stream);
+  if (dim == 3) return d->tf32 ? tcb::launch_bwd<3, 1>(*d, *g, ws, bytes, stream) : tcb::launch_bwd<3, 3>(*d, *g, ws, bytes, stream);
   return CSMPN_ERR_UNSUPPORTED;
 }
 // the backward of a block of this shape fits (shared memory / TMEM plans of every backward kernel)

@@ -144,7 +144,9 @@ __device__ __forceinline__ void gather_chunk_api(const FwdArgs& a, int64_t row0,
 // x0 != nullptr: the assembled input rows are also written to the BPT tensor x0 (kept for the weight-gradient GEMM of
 // the backward) straight from the registers, between the two shared-memory phases: a warp covers two rows x 8 channels
 // x all blades, i.e. full 32-byte sectors of every blade plane.
-template <int DIM>
+// TERMS = 1 (single-pass TF32): the values rounded to nearest TF32 go to the raw slot, x0 keeps the unrounded rows, and
+// there is no `lo` phase.
+template <int DIM, int TERMS = 3>
 __device__ __forceinline__ void store_chunk_api(const Pipe& p, int q, const float4* v, float* x0, int x0_cp, int64_t tile, int kc) {
   constexpr int B = Alg<DIM>::B;
   constexpr int H = ApiItems<DIM>::H, PPR = ApiItems<DIM>::PPR, N = ApiItems<DIM>::N, TOT = ApiItems<DIM>::TOT;
@@ -159,7 +161,8 @@ __device__ __forceinline__ void store_chunk_api(const Pipe& p, int q, const floa
       int r, cl, h;
       ApiItems<DIM>::decode(it, r, cl, h);
       float4 hv;
-      split4(v[i], hv, lv[i]);
+      if constexpr (TERMS == 1) hv = tf32_rna4(v[i]);
+      else split4(v[i], hv, lv[i]);
       const uint32_t off = (4 * h) * kPS + (cl >> 2) * kKH + r * 16 + (cl & 3) * 4;
       *reinterpret_cast<float*>(hi + off) = hv.x;
       *reinterpret_cast<float*>(hi + off + kPS) = hv.y;
@@ -183,6 +186,7 @@ __device__ __forceinline__ void store_chunk_api(const Pipe& p, int q, const floa
       }
     }
   }
+  if constexpr (TERMS == 1) return;
   if (q >= 1) mbar_wait(p.lo_bar, (q - 1) & 1);
 #pragma unroll
   for (int i = 0; i < N; ++i) {
@@ -271,21 +275,22 @@ __device__ __forceinline__ void stage_f1_params(const FwdArgs& a, float* b1_s, f
 // =====================================================================================================================
 // F1: MVLinear (W1) + bias + MVSiLU.  ST (streamed weights, wide blocks): the output channels are produced in passes of
 // a.ns1 channels (accumulators = B * ns1 TMEM columns), the K chunks of the input are walked once per pass and every chunk
-// arrives with its weight unit (tc_block.cuh); the resident weight images do not exist.
-template <int DIM, bool BPT_IN, bool ST>
+// arrives with its weight unit (tc_block.cuh); the resident weight images do not exist.  TERMS: numeric mode
+// (tc_block.cuh, n_images).
+template <int DIM, bool BPT_IN, bool ST, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
   using A = Alg<DIM>;
-  constexpr int B = A::B, G = A::G;
+  constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int C = a.C, Cp = a.Cp, nk = a.kin8 / 8;
   const int NS = ST ? a.ns1 : Cp;                     // output channels per pass
   const int npass = ST ? Cp / NS : 1;
-  const uint32_t wunit = ST ? wunit_bytes<DIM>(NS) : 0u;
+  const uint32_t wunit = ST ? wunit_bytes<DIM>(NS, NI) : 0u;
   const uint32_t half = B * kPS + wunit;
   const uint32_t img = ST ? (uint32_t)NS * 32u : (uint32_t)a.kin8 * Cp * 4;
   uint8_t* wimg = smem + (size_t)kRing * half + B * kPS;
-  float* b1_s = reinterpret_cast<float*>(wimg + (ST ? 0 : (size_t)G * 2 * img));
+  float* b1_s = reinterpret_cast<float*>(wimg + (ST ? 0 : (size_t)G * NI * img));
   float* sa_s = b1_s + Cp;
   float* sb_s = sa_s + Cp * G;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sb_s + Cp * G);
@@ -319,7 +324,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
   const uint32_t tcols = tmem_cols((uint32_t)B * NS);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   stage_f1_params<DIM>(a, b1_s, sa_s, sb_s, [&] {
-    if (!ST) stage_weight_images<DIM, false>(wimg, img, a.w1, C, a.cin, Cp, a.kin8);
+    if (!ST) stage_weight_images<DIM, false, TERMS>(wimg, img, a.w1, C, a.cin, Cp, a.kin8);
   });
   prologue_sync();
   const uint32_t tbase = *tmem_slot;
@@ -334,17 +339,17 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
           feed.refill(q, load);
           if constexpr (ST) {
             p.wait_landed(q);  // the weight unit of this chunk
-            issue_chunk_mma<DIM>(p, q, tbase, NS, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, NS, 0, 0, idesc);
+            issue_chunk_mma<DIM, TERMS>(p, q, tbase, NS, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, NS, 0, 0, idesc);
           } else {
-            issue_chunk_mma<DIM>(p, q, tbase, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
+            issue_chunk_mma<DIM, TERMS>(p, q, tbase, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
           }
         } else if (BPT_IN) {  // converters: split the landed chunk
           p.wait_landed(q);
-          split_chunk<B>(p, q);
+          split_chunk<B, TERMS>(p, q);
         } else {              // converters: gathering producer (wide blocks gather the input rows once per pass)
           if (q >= kRing) p.wait_free(q - kRing);
           float* x0 = ps == 0 ? a.save_x0 : nullptr;
-          store_chunk_api<DIM>(p, q, gv, x0, round_up(a.kin8, 16), tile, kc);
+          store_chunk_api<DIM, TERMS>(p, q, gv, x0, round_up(a.kin8, 16), tile, kc);
           p.conv_done(q);
           if (q + 1 < total_chunks) {
             if ((q + 1) % per_tile == 0) load_gather_idx<DIM>(a, tile_of(q + 1) * kTile, gi);  // first chunk of the next tile
@@ -379,18 +384,18 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
 // Roles: warp 0 issues copies and MMAs only; warps 1-15 convert / gather; warps 4-15 also own the epilogue: lane quadrant
 // warp & 3, channel groups (warp >> 2) - 1, + 3, ... (PendingEpilogue).  Same epilogue body as tc_f1_kernel
 // (f1_epilogue_group): results are bit-identical.
-template <int DIM, bool BPT_IN>
+template <int DIM, bool BPT_IN, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
   using A = Alg<DIM>;
   [[maybe_unused]] constexpr bool TL = true;  // timeline stamps (diagnostics build only, when a.dbg is set)
   [[maybe_unused]] int dbg_n = 0;
-  constexpr int B = A::B, G = A::G;
+  constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int C = a.C, Cp = a.Cp, nk = a.kin8 / 8;
   const uint32_t img = (uint32_t)a.kin8 * Cp * 4;
   uint8_t* wimg = smem + (kRing + 1) * B * kPS;
-  float* b1_s = reinterpret_cast<float*>(wimg + (size_t)G * 2 * img);
+  float* b1_s = reinterpret_cast<float*>(wimg + (size_t)G * NI * img);
   float* sa_s = b1_s + Cp;
   float* sb_s = sa_s + Cp * G;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sb_s + Cp * G);
@@ -415,7 +420,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
   const uint32_t bufcols = (uint32_t)B * Cp;  // <= 256 (host)
   const uint32_t tcols = tmem_cols(2 * bufcols);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
-  stage_f1_params<DIM>(a, b1_s, sa_s, sb_s, [&] { stage_weight_images<DIM, false>(wimg, img, a.w1, C, a.cin, Cp, a.kin8); });
+  stage_f1_params<DIM>(a, b1_s, sa_s, sb_s, [&] { stage_weight_images<DIM, false, TERMS>(wimg, img, a.w1, C, a.cin, Cp, a.kin8); });
   prologue_sync();
   const uint32_t tbase = *tmem_slot;
   const uint32_t idesc = idesc_tf32(kTile, Cp, false, false);
@@ -443,17 +448,17 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
         feed.refill(q, load);
         // buffer t & 1 was read by the epilogue of tile t-2: every epilogue warp finished it before its conv_done of
         // this tile's first chunk (full_bar observed above), so the first MMA may overwrite it
-        issue_chunk_mma<DIM>(p, q, tb, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
+        issue_chunk_mma<DIM, TERMS>(p, q, tb, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
         TSTAMP(38);
       } else {
         if (BPT_IN) {
           p.wait_landed(q);
-          split_chunk<B>(p, q);
+          split_chunk<B, TERMS>(p, q);
         } else {
           TSTAMP(30);
           if (q >= kRing) p.wait_free(q - kRing);
           TSTAMP(31);
-          store_chunk_api<DIM>(p, q, gv, a.save_x0, round_up(a.kin8, 16), tile, kc);
+          store_chunk_api<DIM, TERMS>(p, q, gv, a.save_x0, round_up(a.kin8, 16), tile, kc);
           TSTAMP(32);
           p.conv_done(q);
           TSTAMP(33);
@@ -484,10 +489,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
 // ST (streamed weights, wide blocks): NS = a.ns2 < Cp output channels per pass, weight units streamed with the chunks; the
 // row statistics of the MVLayerNorm accumulate over the passes and the final scaling pass re-reads the product sum `o`
 // from the saved tensor (written by the same thread one pass earlier) instead of keeping it in TMEM.
-template <int DIM, bool TL, bool ST>
+template <int DIM, bool TL, bool ST, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   using A = Alg<DIM>;
-  constexpr int B = A::B, G = A::G, P = A::P;
+  constexpr int B = A::B, G = A::G, P = A::P, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   [[maybe_unused]] int dbg_n = 0;
@@ -495,10 +500,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   const int C = a.C, Cp = a.Cp, nk = Cp / 8;
   const int NS = ST ? a.ns2 : Cp;                      // output channels per pass
   const int npass = ST ? Cp / NS : 1;
-  const uint32_t wunit = ST ? wunit_bytes<DIM>(2 * NS) : 0u;
+  const uint32_t wunit = ST ? wunit_bytes<DIM>(2 * NS, NI) : 0u;
   const uint32_t half = B * kPS + wunit;
   const uint32_t img = ST ? (uint32_t)2 * NS * 32u : (uint32_t)2 * Cp * Cp * 4;  // one image: [2 NS rows (right | left)] x [K]
-  const uint32_t set_bytes = ST ? 0u : G * 2 * img;
+  const uint32_t set_bytes = ST ? 0u : G * NI * img;
   uint8_t* wimg = smem + (size_t)kRing * half + B * kPS;
   float* sn_s = reinterpret_cast<float*>(wimg + (size_t)set_bytes);  // sigmoid(normalization.a) [Cp][G]
   float* wv_s = sn_s + Cp * G;                                           // path weights [Cp][P]
@@ -536,7 +541,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   const float pf_la = tid < C ? __ldg(a.la + tid) : 0.f;
   if (!ST) {
     const WJob wj[2] = {{wimg, a.wr, C, C, 0}, {wimg, a.wl, C, C, Cp}};  // right | left stacked along the image rows
-    stage_weight_jobs<DIM, false, 2>(wj, 2, img, 2 * Cp, Cp, wimg, (uint32_t)G * 2u * img);
+    stage_weight_jobs<DIM, false, 2, TERMS>(wj, 2, img, 2 * Cp, Cp, wimg, (uint32_t)G * (uint32_t)NI * img);
   }
   TSTAMP(4);
   if (tid < Cp * G) sn_s[tid] = tid < C * G ? sigmoidf_(pf_na) : 0.f;
@@ -572,13 +577,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
           TSTAMP(14);
           feed.refill(q, load);
           TSTAMP(16);
-          if constexpr (ST) issue_chunk_mma<DIM>(p, q, tbase, bcols, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, bcols, 0, 0, idesc);
-          else issue_chunk_mma<DIM>(p, q, tbase, bcols, kc > 0, wimg, img, 0, 1, 0, bcols, kc, 0, idesc);
+          if constexpr (ST) issue_chunk_mma<DIM, TERMS>(p, q, tbase, bcols, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, bcols, 0, 0, idesc);
+          else issue_chunk_mma<DIM, TERMS>(p, q, tbase, bcols, kc > 0, wimg, img, 0, 1, 0, bcols, kc, 0, idesc);
           TSTAMP(15);
         } else {          // converters
           p.wait_landed(q);
           TSTAMP(11);
-          split_chunk<B>(p, q);
+          split_chunk<B, TERMS>(p, q);
           TSTAMP(13);
         }
       }
@@ -727,7 +732,9 @@ long long*& debug_buffer() {
 }
 
 // How the two forward kernels of a block of this shape run: weights resident in shared memory, or -- wide blocks --
-// streamed with the K chunks in passes of ns1 / ns2 output channels (tc_block.cuh).
+// streamed with the K chunks in passes of ns1 / ns2 output channels (tc_block.cuh).  The choice is made for the default
+// (split) weight images, so both numeric modes run a shape with the same plan; nimg = 1 (single-pass TF32) only shrinks
+// the shared memory and the streamed image buffers.
 struct FwdPlan {
   bool ok;
   bool st1, st2;
@@ -737,7 +744,7 @@ struct FwdPlan {
 };
 
 template <int DIM>
-FwdPlan fwd_plan(int cin, int c) {
+FwdPlan fwd_plan(int cin, int c, int nimg = 2) {
   constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G, P = Alg<DIM>::P;
   FwdPlan p;
   memset(&p, 0, sizeof(p));
@@ -770,6 +777,14 @@ FwdPlan fwd_plan(int cin, int c) {
     p.s2 = (size_t)kRing * wunit_bytes<DIM>(2 * ns) + ring + par2;
     p.w2_floats = weight_image_floats<DIM>(1, ns, Cp / ns, Cp / 8);
   }
+  if (nimg != 2) {
+    p.s1 = one_cta_per_sm(p.st1 ? (size_t)kRing * wunit_bytes<DIM>(p.ns1, nimg) + ring + par1
+                                : ring + (size_t)G * nimg * kin8 * Cp * 4 + par1);
+    p.s2 = one_cta_per_sm(p.st2 ? (size_t)kRing * wunit_bytes<DIM>(2 * p.ns2, nimg) + ring + par2
+                                : ring + (size_t)2 * G * nimg * Cp * Cp * 4 + par2);
+    if (p.st1) p.w1_floats = weight_image_floats<DIM>(0, p.ns1, Cp / p.ns1, kin8 / 8, nimg);
+    if (p.st2) p.w2_floats = weight_image_floats<DIM>(1, p.ns2, Cp / p.ns2, Cp / 8, nimg);
+  }
   p.ok = true;
   return p;
 }
@@ -781,12 +796,13 @@ inline int64_t align32f(int64_t floats) { return (floats + 31) / 32 * 32; }
 
 template <int DIM>
 int64_t fwd_ws_bytes(const csmpn_block_desc& d) {
-  const FwdPlan p = fwd_plan<DIM>(d.c0 + d.c1 + d.c2, d.c);
+  const FwdPlan p = fwd_plan<DIM>(d.c0 + d.c1 + d.c2, d.c, d.tf32 ? 1 : 2);
   if (!p.ok) return -1;
   return (align32f(p.w1_floats) + align32f(p.w2_floats)) * 4;
 }
 
-template <int DIM>
+// TERMS: numeric mode (csmpn_block_desc.tf32 = 1 -> 1, else 3)
+template <int DIM, int TERMS>
 int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   constexpr int B = Alg<DIM>::B;
   FwdArgs a;
@@ -811,7 +827,7 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   if (a.in_bpt && (d.mode != 0 || d.c1 || d.c2)) return CSMPN_ERR_BAD_ARG;
   if (d.mode == 2 && (d.vt_k < 1 || d.vt_k > 3 || d.vt_fp < 1 || d.c0 % (d.vt_k * d.vt_fp) || d.c1 || d.c2 || !d.src)) return CSMPN_ERR_BAD_ARG;
   if (a.out_bpt && d.res) return CSMPN_ERR_BAD_ARG;
-  const FwdPlan p = fwd_plan<DIM>(a.cin, a.C);
+  const FwdPlan p = fwd_plan<DIM>(a.cin, a.C, n_images(TERMS));
   if (!p.ok) return CSMPN_ERR_UNSUPPORTED;
   if (a.tiles == 0) return CSMPN_OK;
   a.ns1 = p.ns1; a.ns2 = p.ns2;
@@ -825,12 +841,12 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
     a.wimg1 = w1img; a.wimg2 = w2img;
     if (p.st1 && (mask & 1)) {
       WPrepArgs w{d.w1, nullptr, 0, 0, a.C, a.cin, 0, p.ns1, a.Cp / p.ns1, a.kin8 / 8, 0, w1img};
-      int st = launch_weight_images<DIM>(w, p.w1_floats, stream);
+      int st = launch_weight_images<DIM, TERMS>(w, p.w1_floats, stream);
       if (st) return st;
     }
     if (p.st2 && (mask & 2)) {
       WPrepArgs w{d.wr, d.wl, 1, 0, a.C, a.C, 0, p.ns2, a.Cp / p.ns2, a.Cp / 8, 0, w2img};
-      int st = launch_weight_images<DIM>(w, p.w2_floats, stream);
+      int st = launch_weight_images<DIM, TERMS>(w, p.w2_floats, stream);
       if (st) return st;
     }
   }
@@ -846,9 +862,9 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   a.dbg = dbg_f1 ? dbg_buf : nullptr;
   if (mask & 1) {
     const bool overlap = !p.st1 && use_overlapped_epilogue(B, a.Cp);
-    int rc = overlap ? (a.in_bpt ? run(tc_f1db_kernel<DIM, true>, p.s1) : run(tc_f1db_kernel<DIM, false>, p.s1))
-             : a.in_bpt ? (p.st1 ? run(tc_f1_kernel<DIM, true, true>, p.s1) : run(tc_f1_kernel<DIM, true, false>, p.s1))
-                        : (p.st1 ? run(tc_f1_kernel<DIM, false, true>, p.s1) : run(tc_f1_kernel<DIM, false, false>, p.s1));
+    int rc = overlap ? (a.in_bpt ? run(tc_f1db_kernel<DIM, true, TERMS>, p.s1) : run(tc_f1db_kernel<DIM, false, TERMS>, p.s1))
+             : a.in_bpt ? (p.st1 ? run(tc_f1_kernel<DIM, true, true, TERMS>, p.s1) : run(tc_f1_kernel<DIM, true, false, TERMS>, p.s1))
+                        : (p.st1 ? run(tc_f1_kernel<DIM, false, true, TERMS>, p.s1) : run(tc_f1_kernel<DIM, false, false, TERMS>, p.s1));
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_f1_kernel");
   }
@@ -856,10 +872,10 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   if (mask & 2) {
     int rc;
 #ifdef CSMPN_DEBUG_TOOLS
-    if (a.dbg && !p.st2) rc = run(tc_f2_kernel<DIM, true, false>, p.s2);
+    if (a.dbg && !p.st2) rc = run(tc_f2_kernel<DIM, true, false, TERMS>, p.s2);
     else
 #endif
-    rc = p.st2 ? run(tc_f2_kernel<DIM, false, true>, p.s2) : run(tc_f2_kernel<DIM, false, false>, p.s2);
+    rc = p.st2 ? run(tc_f2_kernel<DIM, false, true, TERMS>, p.s2) : run(tc_f2_kernel<DIM, false, false, TERMS>, p.s2);
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_f2_kernel");
   }
@@ -869,8 +885,8 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
 }  // namespace tcb
 
 int tc_block_fwd(int dim, const csmpn_block_desc* d, cudaStream_t stream) {
-  if (dim == 2) return tcb::launch_fwd<2>(*d, stream);
-  if (dim == 3) return tcb::launch_fwd<3>(*d, stream);
+  if (dim == 2) return d->tf32 ? tcb::launch_fwd<2, 1>(*d, stream) : tcb::launch_fwd<2, 3>(*d, stream);
+  if (dim == 3) return d->tf32 ? tcb::launch_fwd<3, 1>(*d, stream) : tcb::launch_fwd<3, 3>(*d, stream);
   return CSMPN_ERR_UNSUPPORTED;
 }
 void tc_set_debug_buffer(long long* p) { tcb::debug_buffer() = p; }

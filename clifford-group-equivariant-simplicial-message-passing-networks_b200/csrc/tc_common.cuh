@@ -13,6 +13,8 @@
 // Every encoding here was pinned on a B200 with tools/tc_probe_raw.py (profiles/r01_tc_probe.log).
 // fp32 accuracy on the TF32 pipe comes from the usual error-compensated split  x = hi + lo  with hi = x with the low
 // 13 mantissa bits cleared (exactly representable in TF32) and three MMAs per product: hi*hi + hi*lo + lo*hi.
+// Single-pass TF32 mode (csmpn_block_desc.tf32, kernels instantiated with TERMS = 1) rounds each operand to nearest TF32
+// once and issues one MMA per product.
 #pragma once
 #include "common.cuh"
 
@@ -185,6 +187,14 @@ __device__ __forceinline__ bool aligned32(const void* p) { return (reinterpret_c
 
 // ------------------------------------------------------------------------------------------------ split
 __device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
+// single-pass TF32 operand: x rounded to the nearest TF32 value (ties away from zero), low 13 mantissa bits zero, so the
+// truncating operand read of kind::tf32 takes it exactly
+__device__ __forceinline__ float tf32_rna(float x) {
+  uint32_t y;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(y) : "f"(x));
+  return __uint_as_float(y);
+}
+__device__ __forceinline__ float4 tf32_rna4(const float4& x) { return make_float4(tf32_rna(x.x), tf32_rna(x.y), tf32_rna(x.z), tf32_rna(x.w)); }
 __device__ __forceinline__ void split4(const float4& x, float4& hi, float4& lo) {
   hi.x = tf32_hi(x.x); hi.y = tf32_hi(x.y); hi.z = tf32_hi(x.z); hi.w = tf32_hi(x.w);
   lo.x = x.x - hi.x; lo.y = x.y - hi.y; lo.z = x.z - hi.z; lo.w = x.w - hi.w;

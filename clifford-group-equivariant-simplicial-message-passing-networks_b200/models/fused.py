@@ -37,6 +37,7 @@ class BlockDesc(ctypes.Structure):
         ("pair_attr", c_int32),
         ("vt_k", c_int32), ("vt_fp", c_int32),
         ("fwd_ws", c_void_p), ("fwd_ws_bytes", c_int64),
+        ("tf32", c_int32),
     ]
 
 
@@ -71,6 +72,17 @@ def _record(kind, dim, d, g=None, ws=None, keep=()):
 def tc_enabled() -> bool:
     """Tensor-core (tcgen05) engine switch: CSMPN_TC=0 forces the FP32 SIMT kernels (tests cross-check the two)."""
     return os.environ.get("CSMPN_TC", "1") != "0"
+
+
+def tc_precision() -> bool:
+    """True when the tensor-core engine runs its channel GEMMs in single-pass TF32 (csmpn_block_desc.tf32): PyTorch's
+    float32 matmul precision for CUDA is "tf32", i.e. ``torch.backends.cuda.matmul.fp32_precision == "tf32"``.  That
+    is what ``torch.set_float32_matmul_precision("high")`` / ``("medium")``, ``torch.backends.cuda.matmul.allow_tf32 =
+    True`` and ``torch.backends.fp32_precision = "tf32"`` select, and what makes the reference's einsum linears run in
+    TF32.  Any other value keeps the default error-compensated fp32 products.  The attribute is read directly:
+    ``torch.get_float32_matmul_precision()`` and ``allow_tf32`` raise once a program has mixed the legacy and the new API.
+    Only the tensor-core engine follows the setting; the FP32 SIMT engine and the unit kernels always compute in fp32."""
+    return torch.backends.cuda.matmul.fp32_precision == "tf32"
 
 
 def tc_supported(dim: int, c_in: int, c: int) -> bool:
@@ -289,7 +301,11 @@ class TcBlockFn(torch.autograd.Function):
 
     cfg: dim, mode, sgraph, rows, in_bpt (p0 is a BPT tensor with cfg["c_in"] channels), out_bpt, need_grad.
     Intermediates and saved tensors are BPT (blade-plane tile) tensors; only the block boundary facing the rest of the
-    model (gathered h / edge_attr, the messages, the layer output and the residual) is in the reference layout."""
+    model (gathered h / edge_attr, the messages, the layer output and the residual) is in the reference layout.
+
+    Numeric mode: the forward reads tc_precision() once and its backward runs in the same mode, even if the setting
+    changes in between.  A captured CUDA graph (GraphedEGCL, GraphedLayerStep, the train-step graphs) keeps the mode that
+    was set at capture time, like every other descriptor field."""
 
     @staticmethod
     def forward(ctx, cfg, p0, p1, p2, res, w1, b1, sa, sb, wr, na, wl, bl, wp, la):
@@ -321,6 +337,7 @@ class TcBlockFn(torch.autograd.Function):
         resc = None if res is None else f32c(res)
         d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, resc, saves, pair)
         d.engine, d.in_bpt, d.out_bpt = 1, int(in_bpt), int(out_bpt)
+        d.tf32 = ctx.tf32 = int(tc_precision())
         d.save_y2 = y2.data_ptr()
         d.save_x0 = None if x0 is None else x0.data_ptr()
         if vt is not None:
@@ -388,6 +405,7 @@ def _tc_block_backward(ctx, gy):
     cin = sum(chans)
     d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, gy, None, (y1, xr, o), pair)
     d.engine, d.in_bpt, d.out_bpt = 1, int(in_bpt), int(out_bpt)
+    d.tf32 = ctx.tf32  # the mode of the forward
     d.save_y2 = y2.data_ptr()
     d.save_x0 = None if x0 is None else x0.data_ptr()
     if vt is not None:
@@ -680,7 +698,8 @@ def _time_call(fn, flush, iters, warm=3):
 def _kernel_stages(d: BlockDesc, g, B: int):
     """(class, description, mask, algorithmic bytes, tensor-pipe FLOPs) of every kernel behind one recorded block call.
     Algorithmic bytes = every tensor the kernel must read or write, once (DESIGN.md section 4); T = one BPT [rows, Cp]
-    tensor, Tin = one BPT [rows, c_in] tensor; tensor-pipe FLOPs count the three TF32 MMAs of a split product."""
+    tensor, Tin = one BPT [rows, c_in] tensor; tensor-pipe FLOPs count the three TF32 MMAs of a split product,
+    or the one MMA of a single-pass TF32 product (d.tf32)."""
     rows, C = int(d.rows), int(d.c)
     cin = d.c0 + d.c1 + d.c2
     cp, cinp = (C + 15) // 16 * 16, (cin + 15) // 16 * 16
@@ -692,20 +711,21 @@ def _kernel_stages(d: BlockDesc, g, B: int):
         if g is None:
             return [("block_fwd (fp32 simt)", "fused CEMLP block forward", 0, src + ref(4 * C), 0)]
         return [("block_bwd (fp32 simt)", "fused CEMLP block backward + parameter-gradient reduce", 0, src + ref(4 * C) + ref(cin), 0)]
+    k = 1 if d.tf32 else 3  # TF32 MMAs per product
     if g is None:
         f1_in = Tin if d.in_bpt else (ref(2 * d.c0) + ref(d.c1) + 12 * rows if d.mode == 1 else ref(cin))
         f1_out = (0 if d.in_bpt else Tin) + 2 * T
         y_out = T if d.out_bpt else ref(C) * (2 if d.res else 1)
-        return [("tc_f1", "input rows (gather | BPT) -> MVLinear W1 + bias -> y1, MVSiLU -> y2", 1, f1_in + f1_out, 3 * rows * 2 * B * C * cin),
-                ("tc_f2", "linear_right/left + normalisation + weighted GP + MVLayerNorm (+residual)", 2, 4 * T + y_out, 3 * rows * 4 * B * C * C)]
+        return [("tc_f1", "input rows (gather | BPT) -> MVLinear W1 + bias -> y1, MVSiLU -> y2", 1, f1_in + f1_out, k * rows * 2 * B * C * cin),
+                ("tc_f2", "linear_right/left + normalisation + weighted GP + MVLayerNorm (+residual)", 2, 4 * T + y_out, k * rows * 4 * B * C * C)]
     gy = T if g.gy_bpt else ref(C)
     gx = 0 if not g.grad_x else (Tin if g.gx_bpt else ref(cin))
     return [("tc_b1", "MVLayerNorm / weighted GP / normalisation adjoints", 1, 6 * T + gy, 0),
-            ("tc_bgemm", "dy2 = dy2p + d WL + dxr WR", 2, 4 * T, 3 * rows * 4 * B * C * C),
+            ("tc_bgemm", "dy2 = dy2p + d WL + dxr WR", 2, 4 * T, k * rows * 4 * B * C * C),
             ("tc_b3", "MVSiLU adjoint", 4, 3 * T, 0),
-            ("tc_bgemm", "grad_x = dy1 W1", 8, T + gx, 3 * rows * 2 * B * C * cin),
-            ("tc_dw", "dWL, dWR = [d|dxr]^T y2", 16, 3 * T, 3 * rows * 4 * B * C * C),
-            ("tc_dw", "dW1 = dy1^T x0", 32, T + Tin, 3 * rows * 2 * B * C * cin),
+            ("tc_bgemm", "grad_x = dy1 W1", 8, T + gx, k * rows * 2 * B * C * cin),
+            ("tc_dw", "dWL, dWR = [d|dxr]^T y2", 16, 3 * T, k * rows * 4 * B * C * C),
+            ("tc_dw", "dW1 = dy1^T x0", 32, T + Tin, k * rows * 2 * B * C * cin),
             ("tc_final", "fixed-order reduction of per-CTA partials", 64, 0, 0)]
 
 

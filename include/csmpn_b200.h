@@ -209,6 +209,13 @@ typedef struct csmpn_block_desc {
   void* fwd_ws;                         /* engine 1, wide blocks (csmpn_block_fwd_workspace > 0): device scratch of the
                                            forward for the pre-split weight images streamed with the K chunks */
   int64_t fwd_ws_bytes;
+  int32_t tf32;                         /* engine 1: 0 = error-compensated fp32 products (x = hi + lo, three TF32 MMAs per
+                                           product; the default), 1 = single-pass TF32: every GEMM operand rounded to
+                                           nearest TF32 once, one MMA per product (what PyTorch does for fp32 matmuls under
+                                           torch.backends.cuda.matmul.fp32_precision = "tf32"); smaller streamed weight
+                                           images (csmpn_block_fwd_workspace / csmpn_block_bwd_workspace).  Engine 0
+                                           ignores it; any other value is CSMPN_ERR_BAD_ARG.  The backward of a block must
+                                           be called with the value of its forward. */
 } csmpn_block_desc;
 
 /* gradients produced by csmpn_block_bwd (all overwritten; parameter gradients reduced deterministically) */
