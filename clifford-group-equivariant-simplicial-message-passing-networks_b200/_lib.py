@@ -59,6 +59,7 @@ def _declare(lib):
         "csmpn_block_fwd": (c_int, [i32, P, P]),
         "csmpn_block_tc_supported": (c_int, [i32, i32, i32]),
         "csmpn_block_tc_plan": (c_int, [i32, i32, i32]),
+        "csmpn_block_tc_passes": (c_int, [i32, i32, i32]),
         "csmpn_block_fwd_workspace": (i64, [i32, P]),
         "csmpn_block_simt_resident": (c_int, [i32, i32, i32]),
         "csmpn_bpt_floats": (i64, [i32, i64, i32]),

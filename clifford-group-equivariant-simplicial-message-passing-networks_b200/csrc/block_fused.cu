@@ -1063,6 +1063,7 @@ int tc_block_bwd(int dim, const csmpn_block_desc* d, const csmpn_block_grads* g,
 int64_t tc_block_bwd_workspace(int dim, const csmpn_block_desc* d);
 int64_t tc_block_fwd_workspace(int dim, const csmpn_block_desc* d);
 int tc_block_plan(int dim, int c_in, int c);
+int tc_block_passes(int dim, int c_in, int c);
 bool tc_block_supported(int dim, int c_in, int c);
 void tc_set_debug_buffer(long long* p);
 }  // namespace csmpn
@@ -1073,6 +1074,7 @@ extern "C" {
 
 int csmpn_block_tc_supported(int dim, int c_in, int c) { return tc_block_supported(dim, c_in, c) ? 1 : 0; }
 int csmpn_block_tc_plan(int dim, int c_in, int c) { return tc_block_plan(dim, c_in, c); }
+int csmpn_block_tc_passes(int dim, int c_in, int c) { return tc_block_passes(dim, c_in, c); }
 
 // > 0 (= rows per shared-memory tile) if the FP32 SIMT engine keeps the three weight matrices of such a block resident in shared memory for both the forward
 // and the backward kernel; 0 if it would fall back to staging them per GEMM (slower than the unit kernels: callers

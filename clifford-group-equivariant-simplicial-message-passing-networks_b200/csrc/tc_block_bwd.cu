@@ -1252,7 +1252,7 @@ int tc_block_bwd_wide(int dim, int c_in, int c) {
   d.c0 = c_in; d.c = c; d.rows = 128;
   tcb::BwdPlan p;
   const int st = dim == 2 ? tcb::make_bwd_plan<2>(d, &p) : dim == 3 ? tcb::make_bwd_plan<3>(d, &p) : -1;
-  return st == CSMPN_OK && p.wide;
+  return st == CSMPN_OK && p.wide ? p.np : 0;
 }
 int64_t tc_block_bwd_workspace(int dim, const csmpn_block_desc* d) {
   if (dim == 2) return tcb::bwd_ws_bytes<2>(*d);

@@ -896,13 +896,20 @@ int64_t tc_block_fwd_workspace(int dim, const csmpn_block_desc* d) {
   return -1;
 }
 bool tc_block_bwd_supported(int dim, int c_in, int c);  // tc_block_bwd.cu
-int tc_block_bwd_wide(int dim, int c_in, int c);         // tc_block_bwd.cu
+int tc_block_bwd_wide(int dim, int c_in, int c);         // tc_block_bwd.cu: np of the wide plan, 0 if resident
 bool tc_block_supported(int dim, int c_in, int c);
 // bit 0: supported, bit 1 / 2: f1 / f2 stream their weights, bit 3: the backward runs the wide plan
 int tc_block_plan(int dim, int c_in, int c) {
   if (!tc_block_supported(dim, c_in, c)) return 0;
   tcb::FwdPlan p = dim == 2 ? tcb::fwd_plan<2>(c_in, c) : tcb::fwd_plan<3>(c_in, c);
   return 1 | (p.st1 ? 2 : 0) | (p.st2 ? 4 : 0) | (tc_block_bwd_wide(dim, c_in, c) ? 8 : 0);
+}
+// output channels per pass: bits 0-9 f1 (ns1), bits 10-19 f2 (ns2; both = Cp with resident weights), bits 20-29 the
+// streamed backward GEMMs (np; 0 for the resident backward); 0 if the engine does not take the shape
+int tc_block_passes(int dim, int c_in, int c) {
+  if (!tc_block_supported(dim, c_in, c)) return 0;
+  tcb::FwdPlan p = dim == 2 ? tcb::fwd_plan<2>(c_in, c) : tcb::fwd_plan<3>(c_in, c);
+  return p.ns1 | (p.ns2 << 10) | (tc_block_bwd_wide(dim, c_in, c) << 20);
 }
 bool tc_block_supported(int dim, int c_in, int c) {
   if (dim == 2) return tcb::fwd_supported<2>(c_in, c) && tc_block_bwd_supported(2, c_in, c);

@@ -86,6 +86,12 @@ def tc_precision() -> bool:
 
 
 def tc_supported(dim: int, c_in: int, c: int) -> bool:
+    """The tensor-core engine takes the block.  In single-pass TF32 mode a block of width 1 stays off it: MVLayerNorm over
+    one channel leaves gradients that are small differences of large terms, and one TF32 rounding of the GEMM operands
+    costs up to 2.5e-2 of them against the fp64 oracle; the FP32 SIMT engine or the unit kernels keep such a block fp32
+    accurate.  (A plain-PyTorch implementation computes one-channel linears as elementwise products, in fp32, too.)"""
+    if c == 1 and tc_precision():
+        return False
     return tc_enabled() and bool(lib().csmpn_block_tc_supported(dim, c_in, c))
 
 

@@ -244,6 +244,10 @@ int csmpn_block_tc_supported(int dim, int c_in, int c);
  * with the K chunks (wide blocks: Cl(3,0) with c >= 64, ...) instead of keeping them resident in shared memory; bit 3 =
  * the backward runs the wide plan (streamed GEMM weights, slab-wise weight-gradient launches, separate MVSiLU adjoint) */
 int csmpn_block_tc_plan(int dim, int c_in, int c);
+/* output channels per pass of such a block on engine 1: bits 0-9 the first forward kernel (ns1), bits 10-19 the second
+ * (ns2; both equal the padded width Cp = 16 * ceil(c / 16) when the weights stay resident), bits 20-29 the streamed
+ * backward GEMMs of the wide plan (np; 0 for the resident backward); 0 if engine 1 does not handle the shape */
+int csmpn_block_tc_passes(int dim, int c_in, int c);
 /* > 0 (the rows per shared-memory tile) if engine 0 keeps the block's weights resident in shared memory (forward and
  * backward), 0 if it would stage them per GEMM; with fewer than 8 rows per tile or staged weights the unit kernels
  * (csmpn_mvlinear_*, csmpn_mvsilu_*, csmpn_wgp_*, ...) composed by the host are the faster path for that shape */
