@@ -78,13 +78,6 @@ def _declare(lib):
         "csmpn_lift_count": (c_int, [P, P, P, P, P, P]),
         "csmpn_lift_fill": (c_int, [P, P, P, i64, P, P, P, P, P]),
     }
-    # bring-up diagnostics: only in a CSMPN_DEBUG_BUILD=1 library (csrc/csmpn_debug.h)
-    debug = {
-        "csmpn_tc_debug_buffer": (c_int, [P]),
-        "csmpn_tc_probe": (c_int, [i32, i32, i32, i32, i32, P, P, P, P]),
-        "csmpn_tc_probe_raw": (c_int, [P, i32, P, i32, P, P, P]),
-    }
-    sigs.update({k: v for k, v in debug.items() if hasattr(lib, k)})
     for name, (res, args) in sigs.items():
         fn = getattr(lib, name)
         fn.restype = res

@@ -1065,7 +1065,6 @@ int64_t tc_block_fwd_workspace(int dim, const csmpn_block_desc* d);
 int tc_block_plan(int dim, int c_in, int c);
 int tc_block_passes(int dim, int c_in, int c);
 bool tc_block_supported(int dim, int c_in, int c);
-void tc_set_debug_buffer(long long* p);
 }  // namespace csmpn
 
 using namespace csmpn;
@@ -1094,16 +1093,6 @@ int csmpn_block_simt_resident(int dim, int c_in, int c) {
   if (!(sf == CSMPN_OK && sb == CSMPN_OK && pf.resident && pb.resident)) return 0;
   return pf.tr < pb.tr ? pf.tr : pb.tr;  // rows per tile that still fit next to the resident weights
 }
-
-#ifdef CSMPN_DEBUG_TOOLS
-}  // extern "C"
-#include "csmpn_debug.h"
-extern "C" {
-int csmpn_tc_debug_buffer(int64_t* device_buffer_1024) {
-  tc_set_debug_buffer((long long*)device_buffer_1024);
-  return CSMPN_OK;
-}
-#endif
 
 int64_t csmpn_bpt_floats(int dim, int64_t rows, int channels) {
   if (dim < 1 || dim > 5 || rows < 0 || channels < 1) return -1;

@@ -8,15 +8,11 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ["api.cu", "elementwise.cu", "linear.cu", "graph.cu", "block_fused.cu", "lift.cu", "tc_block_fwd.cu", "tc_block_bwd.cu"]
-# CSMPN_DEBUG_BUILD=1: also build the bring-up diagnostics (csmpn_debug.h: single-tile tcgen05 probe, in-kernel timelines)
-DEBUG_BUILD = os.environ.get("CSMPN_DEBUG_BUILD", "0") == "1"
-if DEBUG_BUILD:
-    SOURCES.append("tc_probe.cu")
 LIB = os.path.join(HERE, "libcsmpn_b200.so")
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v",
-] + (["-DCSMPN_DEBUG_TOOLS"] if DEBUG_BUILD else [])
+]
 
 
 def _nvcc():

@@ -615,21 +615,7 @@ struct DwArgs {
   int b_c4;       // first 4-channel group of bsrc used by this launch
   int M;          // 64 or 128, >= channels of Acat
   float* partial; // [grid][G][M][cpb]
-  long long* dbg; // optional timeline buffer (csmpn_tc_debug_buffer): CTA 0, threads 0 (issuer) and 32 (converter)
 };
-long long*& debug_buffer();  // tc_block_fwd.cu
-#ifdef CSMPN_DEBUG_TOOLS
-#define DW_STAMP(code)                                                                       \
-  do {                                                                                       \
-    if (TL && a.dbg && blockIdx.x == 0 && (tid == 0 || tid == 32) && dbg_n < 250) {          \
-      a.dbg[(tid ? 512 : 0) + 2 * dbg_n] = (code);                                           \
-      a.dbg[(tid ? 512 : 0) + 2 * dbg_n + 1] = clock64();                                    \
-      ++dbg_n;                                                                               \
-    }                                                                                        \
-  } while (0)
-#else
-#define DW_STAMP(code) do { } while (0)
-#endif
 
 // Step = (tile, blade, half of the tile's rows): 64 rows = 8 K steps.  A landing unit = (tile, blade) = two steps: the
 // blade slabs of the operand tensors ([channels/4][128 rows][4], contiguous in a BPT tensor) arrive with 2-3 large bulk
@@ -642,13 +628,12 @@ constexpr int kDwRows = 64;
 constexpr int kDwLand = 2;                 // landing slots; a slot holds one (tile, blade) = both row halves = two steps
 constexpr uint32_t kLand = kTile * 16;     // landing stride of one 4-channel column: [128 rows][4 channels], as in global memory
 
-template <int DIM, bool TL, int TERMS = 3>
+template <int DIM, int TERMS = 3>
 __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G;
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
-  [[maybe_unused]] int dbg_n = 0;
   const int ca4 = a.cpa >> 2;
   const int na4 = (a.a1 ? 2 : 1) * ca4;  // 4-channel groups of Acat
   const int nb4 = a.cpb >> 2;
@@ -712,10 +697,8 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
     uint32_t grade_used = 0;
     for (int st = 0; st < steps; ++st) {
       const int b = (st >> 1) % B, g = A::grade_of(b);
-      DW_STAMP(30);
       mbar_wait(&full_bar[st & 1], (st >> 1) & 1);
       fence_after_sync();
-      DW_STAMP(31);
       const uint8_t* op_a = ops + (size_t)(st & 1) * op_bytes;
       const uint8_t* op_b = op_a + 2 * (size_t)ga * grp;
       const uint64_t a_hi = desc_mn32b(smem_addr(op_a), grp, 0), a_lo = a_hi + ((uint64_t)ga * grp >> 4);
@@ -735,21 +718,16 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
       }
       mma_commit_w(&op_bar[st & 1]);
       __syncwarp();
-      DW_STAMP(32);
       // both row halves of the landing unit st >> 1 have been converted (full_bar observed above): refill its slot
       if ((st & 1) && loaded < units) { issue(loaded); ++loaded; }
-      DW_STAMP(33);
       grade_used |= 1u << g;
     }
   } else {
     const int ct = tid - 32, nconv = kConvWarps * 32;
     for (int st = 0; st < steps; ++st) {
       const int lu = st >> 1, rh = st & 1;
-      DW_STAMP(40);
       mbar_wait(&load_bar[lu % kDwLand], (lu / kDwLand) & 1);
-      DW_STAMP(41);
       if (st >= 2) mbar_wait(&op_bar[st & 1], ((st - 2) >> 1) & 1);  // the MMAs of step st-2 released this operand buffer
-      DW_STAMP(42);
       const uint8_t* src = land + (size_t)(lu % kDwLand) * land_bytes + (uint32_t)rh * (kDwRows * 16);
       uint8_t* op_a = ops + (size_t)(st & 1) * op_bytes;  // A hi groups, A lo groups
       uint8_t* op_b = op_a + 2 * (size_t)ga * grp;        // B hi groups, B lo groups
@@ -778,7 +756,6 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
       fence_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(&full_bar[st & 1]);
-      DW_STAMP(43);
     }
   }
   uint32_t grade_used = 0;
@@ -1095,12 +1072,7 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   // ---- weight gradients
   DwArgs da;
   memset(&da, 0, sizeof(da));
-  da.dbg = debug_buffer();
-#ifdef CSMPN_DEBUG_TOOLS
-  auto dw_kernel = da.dbg ? tc_dw_kernel<DIM, true, TERMS> : tc_dw_kernel<DIM, false, TERMS>;
-#else
-  auto dw_kernel = tc_dw_kernel<DIM, false, TERMS>;
-#endif
+  auto dw_kernel = tc_dw_kernel<DIM, TERMS>;
   CSMPN_CUDA_TRY(cudaFuncSetAttribute(dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax));
   da.rows = d.rows; da.tiles = p.tiles;
   std::vector<FinalJob> jobs;

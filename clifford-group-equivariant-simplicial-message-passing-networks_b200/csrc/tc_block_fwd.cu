@@ -35,20 +35,7 @@ struct FwdArgs {
   // streamed-weights mode (wide blocks): pre-split weight images in global memory and the channels per pass
   const float *wimg1, *wimg2;
   int ns1, ns2;
-  long long* dbg;  // optional timeline buffer (csmpn_tc_debug_buffer): CTA 0 records clock64() stamps of threads 0 and 64
 };
-#ifdef CSMPN_DEBUG_TOOLS
-#define TSTAMP(code)                                                                         \
-  do {                                                                                       \
-    if (TL && a.dbg && blockIdx.x == 0 && (tid == 0 || tid == 64) && dbg_n < 250) {          \
-      a.dbg[(tid ? 512 : 0) + 2 * dbg_n] = (code);                                           \
-      a.dbg[(tid ? 512 : 0) + 2 * dbg_n + 1] = clock64();                                    \
-      ++dbg_n;                                                                               \
-    }                                                                                        \
-  } while (0)
-#else
-#define TSTAMP(code) do { } while (0)
-#endif
 
 // ---- producer 2: gather / concatenate API-layout rows (all threads) ------------------------------------------------
 // Item = (row r, channel cl of the chunk, blade quad h): one float4.  gather_chunk_api only LOADS (the values stay in
@@ -387,8 +374,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
 template <int DIM, bool BPT_IN, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
   using A = Alg<DIM>;
-  [[maybe_unused]] constexpr bool TL = true;  // timeline stamps (diagnostics build only, when a.dbg is set)
-  [[maybe_unused]] int dbg_n = 0;
   constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
@@ -442,35 +427,26 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
     const uint32_t tb = tbase + (uint32_t)(t & 1) * bufcols;
     for (int kc = 0; kc < nk; ++kc, ++q) {
       if (warp == 0) {  // issuer
-        TSTAMP(36);
         p.wait_full(q);
-        TSTAMP(37);
         feed.refill(q, load);
         // buffer t & 1 was read by the epilogue of tile t-2: every epilogue warp finished it before its conv_done of
         // this tile's first chunk (full_bar observed above), so the first MMA may overwrite it
         issue_chunk_mma<DIM, TERMS>(p, q, tb, Cp, kc > 0, wimg, img, 0, 1, 0, Cp, kc, 0, idesc);
-        TSTAMP(38);
       } else {
         if (BPT_IN) {
           p.wait_landed(q);
           split_chunk<B, TERMS>(p, q);
         } else {
-          TSTAMP(30);
           if (q >= kRing) p.wait_free(q - kRing);
-          TSTAMP(31);
           store_chunk_api<DIM, TERMS>(p, q, gv, a.save_x0, round_up(a.kin8, 16), tile, kc);
-          TSTAMP(32);
           p.conv_done(q);
-          TSTAMP(33);
           if (q + 1 < total_chunks) {
             if ((q + 1) % nk == 0) load_gather_idx<DIM>(a, tile_of(q + 1) * kTile, gi);  // first chunk of the next tile
             gather_chunk_api<DIM>(a, tile_of(q + 1) * kTile, (q + 1) % nk, gv, gi);
           }
           if (a.save_x0 && kc == nk - 1 && (a.kin8 & 8)) zero_chunk_bpt<B>(a.save_x0, round_up(a.kin8, 16), tile, nk);
-          TSTAMP(34);
         }
         pend.step(p, n_c4, epilogue_unit);  // one unit of the previous tile between two chunks of this one
-        TSTAMP(35);
       }
     }
     pend.drain(p, n_c4, epilogue_unit);
@@ -485,18 +461,16 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
 // The two linears share ONE MMA per (blade, split term): the weight images hold linear_right in plane rows [0, NS) and
 // linear_left in rows [NS, 2 NS), so the instruction shape is 128 x 2 NS x 8 and the A operand (the activations, the
 // expensive shared-memory read) is fetched once for both.  Blade b accumulates into columns [2 b NS, 2 (b+1) NS):
-// xr first, xl second.  TL: record the per-phase timeline (diagnostics build).
+// xr first, xl second.
 // ST (streamed weights, wide blocks): NS = a.ns2 < Cp output channels per pass, weight units streamed with the chunks; the
 // row statistics of the MVLayerNorm accumulate over the passes and the final scaling pass re-reads the product sum `o`
 // from the saved tensor (written by the same thread one pass earlier) instead of keeping it in TMEM.
-template <int DIM, bool TL, bool ST, int TERMS = 3>
+template <int DIM, bool ST, int TERMS = 3>
 __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, P = A::P, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
-  [[maybe_unused]] int dbg_n = 0;
-  TSTAMP(2);
   const int C = a.C, Cp = a.Cp, nk = Cp / 8;
   const int NS = ST ? a.ns2 : Cp;                      // output channels per pass
   const int npass = ST ? Cp / NS : 1;
@@ -529,7 +503,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   int q = 0;
   if (warp == 0) feed.prime(load);
 
-  TSTAMP(3);
   const uint32_t tcols = tmem_cols(2 * B * NS);
   if (warp == 0) tmem_alloc(tmem_slot, tcols);
   // the first elements of the small per-channel parameters are requested before the weights are staged (one exposed
@@ -543,7 +516,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
     const WJob wj[2] = {{wimg, a.wr, C, C, 0}, {wimg, a.wl, C, C, Cp}};  // right | left stacked along the image rows
     stage_weight_jobs<DIM, false, 2, TERMS>(wj, 2, img, 2 * Cp, Cp, wimg, (uint32_t)G * (uint32_t)NI * img);
   }
-  TSTAMP(4);
   if (tid < Cp * G) sn_s[tid] = tid < C * G ? sigmoidf_(pf_na) : 0.f;
   for (int i = tid + kThreads; i < Cp * G; i += kThreads) sn_s[i] = (i < C * G) ? sigmoidf_(a.na[i]) : 0.f;
   if (tid < Cp * P) wv_s[tid] = pf_wp0;
@@ -561,7 +533,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
   const bool wide_ok = aligned32(a.y) && (!a.res || aligned32(a.res));
   const uint32_t lane_base = (warp & 3) * 32;
 
-  TSTAMP(1);
   for (int t = 0; t < my_tiles; ++t) {
     const int64_t tile = cta_tile(t);
     const int64_t row0 = tile * kTile;
@@ -571,23 +542,16 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
     for (int ps = 0; ps < npass; ++ps) {
       const int n0 = ps * NS;
       for (int kc = 0; kc < nk; ++kc, ++q) {
-        TSTAMP(10);
         if (warp == 0) {  // issuer
           p.wait_full(q);
-          TSTAMP(14);
           feed.refill(q, load);
-          TSTAMP(16);
           if constexpr (ST) issue_chunk_mma<DIM, TERMS>(p, q, tbase, bcols, kc > 0, p.slot(q) + B * kPS, img, 0, 1, 0, bcols, 0, 0, idesc);
           else issue_chunk_mma<DIM, TERMS>(p, q, tbase, bcols, kc > 0, wimg, img, 0, 1, 0, bcols, kc, 0, idesc);
-          TSTAMP(15);
         } else {          // converters
           p.wait_landed(q);
-          TSTAMP(11);
           split_chunk<B, TERMS>(p, q);
-          TSTAMP(13);
         }
       }
-      TSTAMP(20);
       // y2 of this thread's first channel group is requested before waiting for the MMAs (left operand of the product)
       float4 y2v[B];
       if ((warp >> 2) < (NS >> 2)) {
@@ -595,7 +559,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
         for (int b = 0; b < B; ++b) y2v[b] = *reinterpret_cast<const float4*>(a.y2 + bpt_off(B, Cp, tile, b, (n0 >> 2) + (warp >> 2), r));
       }
       p.wait_mmas(q - 1);
-      TSTAMP(21);
       if (warp == 0) feed.refill_all(q, load);
       // ---- pass 1: per channel normalisation + weighted geometric product; o -> TMEM over xl (ST: -> save_o only)
       for (int c4 = warp >> 2; c4 < (NS >> 2); c4 += 4) {
@@ -653,13 +616,11 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
       if constexpr (!ST) tmem_wait_st();
       fence_before_sync();  // ST: the next pass's first MMA overwrites the accumulators (ordered by the full_bar chain)
     }
-    TSTAMP(22);
     // two copies, alternating by tile: a warp's reads of tile t and another warp's writes of tile t+1 are ordered by the
     // mbarrier chain of the next K loop anyway, but never touch the same words this way
     float* rowsum_t = rowsum_s + (t & 1) * 4 * kTile;
     rowsum_t[(warp >> 2) * kTile + r] = rs;
     __syncthreads();
-    TSTAMP(23);
     const float inv_mu = fast_rcp((rowsum_t[r] + rowsum_t[kTile + r] + rowsum_t[2 * kTile + r] + rowsum_t[3 * kTile + r]) / (float)C + kEps);
     // ---- pass 2: MVLayerNorm scale, residual, output (every channel group this thread handled in pass 1)
     for (int gc4 = warp >> 2; gc4 < (Cp >> 2); gc4 += 4) {
@@ -719,18 +680,11 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
       }
     }
     fence_before_sync();
-    TSTAMP(24);
   }
   tmem_teardown(warp, tbase, tcols);
-  TSTAMP(5);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-long long*& debug_buffer() {
-  static long long* p = nullptr;
-  return p;
-}
-
 // How the two forward kernels of a block of this shape run: weights resident in shared memory, or -- wide blocks --
 // streamed with the K chunks in passes of ns1 / ns2 output channels (tc_block.cuh).  The choice is made for the default
 // (split) weight images, so both numeric modes run a shape with the same plan; nimg = 1 (single-pass TF32) only shrinks
@@ -822,7 +776,6 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   a.w1 = d.w1; a.b1 = d.b1; a.sa = d.sa; a.sb = d.sb; a.wr = d.wr; a.na = d.na; a.wl = d.wl; a.bl = d.bl; a.wp = d.wp; a.la = d.la;
   a.save_y1 = d.save_y1; a.y2 = d.save_y2; a.save_xr = d.save_xr; a.save_o = d.save_o; a.save_x0 = d.save_x0;
   a.y = d.y; a.res = d.res; a.out_bpt = d.out_bpt; a.has_b1 = d.has_b1;
-  a.dbg = debug_buffer();
   if (!a.y2 || !a.y) return CSMPN_ERR_BAD_ARG;
   if (a.in_bpt && (d.mode != 0 || d.c1 || d.c2)) return CSMPN_ERR_BAD_ARG;
   if (d.mode == 2 && (d.vt_k < 1 || d.vt_k > 3 || d.vt_fp < 1 || d.c0 % (d.vt_k * d.vt_fp) || d.c1 || d.c2 || !d.src)) return CSMPN_ERR_BAD_ARG;
@@ -856,10 +809,6 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
     kern<<<grid, kThreads, smem_bytes, stream>>>(a);
     return CSMPN_OK;
   };
-  long long* const dbg_buf = a.dbg;  // diagnostics build: CSMPN_DBG_KERNEL=f1 records the first kernel, default the second
-  const char* dbg_k = getenv("CSMPN_DBG_KERNEL");
-  const bool dbg_f1 = dbg_k && dbg_k[0] == 'f' && dbg_k[1] == '1';
-  a.dbg = dbg_f1 ? dbg_buf : nullptr;
   if (mask & 1) {
     const bool overlap = !p.st1 && use_overlapped_epilogue(B, a.Cp);
     int rc = overlap ? (a.in_bpt ? run(tc_f1db_kernel<DIM, true, TERMS>, p.s1) : run(tc_f1db_kernel<DIM, false, TERMS>, p.s1))
@@ -868,14 +817,8 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_f1_kernel");
   }
-  a.dbg = dbg_f1 ? nullptr : dbg_buf;
   if (mask & 2) {
-    int rc;
-#ifdef CSMPN_DEBUG_TOOLS
-    if (a.dbg && !p.st2) rc = run(tc_f2_kernel<DIM, true, false, TERMS>, p.s2);
-    else
-#endif
-    rc = p.st2 ? run(tc_f2_kernel<DIM, false, true, TERMS>, p.s2) : run(tc_f2_kernel<DIM, false, false, TERMS>, p.s2);
+    int rc = p.st2 ? run(tc_f2_kernel<DIM, true, TERMS>, p.s2) : run(tc_f2_kernel<DIM, false, TERMS>, p.s2);
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_f2_kernel");
   }
@@ -889,7 +832,6 @@ int tc_block_fwd(int dim, const csmpn_block_desc* d, cudaStream_t stream) {
   if (dim == 3) return d->tf32 ? tcb::launch_fwd<3, 1>(*d, stream) : tcb::launch_fwd<3, 3>(*d, stream);
   return CSMPN_ERR_UNSUPPORTED;
 }
-void tc_set_debug_buffer(long long* p) { tcb::debug_buffer() = p; }
 int64_t tc_block_fwd_workspace(int dim, const csmpn_block_desc* d) {
   if (dim == 2) return tcb::fwd_ws_bytes<2>(*d);
   if (dim == 3) return tcb::fwd_ws_bytes<3>(*d);

@@ -10,7 +10,7 @@
 // MN-major TF32 operands (K = plane rows, MMA rows = channels; the weight-gradient GEMMs) only exist in the
 // SWIZZLE_128B_BASE32B layout: 32-channel groups of [rows][128 B], the 32-byte unit index of a row xor-ed with
 // (row & 3); LBO = byte stride between 32-channel groups, SBO = 512 (groups of 4 rows), one K=8 step = 1024 bytes.
-// Every encoding here was pinned on a B200 with tools/tc_probe_raw.py (profiles/r01_tc_probe.log).
+// Every encoding here was pinned on a B200 (profiles/r01_tc_probe.log).
 // fp32 accuracy on the TF32 pipe comes from the usual error-compensated split  x = hi + lo  with hi = x with the low
 // 13 mantissa bits cleared (exactly representable in TF32) and three MMAs per product: hi*hi + hi*lo + lo*hi.
 // Single-pass TF32 mode (csmpn_block_desc.tf32, kernels instantiated with TERMS = 1) rounds each operand to nearest TF32
