@@ -6,11 +6,11 @@ import pytest
 import torch
 
 from conftest import LAYER_FIXTURES, assert_close, load_golden, tols
+from egcl_harness import (DEV, LEAVES, assert_all_close, cemlp_model, egcl_inputs, egcl_model, grads, load_params, mods,
+                          oracle_egcl, run_egcl)
 from oracle import layers_ref as R
 
 pytestmark = pytest.mark.gpu
-
-DEV = "cuda"
 
 
 @pytest.fixture(params=["fused", "unit"])
@@ -20,27 +20,10 @@ def path(request, monkeypatch):
     return request.param
 
 
-def _mods():
-    from csmpn_b200.algebra.cliffordalgebra import CliffordAlgebra
-    from csmpn_b200.models import cegnn_utils as M
-
-    return CliffordAlgebra, M
-
-
-def _load(module, params):
-    missing, unexpected = module.load_state_dict({k: v for k, v in params.items()}, strict=False)
-    assert not unexpected, unexpected
-    assert all("algebra" in m for m in missing), missing
-
-
-def _grads(out, cot, tensors):
-    return torch.autograd.grad(out, tensors, cot.to(out.device), allow_unused=True)
-
-
 @pytest.fixture(scope="module", params=LAYER_FIXTURES)
 def fx(request):
     f = load_golden(request.param)
-    CliffordAlgebra, _ = _mods()
+    CliffordAlgebra, _ = mods()
     f["alg"] = CliffordAlgebra(f["metric"]).to(DEV)
     f["ralg"] = R.RefAlgebra(f["metric"])
     return f
@@ -68,7 +51,7 @@ def test_geometric_product(fx):
     a, b = g["a"].to(DEV).requires_grad_(), g["b"].to(DEV).requires_grad_()
     out = alg.geometric_product(a, b)
     assert_close(out, g["out"], FWD, "gp")
-    ga, gb = _grads(out, g["cot"], [a, b])
+    ga, gb = grads(out, g["cot"], [a, b])
     assert_close(ga, g["ga"], GRAD, "ga")
     assert_close(gb, g["gb"], GRAD, "gb")
     # forms
@@ -89,7 +72,7 @@ def test_geometric_product_broadcast_and_blades(fx):
     ref = R.geometric_product(ralg, ar, br)
     assert_close(out, ref, FWD, "bcast gp")
     cot = torch.randn(37, ralg.B, generator=gen)
-    ga, gb = _grads(out, cot, [ad, bd])
+    ga, gb = grads(out, cot, [ad, bd])
     gar, gbr = torch.autograd.grad(ref, [ar, br], cot)
     assert_close(ga, gar, GRAD, "bcast ga")
     assert_close(gb, gbr, GRAD, "bcast gb")
@@ -98,7 +81,7 @@ def test_geometric_product_broadcast_and_blades(fx):
 @pytest.mark.parametrize("sub", [1, 0])
 def test_mvlinear(fx, sub):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
+    _, M = mods()
     alg, g = fx["alg"], fx[f"mvlinear_{sub}"]
     m = M.MVLinear(alg, g["x"].shape[1], g["y"].shape[1], subspaces=bool(sub)).to(DEV)
     with torch.no_grad():
@@ -107,7 +90,7 @@ def test_mvlinear(fx, sub):
     x = g["x"].to(DEV).requires_grad_()
     y = m(x)
     assert_close(y, g["y"], FWD, "mvlinear")
-    gx, gw, gb = _grads(y, g["cot"], [x, m.weight, m.bias])
+    gx, gw, gb = grads(y, g["cot"], [x, m.weight, m.bias])
     assert_close(gx, g["gx"], GRAD, "gx")
     assert_close(gw, g["gw"], GRAD, "gw")
     assert_close(gb, g["gb"], GRAD, "gb")
@@ -115,7 +98,7 @@ def test_mvlinear(fx, sub):
 
 def test_mvsilu(fx):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
+    _, M = mods()
     alg, g = fx["alg"], fx["mvsilu"]
     m = M.MVSiLU(alg, g["x"].shape[1]).to(DEV)
     with torch.no_grad():
@@ -123,13 +106,13 @@ def test_mvsilu(fx):
     x = g["x"].to(DEV).requires_grad_()
     y = m(x)
     assert_close(y, g["y"], FWD, "mvsilu")
-    for got, key in zip(_grads(y, g["cot"], [x, m.a, m.b]), ("gx", "ga", "gb")):
+    for got, key in zip(grads(y, g["cot"], [x, m.a, m.b]), ("gx", "ga", "gb")):
         assert_close(got, g[key], GRAD, key)
 
 
 def test_mvnorm(fx):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
+    _, M = mods()
     alg, g = fx["alg"], fx["mvnorm"]
     m = M.NormalizationLayer(alg, g["x"].shape[1]).to(DEV)
     with torch.no_grad():
@@ -137,13 +120,13 @@ def test_mvnorm(fx):
     x = g["x"].to(DEV).requires_grad_()
     y = m(x)
     assert_close(y, g["y"], FWD, "mvnorm")
-    for got, key in zip(_grads(y, g["cot"], [x, m.a]), ("gx", "ga")):
+    for got, key in zip(grads(y, g["cot"], [x, m.a]), ("gx", "ga")):
         assert_close(got, g[key], GRAD, key)
 
 
 def test_mvlayernorm(fx):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
+    _, M = mods()
     alg, g = fx["alg"], fx["mvlayernorm"]
     m = M.MVLayerNorm(alg, g["x"].shape[1]).to(DEV)
     with torch.no_grad():
@@ -151,21 +134,20 @@ def test_mvlayernorm(fx):
     x = g["x"].to(DEV).requires_grad_()
     y = m(x)
     assert_close(y, g["y"], FWD, "mvlayernorm")
-    for got, key in zip(_grads(y, g["cot"], [x, m.a]), ("gx", "ga")):
+    for got, key in zip(grads(y, g["cot"], [x, m.a]), ("gx", "ga")):
         assert_close(got, g[key], GRAD, key)
 
 
 def test_sgp(fx):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
+    _, M = mods()
     alg, g = fx["alg"], fx["sgp"]
-    m = M.SteerableGeometricProductLayer(alg, g["x"].shape[1]).to(DEV)
-    _load(m, g["params"])
+    m = load_params(M.SteerableGeometricProductLayer(alg, g["x"].shape[1]).to(DEV), g["params"])
     x = g["x"].to(DEV).requires_grad_()
     y = m(x)
     assert_close(y, g["y"], FWD, "sgp")
     plist = list(m.named_parameters())
-    got = _grads(y, g["cot"], [x] + [p for _, p in plist])
+    got = grads(y, g["cot"], [x] + [p for _, p in plist])
     assert_close(got[0], g["gx"], GRAD, "gx")
     for (n, _), gi in zip(plist, got[1:]):
         assert_close(gi, g["grads"][n], GRAD, n)
@@ -173,16 +155,13 @@ def test_sgp(fx):
 
 def test_cemlp(fx, path):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
-    alg, g = fx["alg"], fx["cemlp"]
-    C = g["y"].shape[1]
-    m = M.CEMLP(alg, g["x"].shape[1], C, C, n_layers=2).to(DEV)
-    _load(m, g["params"])
+    g = fx["cemlp"]
+    m = cemlp_model(fx["metric"], g["x"].shape[1], g["y"].shape[1], 2, g["params"])
     x = g["x"].to(DEV).requires_grad_()
     y = m(x)
     assert_close(y, g["y"], FWD, "cemlp")
     plist = list(m.named_parameters())
-    got = _grads(y, g["cot"], [x] + [p for _, p in plist])
+    got = grads(y, g["cot"], [x] + [p for _, p in plist])
     assert_close(got[0], g["gx"], GRAD, "gx")
     for (n, _), gi in zip(plist, got[1:]):
         assert_close(gi, g["grads"][n], GRAD, n)
@@ -191,21 +170,12 @@ def test_cemlp(fx, path):
 @pytest.mark.parametrize("aggr", ["sum", "mean"])
 def test_egcl(fx, aggr, path):
     FWD, GRAD = tols(fx)
-    _, M = _mods()
-    alg, g = fx["alg"], fx[f"egcl_{aggr}"]
-    C, T = g["h"].shape[1], g["node_attr"].shape[1]
-    m = M.EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=aggr).to(DEV)
-    _load(m, g["params"])
-    h, ea, na = (g[k].to(DEV).requires_grad_() for k in ("h", "edge_attr", "node_attr"))
-    y = m(h, g["edge_index"].to(DEV), ea, na)
-    assert_close(y, g["y"], FWD, "egcl")
-    plist = list(m.named_parameters())
-    got = _grads(y, g["cot"], [h, ea, na] + [p for _, p in plist])
-    assert_close(got[0], g["gh"], GRAD, "gh")
-    assert_close(got[1], g["gedge_attr"], GRAD, "gedge_attr")
-    assert_close(got[2], g["gnode_attr"], GRAD, "gnode_attr")
-    for (n, _), gi in zip(plist, got[3:]):
-        assert_close(gi, g["grads"][n], GRAD, n)
+    g = fx[f"egcl_{aggr}"]
+    m = egcl_model(fx["metric"], g["h"].shape[1], g["node_attr"].shape[1], aggr, g["params"])
+    inp = {"params": g["params"], "h": g["h"], "ei": g["edge_index"], "ea": g["edge_attr"], "na": g["node_attr"],
+           "cot": g["cot"]}
+    ref = {"h": g["gh"], "edge_attr": g["gedge_attr"], "node_attr": g["gnode_attr"], **g["grads"]}
+    assert_all_close(run_egcl(m, inp, tuple(LEAVES), "tensor"), (g["y"], ref), FWD, GRAD, "egcl")
 
 
 # ------------------------------------------------------------------------------------------------
@@ -220,61 +190,23 @@ CASES = [
 ]
 
 
-def _block_diag_graph(n_cplx, n, e, gen):
-    src = torch.randint(0, n, (n_cplx, e), generator=gen)
-    dst = torch.randint(0, n, (n_cplx, e), generator=gen)
-    off = (torch.arange(n_cplx) * n).unsqueeze(1)
-    return torch.stack([(src + off).reshape(-1), (dst + off).reshape(-1)])
-
-
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
 def test_egcl_vs_oracle(case, path):
     name, metric, C, T, ncx, n, e, aggr = case
-    CliffordAlgebra, M = _mods()
-    gen = torch.Generator().manual_seed(hash(name) % 1000)
-    ralg = R.RefAlgebra(metric)
-    B = ralg.B
-    params = R.init_egcl_params(ralg, C, T, gen)
-    N = ncx * n
-    h = torch.randn(N, C, B, generator=gen)
-    ei = _block_diag_graph(ncx, n, e, gen)
-    types = torch.randint(0, T, (N,), generator=gen)
-    emb = torch.randn(T, T, generator=gen)
-    na = torch.zeros(N, T, B)
-    na[..., 0] = emb[types]
-    ea = torch.cat([na[ei[0]], na[ei[1]]], 1)
-    cot = torch.randn(N, C, B, generator=gen)
-
-    hr = h.clone().requires_grad_()
-    pr = {k: v.clone().requires_grad_() for k, v in params.items()}
-    yr = R.egcl(ralg, hr, ei, ea, na, pr, aggr=aggr)
-    names = list(pr)
-    gr = torch.autograd.grad(yr, [hr] + [pr[k] for k in names], cot)
-
-    alg = CliffordAlgebra(metric).to(DEV)
-    m = M.EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=aggr).to(DEV)
-    _load(m, params)
-    hd = h.to(DEV).requires_grad_()
-    y = m(hd, ei.to(DEV), ea.to(DEV), na.to(DEV))
-    assert_close(y, yr, 1e-5, f"{name} fwd")
-    pd = dict(m.named_parameters())
-    got = _grads(y, cot, [hd] + [pd[k] for k in names])
-    assert_close(got[0], gr[0], 1e-4, f"{name} gh")
-    for k, a, b in zip(names, got[1:], gr[1:]):
-        assert_close(a, b, 1e-4, f"{name} {k}")
+    inp = egcl_inputs(case)
+    ref = oracle_egcl(inp, torch.float32, ("h",), "tensor")
+    m = egcl_model(metric, C, T, aggr, inp["params"])
+    assert_all_close(run_egcl(m, inp, ("h",), "tensor"), ref, 1e-5, 1e-4, name)
 
 
 def test_egcl_empty_and_ragged(path):
     """no pairs at all; a receiver with hundreds of pairs; N not a multiple of any tile."""
-    CliffordAlgebra, M = _mods()
     gen = torch.Generator().manual_seed(9)
     ralg = R.RefAlgebra((1, 1, 1))
     C, T, N = 8, 3, 13
     params = R.init_egcl_params(ralg, C, T, gen)
-    alg = CliffordAlgebra((1, 1, 1)).to(DEV)
     for aggr in ("sum", "mean"):
-        m = M.EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=aggr).to(DEV)
-        _load(m, params)
+        m = egcl_model((1, 1, 1), C, T, aggr, params)
         for ei in (torch.zeros(2, 0, dtype=torch.long),
                    torch.stack([torch.randint(0, N, (300,), generator=gen), torch.full((300,), 5)])):
             h = torch.randn(N, C, 8, generator=gen)
@@ -326,13 +258,11 @@ def test_csr_is_stable_sort(small, monkeypatch):
 def test_equivariance_with_correct_inverse():
     """f(rho_w(x)) = rho_w(f(x)) for a random rotor, using w^-1 = beta(w)/q(w) (the reference's ``inverse`` is not
     norm-preserving, SURVEY.md appendix B)."""
-    CliffordAlgebra, M = _mods()
     gen = torch.Generator().manual_seed(4)
     ralg = R.RefAlgebra((1, 1, 1))
-    alg = CliffordAlgebra((1, 1, 1)).to(DEV)
     C = 8
-    m = M.CEMLP(alg, C, C, C, n_layers=2).to(DEV)
-    _load(m, R.init_cemlp_params(ralg, C, C, C, 2, gen))
+    m = cemlp_model((1, 1, 1), C, C, 2, R.init_cemlp_params(ralg, C, C, C, 2, gen))
+    alg = m.algebra
     v1, v2 = torch.zeros(8), torch.zeros(8)
     v1[1:4] = torch.randn(3, generator=gen); v2[1:4] = torch.randn(3, generator=gen)
     w = R.geometric_product(ralg, v1, v2)
@@ -353,7 +283,7 @@ def test_versor_utilities_match_the_reference():
     """the off-path helpers of CliffordAlgebra (alpha_w, inverse, rho, sandwich, output_blades, parity, eta,
     reduce_geometric_product, random_vector / versor shapes) against the reference's definitions on the same inputs
     (tests/golden/versor.pt, made by tests/golden/make_golden_versor.py)."""
-    CliffordAlgebra, _ = _mods()
+    CliffordAlgebra, _ = mods()
     gold = load_golden("versor.pt")
     for metric in ((1, 1), (1, 1, 1)):
         ref = gold[metric]

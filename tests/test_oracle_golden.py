@@ -4,11 +4,8 @@ import pytest
 import torch
 
 from conftest import LAYER_FIXTURES, assert_close, load_golden, tols
+from egcl_harness import grads
 from oracle import layers_ref as R
-
-
-def _grads(out, cot, tensors):
-    return torch.autograd.grad(out, tensors, cot, allow_unused=True)
 
 
 @pytest.fixture(scope="module", params=LAYER_FIXTURES)
@@ -34,7 +31,7 @@ def test_geometric_product(fx):
     a, b = g["a"].clone().requires_grad_(), g["b"].clone().requires_grad_()
     out = R.geometric_product(alg, a, b)
     assert_close(out, g["out"], FWD_TOL, "gp")
-    ga, gb = _grads(out, g["cot"], [a, b])
+    ga, gb = grads(out, g["cot"], [a, b])
     assert_close(ga, g["ga"], GRAD_TOL, "gp ga")
     assert_close(gb, g["gb"], GRAD_TOL, "gp gb")
 
@@ -54,7 +51,7 @@ def test_mvlinear(fx, sub):
     x, w, b = (g[k].clone().requires_grad_() for k in ("x", "weight", "bias"))
     y = R.mvlinear(alg, x, w, b)
     assert_close(y, g["y"], FWD_TOL, "mvlinear")
-    gx, gw, gb = _grads(y, g["cot"], [x, w, b])
+    gx, gw, gb = grads(y, g["cot"], [x, w, b])
     assert_close(gx, g["gx"], GRAD_TOL, "gx")
     assert_close(gw, g["gw"], GRAD_TOL, "gw")
     assert_close(gb, g["gb"], GRAD_TOL, "gb")
@@ -66,7 +63,7 @@ def test_mvsilu(fx):
     x, a, b = (g[k].clone().requires_grad_() for k in ("x", "a", "b"))
     y = R.mvsilu(alg, x, a, b)
     assert_close(y, g["y"], FWD_TOL, "mvsilu")
-    for got, key in zip(_grads(y, g["cot"], [x, a, b]), ("gx", "ga", "gb")):
+    for got, key in zip(grads(y, g["cot"], [x, a, b]), ("gx", "ga", "gb")):
         assert_close(got, g[key], GRAD_TOL, key)
 
 
@@ -76,7 +73,7 @@ def test_mvnorm(fx):
     x, a = (g[k].clone().requires_grad_() for k in ("x", "a"))
     y = R.normalization(alg, x, a)
     assert_close(y, g["y"], FWD_TOL, "mvnorm")
-    for got, key in zip(_grads(y, g["cot"], [x, a]), ("gx", "ga")):
+    for got, key in zip(grads(y, g["cot"], [x, a]), ("gx", "ga")):
         assert_close(got, g[key], GRAD_TOL, key)
 
 
@@ -86,7 +83,7 @@ def test_mvlayernorm(fx):
     x, a = (g[k].clone().requires_grad_() for k in ("x", "a"))
     y = R.mvlayernorm(alg, x, a)
     assert_close(y, g["y"], FWD_TOL, "mvlayernorm")
-    for got, key in zip(_grads(y, g["cot"], [x, a]), ("gx", "ga")):
+    for got, key in zip(grads(y, g["cot"], [x, a]), ("gx", "ga")):
         assert_close(got, g[key], GRAD_TOL, key)
 
 
@@ -98,7 +95,7 @@ def test_sgp(fx):
     y = R.sgp(alg, x, p, "")
     assert_close(y, g["y"], FWD_TOL, "sgp")
     names = list(p)
-    got = _grads(y, g["cot"], [x] + [p[n] for n in names])
+    got = grads(y, g["cot"], [x] + [p[n] for n in names])
     assert_close(got[0], g["gx"], GRAD_TOL, "gx")
     for n, gi in zip(names, got[1:]):
         assert_close(gi, g["grads"][n], GRAD_TOL, n)
@@ -112,7 +109,7 @@ def test_cemlp(fx):
     y = R.cemlp(alg, x, p)
     assert_close(y, g["y"], FWD_TOL, "cemlp")
     names = list(p)
-    got = _grads(y, g["cot"], [x] + [p[n] for n in names])
+    got = grads(y, g["cot"], [x] + [p[n] for n in names])
     assert_close(got[0], g["gx"], GRAD_TOL, "gx")
     for n, gi in zip(names, got[1:]):
         assert_close(gi, g["grads"][n], GRAD_TOL, n)
@@ -127,7 +124,7 @@ def test_egcl(fx, aggr):
     y = R.egcl(alg, h, g["edge_index"], ea, na, p, aggr=aggr)
     assert_close(y, g["y"], FWD_TOL, "egcl")
     names = list(p)
-    got = _grads(y, g["cot"], [h, ea, na] + [p[n] for n in names])
+    got = grads(y, g["cot"], [h, ea, na] + [p[n] for n in names])
     assert_close(got[0], g["gh"], GRAD_TOL, "gh")
     assert_close(got[1], g["gedge_attr"], GRAD_TOL, "gedge_attr")
     assert_close(got[2], g["gnode_attr"], GRAD_TOL, "gnode_attr")

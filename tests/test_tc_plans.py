@@ -15,10 +15,10 @@ import functools
 import pytest
 import torch
 
+from egcl_harness import DEV, block_diag_graph, cemlp_model, egcl_model, mods
 from oracle import layers_ref as R
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda"
 T = 3  # node-attribute types of the EGCL cases: edge_attr has 2T channels
 
 # global criterion (BASELINE.json north star): max-norm relative to the fp64 oracle
@@ -112,13 +112,6 @@ def _block_shapes(case):
     return [(shape[1], C), (C, C)]
 
 
-def _mods():
-    from csmpn_b200.algebra.cliffordalgebra import CliffordAlgebra
-    from csmpn_b200.models import cegnn_utils as M
-
-    return CliffordAlgebra, M
-
-
 # ------------------------------------------------------------------------------------------------ inputs and oracle
 @functools.lru_cache(maxsize=None)
 def _inputs(name):
@@ -131,13 +124,11 @@ def _inputs(name):
         _, ncx, n, e, aggr = shape
         params = R.init_egcl_params(ralg, C, T, gen)
         N = ncx * n
-        off = (torch.arange(ncx) * n).unsqueeze(1)
-        src = (torch.randint(0, n, (ncx, e), generator=gen) + off).reshape(-1)
-        dst = (torch.randint(0, n, (ncx, e), generator=gen) + off).reshape(-1)
+        ei = block_diag_graph(ncx, n, e, gen)
         h = torch.randn(N, C, B, generator=gen)
         na = torch.zeros(N, T, B)
         na[..., 0] = torch.randn(T, T, generator=gen)[torch.randint(0, T, (N,), generator=gen)]
-        return {"params": params, "leaves": {"h": h, "node_attr": na}, "ei": torch.stack([src, dst]), "aggr": aggr,
+        return {"params": params, "leaves": {"h": h, "node_attr": na}, "ei": ei, "aggr": aggr,
                 "cot": torch.randn(N, C, B, generator=gen)}
     _, cin, rows = shape
     params = R.init_cemlp_params(ralg, cin, C, C, 2, gen)
@@ -165,18 +156,12 @@ def _oracle(name, dtype):
 
 def _model(name):
     _, dim, C, shape = BY_NAME[name][:4]
-    CliffordAlgebra, M = _mods()
-    alg = CliffordAlgebra(_metric(dim)).to(DEV)
+    params = _inputs(name)["params"]
     if shape[0] == "egcl":
-        m = M.EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=shape[4])
-        blocks = list(m.edge_model.layers) + list(m.node_model.layers)
-    else:
-        m = M.CEMLP(alg, shape[1], C, C, n_layers=2)
-        blocks = list(m.layers)
-    m = m.to(DEV)
-    missing, unexpected = m.load_state_dict(dict(_inputs(name)["params"]), strict=False)
-    assert not unexpected and all("algebra" in k for k in missing), (missing, unexpected)
-    return alg, m, blocks
+        m = egcl_model(_metric(dim), C, T, shape[4], params)
+        return m.algebra, m, list(m.edge_model.layers) + list(m.node_model.layers)
+    m = cemlp_model(_metric(dim), shape[1], C, 2, params)
+    return m.algebra, m, list(m.layers)
 
 
 class _BlockCallSpy:
@@ -224,7 +209,7 @@ def _ours(name, monkeypatch):
     pd = dict(m.named_parameters())
     n0 = _lib.lib().csmpn_launch_count()
     if shape[0] == "egcl":
-        _, M = _mods()
+        _, M = mods()
         na = leaves["node_attr"]
         y = m(leaves["h"], inp["ei"].to(DEV), M.PairedNodeAttr(na), na)
     else:

@@ -10,9 +10,11 @@ import pytest
 import torch
 
 from conftest import ROOT, load_golden, rel_err
+from egcl_harness import (CASES, DEV, WIDE, assert_all_equal, bench_inputs, egcl_inputs, egcl_model, mods, oracle_egcl,
+                          run_egcl)
 from oracle import layers_ref as R
 
-DEV = "cuda"
+PAIRED = ("h", "node_attr")
 
 # max-norm relative error against the fp64 oracle in TF32 mode.  Largest values measured on a B200 over every case here
 # (DESIGN.md 4.1): forward 1.3e-3, worst gradient 6.0e-3 (both NBA-shaped, Cl(2,0)); md17 model 7.1e-3.  Each bound has at
@@ -87,82 +89,45 @@ def precision(monkeypatch):
     torch.backends.cuda.matmul.fp32_precision = old
 
 
-def _cases():
-    from test_tc_block import CASES, WIDE
-
-    return CASES, WIDE
-
-
-def _mods():
-    from csmpn_b200.algebra.cliffordalgebra import CliffordAlgebra
-    from csmpn_b200.models import cegnn_utils as M
-
-    return CliffordAlgebra, M
-
-
-def _layer(metric, C, T, aggr, params):
-    CliffordAlgebra, M = _mods()
-    alg = CliffordAlgebra(metric).to(DEV)
-    m = M.EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=aggr).to(DEV)
-    missing, unexpected = m.load_state_dict(dict(params), strict=False)
-    assert not unexpected and all("algebra" in k for k in missing), (missing, unexpected)
-    return m
-
-
-def _step(m, h, ei, na, cot, names):
+def _step(m, inp):
     """layer forward + (grad h, grad node_attr, every parameter gradient); edge_attr = node_attr[src] | node_attr[dst]"""
-    _, M = _mods()
-    hd, nad = h.to(DEV).requires_grad_(), na.to(DEV).requires_grad_()
-    y = m(hd, ei.to(DEV), M.PairedNodeAttr(nad), nad)
-    pd = dict(m.named_parameters())
-    g = torch.autograd.grad(y, [hd, nad] + [pd[k] for k in names], cot.to(DEV))
-    torch.cuda.synchronize()
-    return y.detach(), [t.detach() for t in g]
+    return run_egcl(m, inp, PAIRED, "paired")
 
 
-def _oracle64(ralg, params, h, ei, na, cot, aggr):
-    """forward and every gradient of the fp64 oracle (CPU)"""
-    hr, nar = h.double().requires_grad_(), na.double().requires_grad_()
-    pr = {k: v.double().requires_grad_() for k, v in params.items()}
-    yr = R.egcl(ralg, hr, ei, torch.cat([nar[ei[0]], nar[ei[1]]], 1), nar, pr, aggr=aggr)
-    names = list(pr)
-    gr = torch.autograd.grad(yr, [hr, nar] + [pr[k] for k in names], cot.double())
-    return yr.detach(), [t.detach() for t in gr], names
+def _layer(case):
+    name, metric, C, T, ncx, n, e, aggr = case
+    inp = egcl_inputs(case)
+    return egcl_model(metric, C, T, aggr, inp["params"]), inp
 
 
-def _oracle_gpu_tf32(ralg, params, h, ei, na, aggr):
+def _oracle_gpu_tf32(inp):
     """the oracle itself in fp32 on the GPU under the current matmul precision (its linears are einsums): what a
     plain-PyTorch implementation computes with TF32 matmuls"""
     import copy
 
+    ralg = inp["ralg"]
     g = copy.copy(ralg)
     for k, v in vars(ralg).items():
         if torch.is_tensor(v):
             setattr(g, k, v.to(DEV))
-    p = {k: v.to(DEV) for k, v in params.items()}
-    nd, eid = na.to(DEV), ei.to(DEV)
+    p = {k: v.to(DEV) for k, v in inp["params"].items()}
+    nd, eid = inp["na"].to(DEV), inp["ei"].to(DEV)
     with torch.no_grad(), torch.device(DEV):  # the oracle creates its scratch tensors without a device argument
-        return R.egcl(g, h.to(DEV), eid, torch.cat([nd[eid[0]], nd[eid[1]]], 1), nd, p, aggr=aggr)
+        return R.egcl(g, inp["h"].to(DEV), eid, torch.cat([nd[eid[0]], nd[eid[1]]], 1), nd, p, aggr=inp["aggr"])
 
 
-def _errors(y, g, yr, gr):
-    return rel_err(y, yr), max(rel_err(a, b) for a, b in zip(g, gr))
+def _errors(res, ref):
+    return rel_err(res[0], ref[0]), max(rel_err(res[1][k], r) for k, r in ref[1].items())
 
 
-def _check_vs_oracle(case, precision):
-    from test_tc_block import _inputs
-
-    name, metric, C, T, ncx, n, e, aggr = case
-    ralg, params, h, ei, _, na, cot = _inputs(case)
-    yr, gr, names = _oracle64(ralg, params, h, ei, na, cot, aggr)
-    m = _layer(metric, C, T, aggr, params)
+def _check_vs_oracle(name, m, inp, precision):
+    ref = oracle_egcl(inp, torch.float64, PAIRED, "paired")
     res = {}
     for mode in ("ieee", "tf32"):
         precision(mode)
-        res[mode] = _step(m, h, ei, na, cot, names)
-    precision("tf32")
-    e_ref = rel_err(_oracle_gpu_tf32(ralg, params, h, ei, na, aggr), yr)
-    e_def, e_tf = _errors(*res["ieee"], yr, gr), _errors(*res["tf32"], yr, gr)
+        res[mode] = _step(m, inp)
+    e_ref = rel_err(_oracle_gpu_tf32(inp), ref[0])  # under TF32, the mode set last
+    e_def, e_tf = _errors(res["ieee"], ref), _errors(res["tf32"], ref)
     print(f"[tf32] {name}: fp64-oracle error fwd / worst grad: default {e_def[0]:.2e} / {e_def[1]:.2e}, "
           f"tf32 {e_tf[0]:.2e} / {e_tf[1]:.2e}; oracle on the GPU with TF32 matmuls fwd {e_ref:.2e}")
     assert e_tf[0] <= TF32_FWD_TOL and e_tf[1] <= TF32_GRAD_TOL, (name, e_tf)
@@ -172,16 +137,16 @@ def _check_vs_oracle(case, precision):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("idx", range(6), ids=["motion", "md17", "nba", "odd_c", "tiny", "one_tile_exact"])
-def test_tf32_layer_vs_fp64_oracle(idx, precision):
-    _check_vs_oracle(_cases()[0][idx], precision)
+@pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
+def test_tf32_layer_vs_fp64_oracle(case, precision):
+    _check_vs_oracle(case[0], *_layer(case), precision)
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("idx", range(6), ids=["cl3_c64", "cl3_c128", "cl3_c256", "cl2_c128", "cl2_c64", "cl3_c64_multi_tile"])
-def test_tf32_wide_layer_vs_fp64_oracle(idx, precision):
+@pytest.mark.parametrize("case", WIDE, ids=[c[0] for c in WIDE])
+def test_tf32_wide_layer_vs_fp64_oracle(case, precision):
     """streamed weights (the [pass][K chunk][grade][2][R][4] units) and the slab-wise weight-gradient launches"""
-    _check_vs_oracle(_cases()[1][idx], precision)
+    _check_vs_oracle(case[0], *_layer(case), precision)
 
 
 @pytest.mark.gpu
@@ -191,89 +156,56 @@ def test_tf32_md17_bench_batch_vs_fp64_oracle(precision):
     import bench
 
     b = bench.make_batch("md17", 100, 1000)
-    metric, C, aggr = b["metric"], b["C"], b["aggr"]
-    ralg = R.RefAlgebra(metric)
-    params = R.init_egcl_params(ralg, C, 3, torch.Generator().manual_seed(7))
-    case = ("md17_bench", metric, C, 3, None, None, None, aggr)
-    h, ei, na, cot = b["h"], b["edge_index"], b["node_attr"], b["cot"]
-    yr, gr, names = _oracle64(ralg, params, h, ei, na, cot, aggr)
-    m = _layer(metric, C, 3, aggr, params)
-    res = {}
-    for mode in ("ieee", "tf32"):
-        precision(mode)
-        res[mode] = _step(m, h, ei, na, cot, names)
-    e_ref = rel_err(_oracle_gpu_tf32(ralg, params, h, ei, na, aggr), yr)
-    e_def, e_tf = _errors(*res["ieee"], yr, gr), _errors(*res["tf32"], yr, gr)
-    print(f"[tf32] {case[0]}: fp64-oracle error fwd / worst grad: default {e_def[0]:.2e} / {e_def[1]:.2e}, "
-          f"tf32 {e_tf[0]:.2e} / {e_tf[1]:.2e}; oracle on the GPU with TF32 matmuls fwd {e_ref:.2e}")
-    assert e_tf[0] <= TF32_FWD_TOL and e_tf[1] <= TF32_GRAD_TOL, e_tf
-    assert e_tf[0] > e_def[0] and e_tf[1] > e_def[1], (e_tf, e_def)
-
-
-def _small():
-    from test_tc_block import _inputs
-
-    case = _cases()[0][1]  # md17-shaped, several tiles
-    name, metric, C, T, ncx, n, e, aggr = case
-    ralg, params, h, ei, _, na, cot = _inputs(case)
-    return metric, C, T, aggr, params, h, ei, na, cot, list(params)
+    inp = bench_inputs(b)
+    _check_vs_oracle("md17_bench", egcl_model(b["metric"], b["C"], 3, b["aggr"], inp["params"]), inp, precision)
 
 
 @pytest.mark.gpu
 def test_no_state_survives_a_tf32_run(precision):
     """A default run after TF32 runs equals a default run of a fresh model bit for bit (no cached TF32 weight images,
     no sticky descriptor field); wide blocks included (streamed weight images in the workspace)."""
-    from test_tc_block import _inputs
-
-    for case in (_cases()[0][1], _cases()[1][0]):
-        name, metric, C, T, ncx, n, e, aggr = case
-        ralg, params, h, ei, _, na, cot = _inputs(case)
-        names = list(params)
-        m = _layer(metric, C, T, aggr, params)
+    for case in (CASES[1], WIDE[0]):
+        m, inp = _layer(case)
         precision("ieee")
-        first = _step(m, h, ei, na, cot, names)
+        first = _step(m, inp)
         precision("tf32")
-        _step(m, h, ei, na, cot, names)
+        _step(m, inp)
         precision("ieee")
-        after = _step(m, h, ei, na, cot, names)
-        fresh = _step(_layer(metric, C, T, aggr, params), h, ei, na, cot, names)
-        for a, b, c in zip([after[0]] + after[1], [fresh[0]] + fresh[1], [first[0]] + first[1]):
-            assert torch.equal(a, b) and torch.equal(a, c), name
+        after = _step(m, inp)
+        fresh = _step(_layer(case)[0], inp)
+        assert_all_equal(after, fresh, f"{case[0]} after TF32 vs fresh:")
+        assert_all_equal(after, first, f"{case[0]} after TF32 vs before:")
 
 
 @pytest.mark.gpu
 def test_mode_is_fixed_at_forward_time(precision):
     """switching the setting between forward and backward does not change the backward: gradients equal an all-TF32
     step bit for bit (and the other way round)"""
-    _, M = _mods()
-    metric, C, T, aggr, params, h, ei, na, cot, names = _small()
-    m = _layer(metric, C, T, aggr, params)
+    _, M = mods()
+    m, inp = _layer(CASES[1])  # md17-shaped, several tiles
     pd = dict(m.named_parameters())
     for fwd_mode, bwd_mode in (("tf32", "ieee"), ("ieee", "tf32")):
         precision(fwd_mode)
-        ref = _step(m, h, ei, na, cot, names)
-        hd, nad = h.to(DEV).requires_grad_(), na.to(DEV).requires_grad_()
-        y = m(hd, ei.to(DEV), M.PairedNodeAttr(nad), nad)
+        ref = _step(m, inp)
+        hd, nad = inp["h"].to(DEV).requires_grad_(), inp["na"].to(DEV).requires_grad_()
+        y = m(hd, inp["ei"].to(DEV), M.PairedNodeAttr(nad), nad)
         precision(bwd_mode)
-        g = torch.autograd.grad(y, [hd, nad] + [pd[k] for k in names], cot.to(DEV))
+        g = torch.autograd.grad(y, [hd, nad] + [pd[k] for k in inp["params"]], inp["cot"].to(DEV))
         assert torch.equal(y, ref[0])
-        for a, b in zip(g, ref[1]):
+        for a, b in zip(g, ref[1].values()):
             assert torch.equal(a, b), (fwd_mode, bwd_mode)
 
 
 @pytest.mark.gpu
 def test_tf32_is_deterministic_and_kernel_family_independent(precision, monkeypatch):
     """two TF32 runs, and the overlapped-epilogue kernels against the plain ones (CSMPN_TC_OVERLAP=0), bit for bit"""
-    metric, C, T, aggr, params, h, ei, na, cot, names = _small()
-    m = _layer(metric, C, T, aggr, params)
+    m, inp = _layer(CASES[1])
     precision("tf32")
-    runs = [_step(m, h, ei, na, cot, names) for _ in range(2)]
+    runs = [_step(m, inp) for _ in range(2)]
     monkeypatch.setenv("CSMPN_TC_OVERLAP", "0")
-    runs.append(_step(m, h, ei, na, cot, names))
+    runs.append(_step(m, inp))
     for r in runs[1:]:
-        assert torch.equal(r[0], runs[0][0])
-        for a, b in zip(r[1], runs[0][1]):
-            assert torch.equal(a, b)
+        assert_all_equal(r, runs[0], "tf32")
 
 
 @pytest.mark.gpu
@@ -284,13 +216,12 @@ def test_graphed_layer_captured_under_tf32_replays_tf32(precision):
     from csmpn_b200.graphs import GraphedEGCL
     from csmpn_b200.models.ops import CSRGraph
 
-    _, M = _mods()
-    metric, C, T, aggr, params, h, ei, na, cot, names = _small()
-    m = _layer(metric, C, T, aggr, params)
+    _, M = mods()
+    m, inp = _layer(CASES[1])
     plist = list(m.parameters())
-    hd, cotd = h.to(DEV), cot.to(DEV)
-    nad = na.to(DEV).requires_grad_()
-    graph = CSRGraph(ei.to(DEV), h.shape[0])
+    hd, cotd = inp["h"].to(DEV), inp["cot"].to(DEV)
+    nad = inp["na"].to(DEV).requires_grad_()
+    graph = CSRGraph(inp["ei"].to(DEV), hd.shape[0])
     precision("tf32")
     g = GraphedEGCL(m, graph, hd, M.PairedNodeAttr(nad), nad)
     precision("ieee")
@@ -311,11 +242,11 @@ def test_graphed_layer_step_captured_under_tf32_replays_tf32(precision):
     """GraphedLayerStep (forward + backward + gradient pack as one graph) captured under TF32 replays the eager TF32 step
     bit for bit, with the setting switched back before the replay"""
     from csmpn_b200.graphs import GraphedLayerStep
-    from csmpn_b200.models.cegnn_utils import PairedNodeAttr
     from csmpn_b200.models.ops import CSRGraph
 
-    metric, C, T, aggr, params, h, ei, na, cot, names = _small()
-    m = _layer(metric, C, T, aggr, params)
+    _, M = mods()
+    m, inp = _layer(CASES[1])
+    h, ei, na, cot = (inp[k] for k in ("h", "ei", "na", "cot"))
     plist = list(m.parameters())
     h_s, na_s, cot_s = h.to(DEV).clone(), na.to(DEV).clone(), cot.to(DEV).clone()
     precision("tf32")
@@ -324,7 +255,7 @@ def test_graphed_layer_step_captured_under_tf32_replays_tf32(precision):
     y, gh, flat = g()
     precision("tf32")
     h1 = h.to(DEV).requires_grad_()
-    ye = m(h1, CSRGraph(ei.to(DEV), h.shape[0]), PairedNodeAttr(na.to(DEV)), na.to(DEV))
+    ye = m(h1, CSRGraph(ei.to(DEV), h.shape[0]), M.PairedNodeAttr(na.to(DEV)), na.to(DEV))
     ge = torch.autograd.grad(ye, [h1] + plist, cot.to(DEV))
     assert torch.equal(y, ye) and torch.equal(gh, ge[0])
     assert torch.equal(flat, torch.cat([t.reshape(-1) for t in ge[1:]]))

@@ -13,13 +13,12 @@ import pytest
 import torch
 
 from conftest import FWD_TOL, GRAD_TOL, ROOT, rel_err
-from oracle import layers_ref as R
+from egcl_harness import DEV, assert_all_equal, bench_inputs, egcl_model, oracle_egcl
 
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda"
 T = 3
 
 # (id, bench workload, complexes, hidden override, env) -- rows per block in the comments are for the default seed
@@ -33,39 +32,18 @@ REGIME = [
 ]
 
 
-def _oracle(b, params, dtype):
-    ralg = R.RefAlgebra(b["metric"])
-    h = b["h"].to(dtype).requires_grad_()
-    p = {k: v.to(dtype).requires_grad_() for k, v in params.items()}
-    y = R.egcl(ralg, h, b["edge_index"], b["edge_attr"].to(dtype), b["node_attr"].to(dtype), p, aggr=b["aggr"])
-    names = list(p)
-    grads = torch.autograd.grad(y, [h] + [p[k] for k in names], b["cot"].to(dtype))
-    return y.detach(), dict(zip(["h"] + names, grads))
-
-
-def _ours(b, params, graphed=False):
-    from csmpn_b200.algebra.cliffordalgebra import CliffordAlgebra
-    from csmpn_b200.models.cegnn_utils import EGCL
+def _ours(b, inp, graphed=False):
+    from csmpn_b200.graphs import GraphedEGCL
     from csmpn_b200.models.ops import CSRGraph
 
-    alg = CliffordAlgebra(b["metric"]).to(DEV)
-    C = b["C"]
-    m = EGCL(alg, C, C, C, edge_attr_features=2 * T, node_attr_features=T, aggr=b["aggr"]).to(DEV)
-    missing, unexpected = m.load_state_dict(params, strict=False)
-    assert not unexpected and all("algebra" in k for k in missing), (missing, unexpected)
-    d = {k: b[k].to(DEV) for k in ("h", "edge_index", "edge_attr", "node_attr", "cot")}
-    graph = CSRGraph(d["edge_index"], b["N"])
-    named = dict(m.named_parameters())
-    names = list(params)
-    h = d["h"].clone().requires_grad_()
-    if graphed:
-        from csmpn_b200.graphs import GraphedEGCL
-
-        g = GraphedEGCL(m, graph, d["h"], d["edge_attr"], d["node_attr"])
-        y = g(h, d["edge_attr"], d["node_attr"])
-    else:
-        y = m(h, graph, d["edge_attr"], d["node_attr"])
-    grads = torch.autograd.grad(y, [h] + [named[k] for k in names], d["cot"])
+    m = egcl_model(b["metric"], b["C"], T, b["aggr"], inp["params"])
+    h0, ea, na, cot = (inp[k].to(DEV) for k in ("h", "ea", "na", "cot"))
+    graph = CSRGraph(inp["ei"].to(DEV), b["N"])
+    pd = dict(m.named_parameters())
+    names = list(inp["params"])
+    h = h0.clone().requires_grad_()
+    y = GraphedEGCL(m, graph, h0, ea, na)(h, ea, na) if graphed else m(h, graph, ea, na)
+    grads = torch.autograd.grad(y, [h] + [pd[k] for k in names], cot)
     torch.cuda.synchronize()
     return y.detach().cpu(), {k: v.cpu() for k, v in zip(["h"] + names, grads)}
 
@@ -76,6 +54,15 @@ def _check(tag, got, ref32, ref64, tol):
     e32, e64 = rel_err(got, ref32), rel_err(got, ref64.float())
     assert min(e32, e64) <= tol, f"{tag}: rel err vs fp32 oracle {e32:.2e}, vs fp64 oracle {e64:.2e} > {tol:.0e}"
     return e32, e64
+
+
+def _check_vs_oracle(tag, got, inp):
+    """_check of the forward output and every gradient; returns (error vs fp32, vs fp64) per name"""
+    (y32, g32), (y64, g64) = (oracle_egcl(inp, dtype, ("h",), "tensor") for dtype in (torch.float32, torch.float64))
+    worst = {"fwd": _check(f"{tag} fwd", got[0], y32, y64, FWD_TOL)}
+    for k in g32:
+        worst[k] = _check(f"{tag} grad {k}", got[1][k], g32[k], g64[k], GRAD_TOL)
+    return worst
 
 
 @pytest.fixture(scope="module")
@@ -94,19 +81,14 @@ def test_layer_step_matches_oracle_in_bench_regime(case, bench_mod, monkeypatch)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     b = bench_mod.make_batch(workload, ncx, 1000, hidden=hidden)
-    ralg = R.RefAlgebra(b["metric"])
-    params = R.init_egcl_params(ralg, b["C"], T, torch.Generator().manual_seed(7))
+    inp = bench_inputs(b)
     tiles = (b["E"] + 127) // 128
     assert tiles > 148, (name, tiles)  # several tiles per persistent CTA
     assert fused.tc_supported(len(b["metric"]), b["C"] + 2 * T, b["C"]) and b["E"] >= fused.tc_min_rows()
-    y32, g32 = _oracle(b, params, torch.float32)
-    y64, g64 = _oracle(b, params, torch.float64)
     n0 = _lib.lib().csmpn_launch_count()
-    y, g = _ours(b, params)
+    got = _ours(b, inp)
     assert _lib.lib().csmpn_launch_count() - n0 >= 30  # 2 + 7 kernels per tensor-core block
-    worst = {"fwd": _check(f"{name} fwd", y, y32, y64, FWD_TOL)}
-    for k in g32:
-        worst[k] = _check(f"{name} grad {k}", g[k], g32[k], g64[k], GRAD_TOL)
+    worst = _check_vs_oracle(name, got, inp)
     print(f"[regime] {name}: N={b['N']} E={b['E']} tiles={tiles} fwd {worst['fwd'][0]:.1e}/{worst['fwd'][1]:.1e} "
           f"worst grad {max(v[0] for k, v in worst.items() if k != 'fwd'):.1e} (vs fp32 oracle)")
 
@@ -116,40 +98,27 @@ def test_graph_replay_matches_eager_and_oracle_in_bench_regime(workload, bench_m
     """the launch path `bench.py` times: csmpn_b200.graphs.GraphedEGCL on the bench batch -- bit-identical to the eager
     step and within tolerance of the oracle"""
     b = bench_mod.make_batch(workload, 100, 1000)
-    ralg = R.RefAlgebra(b["metric"])
-    params = R.init_egcl_params(ralg, b["C"], T, torch.Generator().manual_seed(7))
-    y_e, g_e = _ours(b, params, graphed=False)
-    y_g, g_g = _ours(b, params, graphed=True)
-    assert torch.equal(y_e, y_g)
-    for k in g_e:
-        assert torch.equal(g_e[k], g_g[k]), k
-    y32, g32 = _oracle(b, params, torch.float32)
-    y64, g64 = _oracle(b, params, torch.float64)
-    _check(f"{workload} graphed fwd", y_g, y32, y64, FWD_TOL)
-    for k in g32:
-        _check(f"{workload} graphed grad {k}", g_g[k], g32[k], g64[k], GRAD_TOL)
+    inp = bench_inputs(b)
+    eager = _ours(b, inp, graphed=False)
+    graphed = _ours(b, inp, graphed=True)
+    assert_all_equal(graphed, eager, f"{workload} graphed vs eager:")
+    _check_vs_oracle(f"{workload} graphed", graphed, inp)
 
 
 def test_step_is_deterministic_in_bench_regime(bench_mod):
     """two runs of the same multi-tile step give bit-identical outputs and gradients (fixed-order reductions, no atomics)"""
     b = bench_mod.make_batch("md17", 100, 1000)
-    params = R.init_egcl_params(R.RefAlgebra(b["metric"]), b["C"], T, torch.Generator().manual_seed(7))
-    y1, g1 = _ours(b, params)
-    y2, g2 = _ours(b, params)
-    assert torch.equal(y1, y2)
-    for k in g1:
-        assert torch.equal(g1[k], g2[k]), k
+    inp = bench_inputs(b)
+    first = _ours(b, inp)
+    assert_all_equal(_ours(b, inp), first, "md17 second run vs first:")
 
 
 def test_overlapped_epilogue_bitwise_in_bench_regime(bench_mod, monkeypatch):
     """three tiles per CTA, alternating TMEM buffers: the overlapped-epilogue kernels reproduce the plain kernels' layer
     output and every gradient bit for bit on the bench batch"""
     b = bench_mod.make_batch("md17", 100, 1000)
-    params = R.init_egcl_params(R.RefAlgebra(b["metric"]), b["C"], T, torch.Generator().manual_seed(7))
+    inp = bench_inputs(b)
     monkeypatch.setenv("CSMPN_TC_OVERLAP", "1")
-    y1, g1 = _ours(b, params)
+    overlapped = _ours(b, inp)
     monkeypatch.setenv("CSMPN_TC_OVERLAP", "0")
-    y0, g0 = _ours(b, params)
-    assert torch.equal(y1, y0)
-    for k in g1:
-        assert torch.equal(g1[k], g0[k]), k
+    assert_all_equal(overlapped, _ours(b, inp), "md17 overlapped vs plain:")
