@@ -1,4 +1,5 @@
-// Fused CEMLP-block kernels (forward and backward) for Euclidean Cl(2,0), Cl(3,0), Cl(5,0).
+// Fused CEMLP-block kernels (forward and backward) for non-degenerate diagonal metrics of dimension 2, 3 and 5.
+// MET instantiations fold the metric into the elementwise stages (common.cuh MetricArg); the GEMMs do not depend on it.
 //
 // One block = MVLinear -> MVSiLU -> SteerableGeometricProductLayer -> MVLayerNorm  (cegnn_utils.py:180-207).
 //
@@ -177,27 +178,27 @@ __device__ __forceinline__ void tma_row_g2s(void* dst_smem, const void* src_gmem
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // ---------------------------------------------------------------------------------------------------
-// thread-local multivector math (Euclidean: q_g = sum of squares)
-template <int DIM>
-__device__ __forceinline__ void silu_gates(const float* y1, const float* a, const float* b, float* sg, float* inv) {
+// thread-local multivector math: quadratic forms q_g = sum_{i in g} qs_i x_i^2 (MET), sums of squares (Euclidean)
+template <int DIM, bool MET>
+__device__ __forceinline__ void silu_gates(const float* y1, const float* a, const float* b, float* sg, float* inv, const float* qs) {
   using A = Alg<DIM>;
 #pragma unroll
   for (int g = 0; g < A::G; ++g) inv[g] = 0.f;
 #pragma unroll
-  for (int i = 0; i < A::B; ++i) inv[A::grade_of(i)] = fmaf(y1[i], y1[i], inv[A::grade_of(i)]);
+  for (int i = 0; i < A::B; ++i) inv[A::grade_of(i)] = fmaf(qs_x<MET>(qs, i, y1[i]), y1[i], inv[A::grade_of(i)]);
   inv[0] = y1[0];
 #pragma unroll
   for (int g = 0; g < A::G; ++g) sg[g] = sigmoidf_(fmaf(a[g], inv[g], b[g]));
 }
 
 // normalisation: xn_i = xr_i * rinv[g];  den_g = s_g (nrm_g - 1) + 1 + eps
-template <int DIM>
-__device__ __forceinline__ void norm_factors(const float* xr, const float* s, float* q, float* nrm, float* rinv) {
+template <int DIM, bool MET>
+__device__ __forceinline__ void norm_factors(const float* xr, const float* s, float* q, float* nrm, float* rinv, const float* qs) {
   using A = Alg<DIM>;
 #pragma unroll
   for (int g = 0; g < A::G; ++g) q[g] = 0.f;
 #pragma unroll
-  for (int i = 0; i < A::B; ++i) q[A::grade_of(i)] = fmaf(xr[i], xr[i], q[A::grade_of(i)]);
+  for (int i = 0; i < A::B; ++i) q[A::grade_of(i)] = fmaf(qs_x<MET>(qs, i, xr[i]), xr[i], q[A::grade_of(i)]);
 #pragma unroll
   for (int g = 0; g < A::G; ++g) {
     nrm[g] = smooth_abs_sqrt(q[g]);
@@ -205,11 +206,12 @@ __device__ __forceinline__ void norm_factors(const float* xr, const float* s, fl
   }
 }
 
-template <int DIM>
-__device__ __forceinline__ float mv_sumsq(const float* x) {
+// full quadratic form Q = sum_i qs_i x_i^2 (MVLayerNorm)
+template <int DIM, bool MET>
+__device__ __forceinline__ float mv_q(const float* x, const float* qs) {
   float Q = 0.f;
 #pragma unroll
-  for (int i = 0; i < Alg<DIM>::B; ++i) Q = fmaf(x[i], x[i], Q);
+  for (int i = 0; i < Alg<DIM>::B; ++i) Q = fmaf(qs_x<MET>(qs, i, x[i]), x[i], Q);
   return Q;
 }
 
@@ -425,8 +427,8 @@ struct ChanParams {
 
 // ===================================================================================================
 // forward
-template <int DIM>
-__global__ void __launch_bounds__(256, 1) block_fwd_kernel(csmpn_block_desc d, FusedPlan p) {
+template <int DIM, bool MET>
+__global__ void __launch_bounds__(256, 1) block_fwd_kernel(csmpn_block_desc d, FusedPlan p, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G;
   extern __shared__ __align__(128) float smem[];
@@ -480,7 +482,7 @@ __global__ void __launch_bounds__(256, 1) block_fwd_kernel(csmpn_block_desc d, F
         load_vec<B>(y1, q);
         y1[0] += cp.b1;
         if (d.save_y1 && r < valid) store_vec<B>(d.save_y1 + ((row0 + r) * C + n_e) * B, y1);
-        silu_gates<DIM>(y1, cp.sa, cp.sb, sg, inv);
+        silu_gates<DIM, MET>(y1, cp.sa, cp.sb, sg, inv, mp.qs);
 #pragma unroll
         for (int i = 0; i < B; ++i) y1[i] *= sg[A::grade_of(i)];
         store_vec<B>(q, y1);
@@ -498,16 +500,16 @@ __global__ void __launch_bounds__(256, 1) block_fwd_kernel(csmpn_block_desc d, F
         load_vec<B>(y2, tB + r * p.s1 + n_e * B);
         load_vec<B>(o, tC + r * p.s2 + n_e * B);
         if (d.save_xr && r < valid) store_vec<B>(d.save_xr + ((row0 + r) * C + n_e) * B, xr);
-        norm_factors<DIM>(xr, cp.sn, q, nrm, rinv);
+        norm_factors<DIM, MET>(xr, cp.sn, q, nrm, rinv, mp.qs);
 #pragma unroll
         for (int i = 0; i < B; ++i) xr[i] *= rinv[A::grade_of(i)];
         o[0] += cp.bl;
-        A::template wgp<false>(y2, xr, cp.wv, nullptr, o);
+        A::template wgp<MET>(y2, xr, cp.wv, mp.mf, o);
 #pragma unroll
         for (int i = 0; i < B; ++i) o[i] *= kInvSqrt2;
         if (d.save_o && r < valid) store_vec<B>(d.save_o + ((row0 + r) * C + n_e) * B, o);
         store_vec<B>(tC + r * p.s2 + n_e * B, o);
-        nu_s[r * C + n_e] = smooth_abs_sqrt(mv_sumsq<DIM>(o));
+        nu_s[r * C + n_e] = smooth_abs_sqrt(mv_q<DIM, MET>(o, mp.qs));
       }
     }
     g.sync();
@@ -663,9 +665,9 @@ __device__ __forceinline__ void dx_pass(const Grp& g, const float* __restrict__ 
 
 // ===================================================================================================
 // backward
-template <int DIM>
+template <int DIM, bool MET>
 __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, csmpn_block_grads gr, FusedPlan p,
-                                                           BwdWorkspace ws) {
+                                                           BwdWorkspace ws, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, P = A::P, NCH = FCfg<DIM>::NCH;
   extern __shared__ __align__(128) float smem[];
@@ -737,7 +739,7 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
         float dot = 0.f;
 #pragma unroll
         for (int i = 0; i < B; ++i) dot = fmaf(dy[i], o[i], dot);
-        nu_s[r * C + n_e] = smooth_abs_sqrt(mv_sumsq<DIM>(o));
+        nu_s[r * C + n_e] = smooth_abs_sqrt(mv_q<DIM, MET>(o, mp.qs));
         dt_s[r * C + n_e] = cp.la * dot;
       }
     }
@@ -766,12 +768,12 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
 #pragma unroll
           for (int i = 0; i < B; ++i) dot = fmaf(dd[i], o[i], dot);
           g_la = fmaf(dot, inv_mu, g_la);
-          const float Q = mv_sumsq<DIM>(o);
+          const float Q = mv_q<DIM, MET>(o, mp.qs);
           const float nu = smooth_abs_sqrt(Q);
           const float k1 = cp.la * inv_mu * kInvSqrt2;
           const float k2 = dmu_s[r] * Q / (nu * nu * nu) * kInvSqrt2;
 #pragma unroll
-          for (int i = 0; i < B; ++i) dd[i] = fmaf(k1, dd[i], k2 * o[i]);  // d = do / sqrt2
+          for (int i = 0; i < B; ++i) dd[i] = fmaf(k1, dd[i], k2 * qs_x<MET>(mp.qs, i, o[i]));  // d = do / sqrt2
         }
         store_vec<B>(t2 + r * p.s2 + n_e * B, dd);
         g_bl += dd[0];
@@ -779,17 +781,17 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
         {
           float sg[G], inv[G];
           load_vec<B>(y2, t4 + r * p.s2 + n_e * B);  // y1
-          silu_gates<DIM>(y2, cp.sa, cp.sb, sg, inv);
+          silu_gates<DIM, MET>(y2, cp.sa, cp.sb, sg, inv, mp.qs);
 #pragma unroll
           for (int i = 0; i < B; ++i) y2[i] *= sg[A::grade_of(i)];
         }
         store_vec<B>(t1 + r * p.s1 + n_e * B, y2);
         load_vec<B>(xr, t3 + r * p.s3 + n_e * B);
         float q[G], nrm[G], rinv[G], xn[B], dxn[B], dy2[B];
-        norm_factors<DIM>(xr, cp.sn, q, nrm, rinv);
+        norm_factors<DIM, MET>(xr, cp.sn, q, nrm, rinv, mp.qs);
 #pragma unroll
         for (int i = 0; i < B; ++i) { xn[i] = xr[i] * rinv[A::grade_of(i)]; dy2[i] = 0.f; dxn[i] = 0.f; }
-        A::template wgp_bwd<false>(y2, xn, cp.wv, dd, nullptr, dy2, dxn, g_w);
+        A::template wgp_bwd<MET>(y2, xn, cp.wv, dd, mp.mf, dy2, dxn, g_w);
         store_vec<B>(t4 + r * p.s2 + n_e * B, dy2);
         float t[G];
 #pragma unroll
@@ -804,7 +806,7 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
           coef[g] = ddn * cp.sn[g] * q[g] / (nrm[g] * nrm[g] * nrm[g]);
         }
 #pragma unroll
-        for (int i = 0; i < B; ++i) dxn[i] = fmaf(dxn[i], rinv[A::grade_of(i)], coef[A::grade_of(i)] * xr[i]);
+        for (int i = 0; i < B; ++i) dxn[i] = fmaf(dxn[i], rinv[A::grade_of(i)], coef[A::grade_of(i)] * qs_x<MET>(mp.qs, i, xr[i]));
         store_vec<B>(t3 + r * p.s3 + n_e * B, dxn);  // dxr
       }
     }
@@ -859,7 +861,7 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
         float y1[B], dy[B], sg[G], inv[G], t[G];
         load_vec<B>(y1, t2 + r * p.s2 + n_e * B);
         load_vec<B>(dy, t4 + r * p.s2 + n_e * B);
-        silu_gates<DIM>(y1, cp.sa, cp.sb, sg, inv);
+        silu_gates<DIM, MET>(y1, cp.sa, cp.sb, sg, inv, mp.qs);
 #pragma unroll
         for (int g = 0; g < G; ++g) t[g] = 0.f;
 #pragma unroll
@@ -874,7 +876,7 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
 #pragma unroll
         for (int i = 0; i < B; ++i) {
           const int g = A::grade_of(i);
-          const float dinv = (g == 0) ? 1.f : 2.f * y1[i];
+          const float dinv = (g == 0) ? 1.f : 2.f * qs_x<MET>(mp.qs, i, y1[i]);
           dy[i] = fmaf(sg[g], dy[i], ds[g] * cp.sa[g] * dinv);
         }
         g_b1 += dy[0];
@@ -965,19 +967,26 @@ __global__ void __launch_bounds__(256) block_bwd_final_kernel(FinalSegs segs) {
   }
 }
 
+template <int DIM, bool MET>
+int run_block_fwd(const csmpn_block_desc& d, const FusedPlan& p, MetricArg<MET> mp, cudaStream_t s) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    CSMPN_CUDA_TRY(cudaFuncSetAttribute(block_fwd_kernel<DIM, MET>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem + 1024));
+    attr_set = true;
+  }
+  block_fwd_kernel<DIM, MET><<<p.grid, p.threads * p.ng, p.smem, s>>>(d, p, mp);
+  CSMPN_LAUNCH_CHECK("block_fwd");
+  return CSMPN_OK;
+}
+
 template <int DIM>
 int launch_block_fwd(const csmpn_block_desc& d, cudaStream_t s) {
   FusedPlan p;
   int st = make_fused_plan<DIM>(d, false, &p);
   if (st) return st;
-  static bool attr_set = false;
-  if (!attr_set) {
-    CSMPN_CUDA_TRY(cudaFuncSetAttribute(block_fwd_kernel<DIM>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem + 1024));
-    attr_set = true;
-  }
-  block_fwd_kernel<DIM><<<p.grid, p.threads * p.ng, p.smem, s>>>(d, p);
-  CSMPN_LAUNCH_CHECK("block_fwd");
-  return CSMPN_OK;
+  MetricParams mp;
+  if (block_metric(DIM, d, &mp)) return run_block_fwd<DIM, true>(d, p, mp, s);
+  return run_block_fwd<DIM, false>(d, p, NoMetric{}, s);
 }
 
 template <int DIM>
@@ -991,9 +1000,23 @@ int64_t block_bwd_ws_bytes(const csmpn_block_desc& d, FusedPlan* pp) {
   return words * 4;
 }
 
+template <int DIM, bool MET>
+int run_block_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, const FusedPlan& p, const BwdWorkspace& ws,
+                  MetricArg<MET> mp, cudaStream_t s) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    CSMPN_CUDA_TRY(cudaFuncSetAttribute(block_bwd_kernel<DIM, MET>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem + 1024));
+    attr_set = true;
+  }
+  block_bwd_kernel<DIM, MET><<<p.grid, p.threads * p.ng, p.smem, s>>>(d, g, p, ws, mp);
+  CSMPN_LAUNCH_CHECK("block_bwd");
+  return CSMPN_OK;
+}
+
 template <int DIM>
 int launch_block_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* workspace, int64_t bytes, cudaStream_t s) {
   FusedPlan p;
+  int st;
   const int64_t need = block_bwd_ws_bytes<DIM>(d, &p);
   if (need < 0) return CSMPN_ERR_UNSUPPORTED;
   if (!workspace || bytes < need) return CSMPN_ERR_WORKSPACE;
@@ -1007,13 +1030,9 @@ int launch_block_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void
   ws.small = ws.dwl + slots * c * c * G;
   const size_t dw_bytes = (size_t)((char*)ws.small - (char*)workspace);
   CSMPN_CUDA_TRY(cudaMemsetAsync(workspace, 0, dw_bytes, s));  // the small partials are written, not accumulated
-  static bool attr_set = false;
-  if (!attr_set) {
-    CSMPN_CUDA_TRY(cudaFuncSetAttribute(block_bwd_kernel<DIM>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem + 1024));
-    attr_set = true;
-  }
-  block_bwd_kernel<DIM><<<p.grid, p.threads * p.ng, p.smem, s>>>(d, g, p, ws);
-  CSMPN_LAUNCH_CHECK("block_bwd");
+  MetricParams mp;
+  st = block_metric(DIM, d, &mp) ? run_block_bwd<DIM, true>(d, g, p, ws, mp, s) : run_block_bwd<DIM, false>(d, g, p, ws, NoMetric{}, s);
+  if (st) return st;
   const int small_words = c * (P + 3 * G + 3);
   FinalSegs fs;
   int k = 0;
@@ -1051,6 +1070,9 @@ inline int check_desc(int dim, const csmpn_block_desc* d) {
   if (!d->w1 || !d->sa || !d->sb || !d->wr || !d->na || !d->wl || !d->bl || !d->wp || !d->la) return CSMPN_ERR_BAD_ARG;
   if (d->has_b1 && !d->b1) return CSMPN_ERR_BAD_ARG;
   if (d->tf32 != 0 && d->tf32 != 1) return CSMPN_ERR_BAD_ARG;
+  if (d->metric)  // degenerate metrics (a zero entry) change the grade-path set of the product: unit kernels only
+    for (int i = 0; i < dim; ++i)
+      if (d->metric[i] == 0.f) return CSMPN_ERR_UNSUPPORTED;
   return CSMPN_OK;
 }
 

@@ -48,6 +48,24 @@ struct MetricParams {
   int euclid;    // 1 if every metric entry is exactly 1
 };
 
+// Metric operand of the fused block kernels: the Euclidean instantiations (MET = false) take an empty struct whose
+// null tables are never read (the generated products and the quadratic forms fold them out at compile time), the
+// non-Euclidean ones take MetricParams by value.
+struct NoMetric {
+  static constexpr const float* mf = nullptr;
+  static constexpr const float* qs = nullptr;
+};
+template <bool MET> struct MetricArgT { using type = NoMetric; };
+template <> struct MetricArgT<true> { using type = MetricParams; };
+template <bool MET> using MetricArg = typename MetricArgT<MET>::type;
+
+// qs_i x_i (MET) or x_i: one factor of the quadratic-form term qs_i x_i^2 and of its derivative 2 qs_i x_i
+template <bool MET>
+__device__ __forceinline__ float qs_x(const float* qs, int i, float x) {
+  if constexpr (MET) return qs[i] * x;
+  else return x;
+}
+
 // bitmap of blade `idx` in short-lex order, host side
 inline void host_blade_bitmaps(int dim, int* bitmap_of_index) {
   int n = 0;
@@ -88,6 +106,12 @@ inline int make_metric_params(int dim, const float* metric, MetricParams* mp) {
   // beta_i * c[i,0,i] = beta_i * reorder_sign(b,b) * mf[b]; beta_i * reorder_sign(b,b) == +1 for every blade
   for (int i = 0; i < B; ++i) mp->qs[i] = mp->mf[bitmaps[i]];
   return CSMPN_OK;
+}
+
+// metric of a fused block call (csmpn_block_desc.metric, NULL = Euclidean): true, with *mp filled, when the
+// non-Euclidean kernels must run
+inline bool block_metric(int dim, const csmpn_block_desc& d, MetricParams* mp) {
+  return d.metric && make_metric_params(dim, d.metric, mp) == CSMPN_OK && !mp->euclid;
 }
 
 // dispatch a runtime dim (1..5) to a compile-time template argument

@@ -45,26 +45,27 @@ __device__ __forceinline__ float fast_sigmoid(float v) { return fast_rcp(1.f + f
 // (q^2 + 1e-16)^(1/4)
 __device__ __forceinline__ float fast_sas(float q) { return fast_sqrt(fast_sqrt(fmaf(q, q, kSmoothEps))); }
 
-template <int DIM>
-__device__ __forceinline__ void silu_gates(const float* y1, const float* a, const float* b, float* sg, float* inv) {
+// Quadratic forms: q_g = sum_{i in g} qs_i x_i^2 with the metric's signs and scales qs (MET), sums of squares (Euclidean)
+template <int DIM, bool MET>
+__device__ __forceinline__ void silu_gates(const float* y1, const float* a, const float* b, float* sg, float* inv, const float* qs) {
   using A = Alg<DIM>;
 #pragma unroll
   for (int g = 0; g < A::G; ++g) inv[g] = 0.f;
 #pragma unroll
-  for (int i = 0; i < A::B; ++i) inv[A::grade_of(i)] = fmaf(y1[i], y1[i], inv[A::grade_of(i)]);
+  for (int i = 0; i < A::B; ++i) inv[A::grade_of(i)] = fmaf(qs_x<MET>(qs, i, y1[i]), y1[i], inv[A::grade_of(i)]);
   inv[0] = y1[0];
 #pragma unroll
   for (int g = 0; g < A::G; ++g) sg[g] = fast_sigmoid(fmaf(a[g], inv[g], b[g]));
 }
 
 // normalisation: xn_i = xr_i * rinv[g];  den_g = s_g (nrm_g - 1) + 1 + eps
-template <int DIM>
-__device__ __forceinline__ void norm_factors(const float* xr, const float* s, float* q, float* nrm, float* rinv) {
+template <int DIM, bool MET>
+__device__ __forceinline__ void norm_factors(const float* xr, const float* s, float* q, float* nrm, float* rinv, const float* qs) {
   using A = Alg<DIM>;
 #pragma unroll
   for (int g = 0; g < A::G; ++g) q[g] = 0.f;
 #pragma unroll
-  for (int i = 0; i < A::B; ++i) q[A::grade_of(i)] = fmaf(xr[i], xr[i], q[A::grade_of(i)]);
+  for (int i = 0; i < A::B; ++i) q[A::grade_of(i)] = fmaf(qs_x<MET>(qs, i, xr[i]), xr[i], q[A::grade_of(i)]);
 #pragma unroll
   for (int g = 0; g < A::G; ++g) {
     nrm[g] = fast_sas(q[g]);
@@ -72,11 +73,12 @@ __device__ __forceinline__ void norm_factors(const float* xr, const float* s, fl
   }
 }
 
-template <int DIM>
-__device__ __forceinline__ float mv_sumsq(const float* x) {
+// full quadratic form Q = sum_i qs_i x_i^2 (MVLayerNorm)
+template <int DIM, bool MET>
+__device__ __forceinline__ float mv_q(const float* x, const float* qs) {
   float Q = 0.f;
 #pragma unroll
-  for (int i = 0; i < Alg<DIM>::B; ++i) Q = fmaf(x[i], x[i], Q);
+  for (int i = 0; i < Alg<DIM>::B; ++i) Q = fmaf(qs_x<MET>(qs, i, x[i]), x[i], Q);
   return Q;
 }
 

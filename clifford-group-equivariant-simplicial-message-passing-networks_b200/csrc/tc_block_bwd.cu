@@ -1,4 +1,5 @@
-// Tensor-core backward of one CEMLP block (autograd of cegnn_utils.py:180-207) for Euclidean Cl(2,0) / Cl(3,0).
+// Tensor-core backward of one CEMLP block (autograd of cegnn_utils.py:180-207) for non-degenerate diagonal metrics of
+// dimension 2 and 3 (MET: the metric's quadratic-form signs qs and product factors mf in tc_b1 / tc_b3).
 //
 // All intermediates are BPT tensors (tc_block.cuh).  Saved by the forward: y1 (pre-SiLU), y2 (post-SiLU), xr
 // (pre-normalisation), o (pre-LayerNorm), and x0 (the assembled input row) when the input was not already BPT.
@@ -88,8 +89,8 @@ __device__ __forceinline__ void read_stage(float* v, const float* st, int lane) 
 // CP channels per CTA (CP * 8 threads); CPT = padded channel count of the tensors.  Wide blocks (CPT > CP = 64) run one
 // CTA per (work unit, 64-channel slab = blockIdx.y); the row statistics of the layer norm need every channel, so each
 // CTA walks phase 1 over all slabs and phase 2 over its own.
-template <int DIM, int CP, int CPT>
-__global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs a) {
+template <int DIM, int CP, int CPT, bool MET>
+__global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs a, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, P = A::P, NP = P + G + 2;
   constexpr int NSLAB = CPT / CP;
@@ -183,7 +184,7 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs 
         float dot = 0.f;
 #pragma unroll
         for (int b = 0; b < B; ++b) dot = fmaf(dy[b], o[b], dot);
-        float nu = okx ? fast_sas(mv_sumsq<DIM>(o)) : 0.f;
+        float nu = okx ? fast_sas(mv_q<DIM, MET>(o, mp.qs)) : 0.f;
         float dt = okx ? lax * dot : 0.f;
         nu += __shfl_xor_sync(0xffffffffu, nu, 1); dt += __shfl_xor_sync(0xffffffffu, dt, 1);
         nu += __shfl_xor_sync(0xffffffffu, nu, 2); dt += __shfl_xor_sync(0xffffffffu, dt, 2);
@@ -216,12 +217,12 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs 
 #pragma unroll
         for (int b = 0; b < B; ++b) dot = fmaf(dd[b], o[b], dot);
         if (ok) g_la = fmaf(dot, inv_mu, g_la);
-        const float Q = mv_sumsq<DIM>(o);
+        const float Q = mv_q<DIM, MET>(o, mp.qs);
         const float nu = fast_sas(Q);
         const float k1 = la * inv_mu * kInvSqrt2;
         const float k2 = dmu_s[r] * Q * fast_rcp(nu * nu * nu) * kInvSqrt2;
 #pragma unroll
-        for (int b = 0; b < B; ++b) dd[b] = ok ? fmaf(k1, dd[b], k2 * o[b]) : 0.f;  // d = do / sqrt2
+        for (int b = 0; b < B; ++b) dd[b] = ok ? fmaf(k1, dd[b], k2 * qs_x<MET>(mp.qs, b, o[b])) : 0.f;  // d = do / sqrt2
       }
       store_mv_bpt<DIM>(a.d, dd, Cp, tile, c4, r, j);
       g_bl += dd[0];
@@ -229,10 +230,10 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs 
       read_stage<DIM>(y2, stage_of(s, 2), lane);
       read_stage<DIM>(xr, stage_of(s, 3), lane);
       float q[G], nrm[G], rinv[G], xn[B], dxn[B], dy2[B];
-      norm_factors<DIM>(xr, sn, q, nrm, rinv);
+      norm_factors<DIM, MET>(xr, sn, q, nrm, rinv, mp.qs);
 #pragma unroll
       for (int b = 0; b < B; ++b) { xn[b] = xr[b] * rinv[A::grade_of(b)]; dy2[b] = 0.f; dxn[b] = 0.f; }
-      A::template wgp_bwd<false>(y2, xn, wv, dd, nullptr, dy2, dxn, g_w);
+      A::template wgp_bwd<MET>(y2, xn, wv, dd, mp.mf, dy2, dxn, g_w);
       store_mv_bpt<DIM>(a.dy2p, dy2, Cp, tile, c4, r, j);
       float t[G], coef[G];
 #pragma unroll
@@ -246,7 +247,7 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs 
         coef[g] = ddn * sn[g] * q[g] * fast_rcp(nrm[g] * nrm[g] * nrm[g]);
       }
 #pragma unroll
-      for (int b = 0; b < B; ++b) dxn[b] = fmaf(dxn[b], rinv[A::grade_of(b)], coef[A::grade_of(b)] * xr[b]);
+      for (int b = 0; b < B; ++b) dxn[b] = fmaf(dxn[b], rinv[A::grade_of(b)], coef[A::grade_of(b)] * qs_x<MET>(mp.qs, b, xr[b]));
       store_mv_bpt<DIM>(a.dxr, dxn, Cp, tile, c4, r, j);
     }
   }
@@ -267,8 +268,8 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b1_kernel(EwArgs 
   { const float v = red(g_bl); if (rr == 0 && ch_ok) out[P + G + 1] = v; }
 }
 
-template <int DIM, int CP, int CPT>
-__global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b3_kernel(EwArgs a) {
+template <int DIM, int CP, int CPT, bool MET>
+__global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b3_kernel(EwArgs a, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, NP = 2 * G + 1;
   extern __shared__ float sm[];
@@ -317,7 +318,7 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b3_kernel(EwArgs 
       float y1[B], dy[B], sg[G], inv[G], t[G], ds[G];
       read_stage<DIM>(y1, stage_of(s, 0), lane);
       read_stage<DIM>(dy, stage_of(s, 1), lane);
-      silu_gates<DIM>(y1, sa, sb, sg, inv);
+      silu_gates<DIM, MET>(y1, sa, sb, sg, inv, mp.qs);
 #pragma unroll
       for (int g = 0; g < G; ++g) t[g] = 0.f;
 #pragma unroll
@@ -331,7 +332,7 @@ __global__ void __launch_bounds__(CP * 8, CP <= 32 ? 2 : 1) tc_b3_kernel(EwArgs 
 #pragma unroll
       for (int b = 0; b < B; ++b) {
         const int g = A::grade_of(b);
-        const float dinv = (g == 0) ? 1.f : 2.f * y1[b];
+        const float dinv = (g == 0) ? 1.f : 2.f * qs_x<MET>(mp.qs, b, y1[b]);
         dy[b] = ok ? fmaf(sg[g], dy[b], ds[g] * sa[g] * dinv) : 0.f;
       }
       g_b1 += dy[0];
@@ -955,9 +956,11 @@ int make_bwd_plan(const csmpn_block_desc& d, BwdPlan* p) {
   return CSMPN_OK;
 }
 
-// TERMS: numeric mode (csmpn_block_desc.tf32 = 1 -> 1, else 3); the elementwise kernels do not depend on it
-template <int DIM, int TERMS>
-int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* workspace, int64_t bytes, cudaStream_t stream) {
+// TERMS: numeric mode (csmpn_block_desc.tf32 = 1 -> 1, else 3); the elementwise kernels do not depend on it.  MET: the
+// elementwise kernels run with the non-Euclidean metric mp; the GEMMs do not depend on it.
+template <int DIM, int TERMS, bool MET>
+int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* workspace, int64_t bytes, MetricArg<MET> mp,
+               cudaStream_t stream) {
   constexpr int B = Alg<DIM>::B, G = Alg<DIM>::G, P = Alg<DIM>::P, NI = n_images(TERMS);
   BwdPlan p;
   int st = make_bwd_plan<DIM>(d, &p);
@@ -996,12 +999,12 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
     const size_t sm1 = (size_t)(2 * (cps / 4) * kTile + 2 * kTile) * 4 + (size_t)2 * 4 * B * ew_threads * 4;
     auto run = [&](auto kern) -> int {
       CSMPN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm1));
-      kern<<<ew_grid, ew_threads, sm1, stream>>>(e);
+      kern<<<ew_grid, ew_threads, sm1, stream>>>(e, mp);
       return CSMPN_OK;
     };
-    int rc = Cp == 16 ? run(tc_b1_kernel<DIM, 16, 16>) : Cp == 32 ? run(tc_b1_kernel<DIM, 32, 32>)
-             : Cp == 48 ? run(tc_b1_kernel<DIM, 48, 48>) : Cp == 64 ? run(tc_b1_kernel<DIM, 64, 64>)
-             : Cp == 128 ? run(tc_b1_kernel<DIM, 64, 128>) : run(tc_b1_kernel<DIM, 64, 256>);
+    int rc = Cp == 16 ? run(tc_b1_kernel<DIM, 16, 16, MET>) : Cp == 32 ? run(tc_b1_kernel<DIM, 32, 32, MET>)
+             : Cp == 48 ? run(tc_b1_kernel<DIM, 48, 48, MET>) : Cp == 64 ? run(tc_b1_kernel<DIM, 64, 64, MET>)
+             : Cp == 128 ? run(tc_b1_kernel<DIM, 64, 128, MET>) : run(tc_b1_kernel<DIM, 64, 256, MET>);
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_b1_kernel");
   }
@@ -1039,12 +1042,12 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
     const size_t sm3 = (size_t)2 * 2 * B * ew_threads * 4;
     auto run = [&](auto kern) -> int {
       CSMPN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm3));
-      kern<<<ew_grid, ew_threads, sm3, stream>>>(e);
+      kern<<<ew_grid, ew_threads, sm3, stream>>>(e, mp);
       return CSMPN_OK;
     };
-    int rc = Cp == 16 ? run(tc_b3_kernel<DIM, 16, 16>) : Cp == 32 ? run(tc_b3_kernel<DIM, 32, 32>)
-             : Cp == 48 ? run(tc_b3_kernel<DIM, 48, 48>) : Cp == 64 ? run(tc_b3_kernel<DIM, 64, 64>)
-             : Cp == 128 ? run(tc_b3_kernel<DIM, 64, 128>) : run(tc_b3_kernel<DIM, 64, 256>);
+    int rc = Cp == 16 ? run(tc_b3_kernel<DIM, 16, 16, MET>) : Cp == 32 ? run(tc_b3_kernel<DIM, 32, 32, MET>)
+             : Cp == 48 ? run(tc_b3_kernel<DIM, 48, 48, MET>) : Cp == 64 ? run(tc_b3_kernel<DIM, 64, 64, MET>)
+             : Cp == 128 ? run(tc_b3_kernel<DIM, 64, 128, MET>) : run(tc_b3_kernel<DIM, 64, 256, MET>);
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_b3_kernel");
   }
@@ -1194,6 +1197,13 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   return CSMPN_OK;
 }
 
+template <int DIM, int TERMS>
+int launch_bwd_metric(const csmpn_block_desc& d, const csmpn_block_grads& g, void* workspace, int64_t bytes, cudaStream_t stream) {
+  MetricParams mp;
+  if (block_metric(DIM, d, &mp)) return launch_bwd<DIM, TERMS, true>(d, g, workspace, bytes, mp, stream);
+  return launch_bwd<DIM, TERMS, false>(d, g, workspace, bytes, NoMetric{}, stream);
+}
+
 template <int DIM>
 int64_t bwd_ws_bytes(const csmpn_block_desc& d) {
   BwdPlan p;
@@ -1204,8 +1214,8 @@ int64_t bwd_ws_bytes(const csmpn_block_desc& d) {
 }  // namespace tcb
 
 int tc_block_bwd(int dim, const csmpn_block_desc* d, const csmpn_block_grads* g, void* ws, int64_t bytes, cudaStream_t stream) {
-  if (dim == 2) return d->tf32 ? tcb::launch_bwd<2, 1>(*d, *g, ws, bytes, stream) : tcb::launch_bwd<2, 3>(*d, *g, ws, bytes, stream);
-  if (dim == 3) return d->tf32 ? tcb::launch_bwd<3, 1>(*d, *g, ws, bytes, stream) : tcb::launch_bwd<3, 3>(*d, *g, ws, bytes, stream);
+  if (dim == 2) return d->tf32 ? tcb::launch_bwd_metric<2, 1>(*d, *g, ws, bytes, stream) : tcb::launch_bwd_metric<2, 3>(*d, *g, ws, bytes, stream);
+  if (dim == 3) return d->tf32 ? tcb::launch_bwd_metric<3, 1>(*d, *g, ws, bytes, stream) : tcb::launch_bwd_metric<3, 3>(*d, *g, ws, bytes, stream);
   return CSMPN_ERR_UNSUPPORTED;
 }
 // the backward of a block of this shape fits (shared memory / TMEM plans of every backward kernel)

@@ -1,4 +1,4 @@
-// Tensor-core forward of one CEMLP block (cegnn_utils.py:180-207) for Euclidean Cl(2,0) / Cl(3,0):
+// Tensor-core forward of one CEMLP block (cegnn_utils.py:180-207) for non-degenerate diagonal metrics of dimension 2 and 3:
 //
 //   tc_f1_kernel:  x0 (gathered / concatenated API-layout rows, or a BPT tensor) --MVLinear W1--> y1 (+bias, saved)
 //                  --MVSiLU--> y2 (BPT)
@@ -202,9 +202,9 @@ __device__ __forceinline__ void zero_chunk_bpt(float* dst, int cp, int64_t tile,
 
 // F1 epilogue of channel group gc4 of row r of `tile`, from the accumulators already loaded from TMEM (v): bias -> y1
 // (saved when requested), MVSiLU -> y2.  b1_s / sa_s / sb_s: the bias and gate parameters staged in shared memory.
-template <int DIM>
+template <int DIM, bool MET>
 __device__ __forceinline__ void f1_epilogue_group(const FwdArgs& a, float (&v)[Alg<DIM>::B][4], int64_t tile, int gc4, int r,
-                                                  const float* b1_s, const float* sa_s, const float* sb_s) {
+                                                  const float* b1_s, const float* sa_s, const float* sb_s, const float* qs) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G;
   const bool row_ok = tile * kTile + r < a.rows;
@@ -230,7 +230,7 @@ __device__ __forceinline__ void f1_epilogue_group(const FwdArgs& a, float (&v)[A
     float y1[B], sg[G], inv[G];
 #pragma unroll
     for (int b = 0; b < B; ++b) y1[b] = v[b][j];
-    silu_gates<DIM>(y1, sa_s + ch * G, sb_s + ch * G, sg, inv);
+    silu_gates<DIM, MET>(y1, sa_s + ch * G, sb_s + ch * G, sg, inv, qs);
 #pragma unroll
     for (int b = 0; b < B; ++b) v[b][j] = y1[b] * sg[A::grade_of(b)];
   }
@@ -263,9 +263,9 @@ __device__ __forceinline__ void stage_f1_params(const FwdArgs& a, float* b1_s, f
 // F1: MVLinear (W1) + bias + MVSiLU.  ST (streamed weights, wide blocks): the output channels are produced in passes of
 // a.ns1 channels (accumulators = B * ns1 TMEM columns), the K chunks of the input are walked once per pass and every chunk
 // arrives with its weight unit (tc_block.cuh); the resident weight images do not exist.  TERMS: numeric mode
-// (tc_block.cuh, n_images).
-template <int DIM, bool BPT_IN, bool ST, int TERMS = 3>
-__global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
+// (tc_block.cuh, n_images).  MET: non-Euclidean metric (mp, common.cuh MetricArg) in the MVSiLU invariants.
+template <int DIM, bool BPT_IN, bool ST, int TERMS, bool MET>
+__global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -354,7 +354,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
 #pragma unroll
         for (int b = 0; b < B; ++b) tmem_ld4(tmem_at(tbase, (warp & 3) * 32, b * NS + c4 * 4), v[b]);
         tmem_wait_ld();
-        f1_epilogue_group<DIM>(a, v, tile, (n0 >> 2) + c4, r, b1_s, sa_s, sb_s);
+        f1_epilogue_group<DIM, MET>(a, v, tile, (n0 >> 2) + c4, r, b1_s, sa_s, sb_s, mp.qs);
       }
       fence_before_sync();  // the next pass's first MMA overwrites these accumulators (tc_block.cuh: reuse rules)
     }
@@ -371,8 +371,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1_kernel(FwdArgs a) {
 // Roles: warp 0 issues copies and MMAs only; warps 1-15 convert / gather; warps 4-15 also own the epilogue: lane quadrant
 // warp & 3, channel groups (warp >> 2) - 1, + 3, ... (PendingEpilogue).  Same epilogue body as tc_f1_kernel
 // (f1_epilogue_group): results are bit-identical.
-template <int DIM, bool BPT_IN, int TERMS = 3>
-__global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
+template <int DIM, bool BPT_IN, int TERMS, bool MET>
+__global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -418,7 +418,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
 #pragma unroll
     for (int b = 0; b < B; ++b) tmem_ld4(tmem_at(tb, (warp & 3) * 32, b * Cp + c4 * 4), v[b]);
     tmem_wait_ld();
-    f1_epilogue_group<DIM>(a, v, tile, c4, r, b1_s, sa_s, sb_s);
+    f1_epilogue_group<DIM, MET>(a, v, tile, c4, r, b1_s, sa_s, sb_s, mp.qs);
   };
   PendingEpilogue pend;
 
@@ -465,8 +465,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f1db_kernel(FwdArgs a) {
 // ST (streamed weights, wide blocks): NS = a.ns2 < Cp output channels per pass, weight units streamed with the chunks; the
 // row statistics of the MVLayerNorm accumulate over the passes and the final scaling pass re-reads the product sum `o`
 // from the saved tensor (written by the same thread one pass earlier) instead of keeping it in TMEM.
-template <int DIM, bool ST, int TERMS = 3>
-__global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
+template <int DIM, bool ST, int TERMS, bool MET>
+__global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a, MetricArg<MET> mp) {
   using A = Alg<DIM>;
   constexpr int B = A::B, G = A::G, P = A::P, NI = n_images(TERMS);
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -591,15 +591,15 @@ __global__ void __launch_bounds__(kThreads, 1) tc_f2_kernel(FwdArgs a) {
           for (int b = 0; b < B; ++b) { xn[b] = xr[b][j]; oj[b] = o[b][j]; }
 #pragma unroll
           for (int b = 0; b < B; ++b) y2[b] = j == 0 ? y2v[b].x : j == 1 ? y2v[b].y : j == 2 ? y2v[b].z : y2v[b].w;
-          norm_factors<DIM>(xn, sn_s + ch * G, qv, nrm, rinv);
+          norm_factors<DIM, MET>(xn, sn_s + ch * G, qv, nrm, rinv, mp.qs);
 #pragma unroll
           for (int b = 0; b < B; ++b) xn[b] *= rinv[A::grade_of(b)];
           oj[0] += bl_s[ch];
-          A::template wgp<false>(y2, xn, wv_s + ch * P, nullptr, oj);
+          A::template wgp<MET>(y2, xn, wv_s + ch * P, mp.mf, oj);
           const bool ok = row_ok && ch < C;
 #pragma unroll
           for (int b = 0; b < B; ++b) oj[b] = ok ? oj[b] * kInvSqrt2 : 0.f;
-          if (ok) rs += fast_sas(mv_sumsq<DIM>(oj));
+          if (ok) rs += fast_sas(mv_q<DIM, MET>(oj, mp.qs));
 #pragma unroll
           for (int b = 0; b < B; ++b) o[b][j] = oj[b];
         }
@@ -755,9 +755,9 @@ int64_t fwd_ws_bytes(const csmpn_block_desc& d) {
   return (align32f(p.w1_floats) + align32f(p.w2_floats)) * 4;
 }
 
-// TERMS: numeric mode (csmpn_block_desc.tf32 = 1 -> 1, else 3)
-template <int DIM, int TERMS>
-int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
+// TERMS: numeric mode (csmpn_block_desc.tf32 = 1 -> 1, else 3); MET: non-Euclidean metric mp
+template <int DIM, int TERMS, bool MET>
+int launch_fwd(const csmpn_block_desc& d, MetricArg<MET> mp, cudaStream_t stream) {
   constexpr int B = Alg<DIM>::B;
   FwdArgs a;
   memset(&a, 0, sizeof(a));
@@ -806,30 +806,37 @@ int launch_fwd(const csmpn_block_desc& d, cudaStream_t stream) {
   const int grid = a.tiles < sm_count_cached() ? a.tiles : sm_count_cached();
   auto run = [&](auto kern, size_t smem_bytes) -> int {
     CSMPN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-    kern<<<grid, kThreads, smem_bytes, stream>>>(a);
+    kern<<<grid, kThreads, smem_bytes, stream>>>(a, mp);
     return CSMPN_OK;
   };
   if (mask & 1) {
     const bool overlap = !p.st1 && use_overlapped_epilogue(B, a.Cp);
-    int rc = overlap ? (a.in_bpt ? run(tc_f1db_kernel<DIM, true, TERMS>, p.s1) : run(tc_f1db_kernel<DIM, false, TERMS>, p.s1))
-             : a.in_bpt ? (p.st1 ? run(tc_f1_kernel<DIM, true, true, TERMS>, p.s1) : run(tc_f1_kernel<DIM, true, false, TERMS>, p.s1))
-                        : (p.st1 ? run(tc_f1_kernel<DIM, false, true, TERMS>, p.s1) : run(tc_f1_kernel<DIM, false, false, TERMS>, p.s1));
+    int rc = overlap ? (a.in_bpt ? run(tc_f1db_kernel<DIM, true, TERMS, MET>, p.s1) : run(tc_f1db_kernel<DIM, false, TERMS, MET>, p.s1))
+             : a.in_bpt ? (p.st1 ? run(tc_f1_kernel<DIM, true, true, TERMS, MET>, p.s1) : run(tc_f1_kernel<DIM, true, false, TERMS, MET>, p.s1))
+                        : (p.st1 ? run(tc_f1_kernel<DIM, false, true, TERMS, MET>, p.s1) : run(tc_f1_kernel<DIM, false, false, TERMS, MET>, p.s1));
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_f1_kernel");
   }
   if (mask & 2) {
-    int rc = p.st2 ? run(tc_f2_kernel<DIM, true, TERMS>, p.s2) : run(tc_f2_kernel<DIM, false, TERMS>, p.s2);
+    int rc = p.st2 ? run(tc_f2_kernel<DIM, true, TERMS, MET>, p.s2) : run(tc_f2_kernel<DIM, false, TERMS, MET>, p.s2);
     if (rc) return rc;
     CSMPN_LAUNCH_CHECK("tc_f2_kernel");
   }
   return CSMPN_OK;
 }
 
+template <int DIM, int TERMS>
+int launch_fwd_metric(const csmpn_block_desc& d, cudaStream_t stream) {
+  MetricParams mp;
+  if (block_metric(DIM, d, &mp)) return launch_fwd<DIM, TERMS, true>(d, mp, stream);
+  return launch_fwd<DIM, TERMS, false>(d, NoMetric{}, stream);
+}
+
 }  // namespace tcb
 
 int tc_block_fwd(int dim, const csmpn_block_desc* d, cudaStream_t stream) {
-  if (dim == 2) return d->tf32 ? tcb::launch_fwd<2, 1>(*d, stream) : tcb::launch_fwd<2, 3>(*d, stream);
-  if (dim == 3) return d->tf32 ? tcb::launch_fwd<3, 1>(*d, stream) : tcb::launch_fwd<3, 3>(*d, stream);
+  if (dim == 2) return d->tf32 ? tcb::launch_fwd_metric<2, 1>(*d, stream) : tcb::launch_fwd_metric<2, 3>(*d, stream);
+  if (dim == 3) return d->tf32 ? tcb::launch_fwd_metric<3, 1>(*d, stream) : tcb::launch_fwd_metric<3, 3>(*d, stream);
   return CSMPN_ERR_UNSUPPORTED;
 }
 int64_t tc_block_fwd_workspace(int dim, const csmpn_block_desc* d) {

@@ -11,8 +11,9 @@ Same class names, constructor signatures, parameter names / shapes / initialiser
   MVLayerNorm                     ATen launches
   SteerableGeometricProductLayer  sign/index-table weighted product; the [C,B,B,B] weight of
                                   cegnn_utils.py:126-140 is never built
-  CEMLP / EGCL                    fused block kernels (gather -> block -> ... -> CSR segment reduce) when the
-                                  algebra is Euclidean; composition of the unit kernels otherwise
+  CEMLP / EGCL                    fused block kernels (gather -> block -> ... -> CSR segment reduce) for every
+                                  non-degenerate metric of dimension 2, 3, 5 (fused.enabled); composition of the
+                                  unit kernels otherwise
 """
 from __future__ import annotations
 

@@ -6,9 +6,10 @@ One autograd node per CEMLP block.  The EGCL layer becomes
     block(concat: h | agg | node_attr)        ->  block(dense, + residual)
 
 with every per-pair tensor kept in receiver-sorted order so the reduce reads contiguous rows and is
-deterministic.  Enabled for Euclidean algebras of dimension 2, 3 and 5 (the reference's models); other
-algebras use the unit kernels.  ``CSMPN_FUSED=0`` forces the unit-kernel composition (used by tests to
-cross-check the two paths).
+deterministic.  Enabled for every non-degenerate diagonal metric (Euclidean, Cl(p,q), rescaled) of dimension 2, 3
+and 5; the descriptors carry the algebra's metric and the kernels fold it into their elementwise stages.  Degenerate
+metrics and other dimensions use the unit kernels.  ``CSMPN_FUSED=0`` forces the unit-kernel composition (used by
+tests to cross-check the two paths).
 """
 from __future__ import annotations
 
@@ -38,6 +39,7 @@ class BlockDesc(ctypes.Structure):
         ("vt_k", c_int32), ("vt_fp", c_int32),
         ("fwd_ws", c_void_p), ("fwd_ws_bytes", c_int64),
         ("tf32", c_int32),
+        ("metric", c_void_p),
     ]
 
 
@@ -111,9 +113,12 @@ def available() -> bool:
 
 
 def enabled(algebra) -> bool:
+    """The fused block engines take the algebra's CEMLPs and EGCLs: dimension in FUSED_DIMS and a non-degenerate metric.
+    A zero entry (e.g. PGA Cl(3,0,1)) changes the grade-path set of the weighted product (cegnn_utils._euclid_path_cols),
+    which the fused backward does not remap."""
     if os.environ.get("CSMPN_FUSED", "1") == "0":
         return False
-    return bool(getattr(algebra, "is_euclidean", False)) and algebra.dim in FUSED_DIMS
+    return algebra.dim in FUSED_DIMS and all(m != 0.0 for m in algebra._metric_list)
 
 
 def _block_supported(layer) -> bool:
@@ -130,7 +135,19 @@ def _block_supported(layer) -> bool:
     # wide blocks whose weights leave room for fewer than 4 rows per shared-memory tile of the SIMT engine run on the
     # tensor-core engine with streamed weights (csmpn_block_tc_plan); what neither engine takes is composed from unit kernels
     dim = lin.algebra.dim
-    return _fits_fused(dim, lin.in_features, lin.out_features) or (dim in (2, 3) and tc_supported(dim, lin.in_features, lin.out_features))
+    return _fits_fused(dim, lin.in_features, lin.out_features) or (
+        dim in (2, 3) and tc_metric(lin.algebra) and tc_supported(dim, lin.in_features, lin.out_features))
+
+
+def tc_metric(algebra) -> bool:
+    """The tensor-core engine takes the algebra's blocks: every metric entry is positive (Euclidean or rescaled), so every
+    quadratic form of the block is positive definite.  With a negative entry the forms are indefinite: they cancel towards
+    0 where the normalisation and MVLayerNorm derivatives ~ q / (q^2 + eps)^(3/4) are steepest, and the engine's
+    approximate SFU reciprocals / square roots and split-TF32 products then leave gradient errors 3-9x (worst 1.4, Cl(2,1)
+    EGCL at 4 164 simplices) above the fp32 oracle's own error against fp64, where the FP32 SIMT engine and the unit kernels
+    stay within it (B200 measurement, DESIGN.md 4.5).  Such blocks run on the FP32 SIMT engine, or on unit kernels when it
+    cannot hold them, in either precision mode."""
+    return all(m > 0.0 for m in algebra._metric_list)
 
 
 _FITS: dict = {}
@@ -180,9 +197,12 @@ def sorted_graph(g: ops.CSRGraph) -> SortedGraph:
     return sg
 
 
-def _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, res, saves, pair_attr=False):
+def _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, res, saves, pair_attr=False, metric=None):
+    """metric: the algebra's host metric array (CliffordAlgebra._metric_c); None = Euclidean.  The descriptor holds its
+    address, so the caller keeps the array alive while the descriptor is in use."""
     w1, b1, sa, sb, wr, na, wl, bl, wp, la = params
     d = BlockDesc()
+    d.metric = None if metric is None else ctypes.addressof(metric)
     d.pair_attr = int(bool(pair_attr))
     d.mode, d.c0, d.c1, d.c2, d.c = mode, chans[0], chans[1], chans[2], c
     d.has_b1 = int(b1 is not None)
@@ -225,14 +245,15 @@ class FusedBlockFn(torch.autograd.Function):
         need_grad = cfg["need_grad"]
         saves = tuple(torch.empty((rows, c, B), dtype=torch.float32, device=dev) for _ in range(3)) if need_grad else None
         resc = None if res is None else f32c(res)
-        d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, resc, saves, pair)
+        d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, resc, saves, pair, cfg.get("metric"))
         check(lib().csmpn_block_fwd(dim, ctypes.byref(d), stream_ptr(dev)), "block_fwd")
-        _record("fwd", dim, d, keep=[srcs, params, y, resc, saves])
+        _record("fwd", dim, d, keep=[srcs, params, y, resc, saves, cfg.get("metric")])
         if need_grad:
             ctx.save_for_backward(*[t for t in srcs if t is not None], *[t for t in params if t is not None], *saves)
             ctx.meta = (dim, mode, sgraph, chans, c, rows, [t is not None for t in srcs], [t is not None for t in params],
                         res is not None, [None if t is None else t.shape for t in (w1, b1, sa, sb, wr, na, wl, bl, wp, la)],
                         [None if t is None else t.shape for t in (p0, p1, p2)], pair)
+            ctx.metric = cfg.get("metric")
         return y
 
     @staticmethod
@@ -247,7 +268,7 @@ class FusedBlockFn(torch.autograd.Function):
         B = 1 << dim
         cin = sum(chans)
         y_dummy = gy  # desc.y is not written by the backward
-        d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y_dummy, None, saves, pair)
+        d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y_dummy, None, saves, pair, ctx.metric)
         gx = torch.empty((rows, cin, B), dtype=torch.float32, device=dev)
         pg = [None if t is None else torch.empty_like(t) for t in params]
         g = BlockGrads()
@@ -260,7 +281,7 @@ class FusedBlockFn(torch.autograd.Function):
             raise _lib.CsmpnError("fused block backward: unsupported configuration")
         ws = workspace(nbytes, dev)
         check(lib().csmpn_block_bwd(dim, ctypes.byref(d), ctypes.byref(g), ptr(ws), ws.numel(), stream_ptr(dev)), "block_bwd")
-        _record("bwd", dim, d, g, ws, keep=[srcs, params, saves, gy, gx, pg])
+        _record("bwd", dim, d, g, ws, keep=[srcs, params, saves, gy, gx, pg, ctx.metric])
         # split the gradient of the assembled input row back onto the sources
         gsrc = [None, None, None]
         if mode == 0:
@@ -341,7 +362,7 @@ class TcBlockFn(torch.autograd.Function):
         saves = tuple(bpt_empty(dim, rows, c, dev) for _ in range(3)) if need_grad else None
         x0 = bpt_empty(dim, rows, cin, dev) if (need_grad and not in_bpt) else None
         resc = None if res is None else f32c(res)
-        d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, resc, saves, pair)
+        d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, y, resc, saves, pair, cfg.get("metric"))
         d.engine, d.in_bpt, d.out_bpt = 1, int(in_bpt), int(out_bpt)
         d.tf32 = ctx.tf32 = int(tc_precision())
         d.save_y2 = y2.data_ptr()
@@ -359,7 +380,7 @@ class TcBlockFn(torch.autograd.Function):
                 scratch_o = bpt_empty(dim, rows, c, dev)
                 d.save_o = scratch_o.data_ptr()
         check(lib().csmpn_block_fwd(dim, ctypes.byref(d), stream_ptr(dev)), "block_fwd (tensor-core)")
-        _record("fwd", dim, d, keep=[srcs, params, y, resc, saves, y2, x0, wsf, scratch_o])
+        _record("fwd", dim, d, keep=[srcs, params, y, resc, saves, y2, x0, wsf, scratch_o, cfg.get("metric")])
         red = cfg.get("reduce")   # (SortedGraph, mean): return the per-receiver aggregate of the rows instead of the rows
         if red is not None:
             csr = red[0].csr
@@ -376,6 +397,7 @@ class TcBlockFn(torch.autograd.Function):
             ctx.meta = (dim, mode, sgraph, chans, c, rows, [t is not None for t in srcs], [t is not None for t in params],
                         res is not None, [None if t is None else t.shape for t in (w1, b1, sa, sb, wr, na, wl, bl, wp, la)],
                         [None if t is None else t.shape for t in (p0, p1, p2)], in_bpt, out_bpt, x0 is not None, pair, vt)
+            ctx.metric = cfg.get("metric")
         return y
 
     @staticmethod
@@ -409,7 +431,7 @@ def _tc_block_backward(ctx, gy):
         gy = f32c(gy)
     dev = gy.device
     cin = sum(chans)
-    d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, gy, None, (y1, xr, o), pair)
+    d = _fill_desc(dim, mode, srcs, chans, rows, c, params, sgraph, gy, None, (y1, xr, o), pair, ctx.metric)
     d.engine, d.in_bpt, d.out_bpt = 1, int(in_bpt), int(out_bpt)
     d.tf32 = ctx.tf32  # the mode of the forward
     d.save_y2 = y2.data_ptr()
@@ -434,7 +456,7 @@ def _tc_block_backward(ctx, gy):
     if nbytes < 0:
         raise _lib.CsmpnError("tensor-core block backward: unsupported configuration")
     ws = workspace(nbytes, dev)
-    _record("bwd", dim, d, g, ws, keep=[srcs, params, y1, xr, o, y2, x0, gy, gx, pg])
+    _record("bwd", dim, d, g, ws, keep=[srcs, params, y1, xr, o, y2, x0, gy, gx, pg, ctx.metric])
     if _fork_enabled():
         _tc_backward_forked(dim, d, g, ws, dev)
     else:
@@ -573,7 +595,7 @@ def tc_min_rows() -> int:
 
 def _block_uses_tc(algebra, layer, need_grad, rows=None) -> bool:
     lin = layer[0]
-    if algebra.dim not in (2, 3):
+    if algebra.dim not in (2, 3) or not tc_metric(algebra):
         return False
     if not tc_supported(algebra.dim, lin.in_features, lin.out_features):
         return False
@@ -597,7 +619,8 @@ def block_forward(algebra, layer, x, p1=None, p2=None, res=None, mode=0, sgraph=
         return y if res is None else res + y
     params = _block_params(layer)
     need_grad = _need_grad(x, p1, p2, res, *params)
-    cfg = {"dim": algebra.dim, "mode": mode, "sgraph": sgraph, "need_grad": need_grad, "pair_attr": pair_attr}
+    cfg = {"dim": algebra.dim, "mode": mode, "sgraph": sgraph, "need_grad": need_grad, "pair_attr": pair_attr,
+           "metric": algebra._metric_c}
     rows_now = bpt_rows if in_bpt else (sgraph.csr.n_pairs if mode == 1 else x.shape[0])
     if in_bpt or _block_uses_tc(algebra, layer, need_grad, rows_now):
         cfg.update(in_bpt=in_bpt, out_bpt=out_bpt, rows=bpt_rows, c_in=layer[0].in_features)
@@ -627,7 +650,7 @@ def embed_rows_forward(algebra, blocks, table, vertex_rows, fp):
     if (not all(_block_supported(b) for b in blocks) or lin.in_features != table.shape[1] * k or table.requires_grad
             or not _chain_uses_tc(algebra, blocks, need_grad, rows)):
         return None
-    cfg = {"dim": algebra.dim, "mode": 2, "sgraph": None, "need_grad": need_grad, "pair_attr": False,
+    cfg = {"dim": algebra.dim, "mode": 2, "sgraph": None, "need_grad": need_grad, "pair_attr": False, "metric": algebra._metric_c,
            "vertex_table": (vertex_rows.contiguous(), int(fp)), "in_bpt": False, "out_bpt": len(blocks) > 1, "rows": None,
            "c_in": lin.in_features}
     u = TcBlockFn.apply(cfg, f32c(table), None, None, None, *_block_params(blocks[0]))

@@ -33,7 +33,7 @@ enum csmpn_status {
   CSMPN_OK = 0,
   CSMPN_ERR_BAD_DIM = -1,       /* dim outside 1..5 */
   CSMPN_ERR_BAD_ARG = -2,       /* null pointer / negative size / inconsistent sizes */
-  CSMPN_ERR_UNSUPPORTED = -3,   /* configuration not built (e.g. fused path with a non-Euclidean metric) */
+  CSMPN_ERR_UNSUPPORTED = -3,   /* configuration not built (e.g. fused path with a degenerate metric) */
   CSMPN_ERR_CUDA = -4,          /* a CUDA runtime call failed; see csmpn_last_cuda_error() */
   CSMPN_ERR_WORKSPACE = -5      /* workspace too small */
 };
@@ -152,7 +152,8 @@ int csmpn_segment_expand(const float* grad_out, const int64_t* dst, const int32_
 /* ---- fused CEMLP block  (one [MVLinear, MVSiLU, SteerableGeometricProductLayer, MVLayerNorm] block of CEMLP,
  *      cegnn_utils.py:180-207; with the gather of EGCL.message :254-262 or the concat of EGCL.update :264-275
  *      folded into its prologue and the residual of :272-273 into its epilogue) --------------------------------
- * Euclidean metrics, dim in {2,3,5}.  Rows are processed in tiles held in shared memory; the three per-grade
+ * Non-degenerate diagonal metrics (`metric`: every entry nonzero, e.g. Cl(p,q) or a rescaled Euclidean metric), dim
+ * in {2,3,5} on engine 0 and {2,3} on engine 1.  Rows are processed in tiles held in shared memory; the three per-grade
  * channel GEMMs, the gates, norms and the weighted geometric product of a block never leave the SM.
  *
  * Input row r (c_in = c0 + c1 + c2 channels):
@@ -216,6 +217,12 @@ typedef struct csmpn_block_desc {
                                            images (csmpn_block_fwd_workspace / csmpn_block_bwd_workspace).  Engine 0
                                            ignores it; any other value is CSMPN_ERR_BAD_ARG.  The backward of a block must
                                            be called with the value of its forward. */
+  const float* metric;                  /* HOST array of `dim` floats read at launch (as the `metric` argument of the unit
+                                           entry points), or NULL; NULL or all ones = Euclidean.  A zero entry (degenerate
+                                           metric) is CSMPN_ERR_UNSUPPORTED: compose such blocks from the unit kernels.
+                                           The metric folds into the elementwise stages only (quadratic forms of MVSiLU,
+                                           the normalisation and MVLayerNorm, and the weighted geometric product); a CUDA
+                                           graph keeps the metric of its capture. */
 } csmpn_block_desc;
 
 /* gradients produced by csmpn_block_bwd (all overwritten; parameter gradients reduced deterministically) */
