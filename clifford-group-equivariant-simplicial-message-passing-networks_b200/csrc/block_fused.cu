@@ -933,40 +933,6 @@ __global__ void __launch_bounds__(256, 1) block_bwd_kernel(csmpn_block_desc d, c
   }
 }
 
-// ---------------------------------------------------------------------------------------------------
-// final fixed-order reduction of the per-CTA partials into the parameter gradients: 16 consecutive elements per CTA x
-// 16 partial groups.  Thread (e, pg) sums partials pg, pg+16, ... in order (all loads independent, 64 contiguous bytes
-// per partial row), then the 16 group sums are combined in a fixed order: bit-reproducible run to run.
-struct FinalSeg { const float* in; float* out; int n; int parts; int64_t stride; };
-struct FinalSegs { FinalSeg s[10]; int count; int total; };
-
-__global__ void __launch_bounds__(256) block_bwd_final_kernel(FinalSegs segs) {
-  __shared__ float red[16][17];
-  const int e = threadIdx.x & 15, pg = threadIdx.x >> 4;
-  int q = (int)blockIdx.x * 16 + e;
-  float s = 0.f;
-  float* outp = nullptr;
-  if (q < segs.total) {
-    int k = 0;
-    while (k < segs.count - 1 && q >= segs.s[k].n) { q -= segs.s[k].n; ++k; }
-    const FinalSeg& sg = segs.s[k];
-    if (sg.out != nullptr && q < sg.n) {
-      const float* in = sg.in + q;
-#pragma unroll 4
-      for (int pidx = pg; pidx < sg.parts; pidx += 16) s += in[(size_t)pidx * sg.stride];
-      outp = sg.out + q;
-    }
-  }
-  red[pg][e] = s;
-  __syncthreads();
-  if (pg == 0 && outp) {
-    float t = 0.f;
-#pragma unroll
-    for (int i = 0; i < 16; ++i) t += red[i][e];
-    *outp = t;
-  }
-}
-
 template <int DIM, bool MET>
 int run_block_fwd(const csmpn_block_desc& d, const FusedPlan& p, MetricArg<MET> mp, cudaStream_t s) {
   static bool attr_set = false;
@@ -1033,11 +999,13 @@ int launch_block_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void
   MetricParams mp;
   st = block_metric(DIM, d, &mp) ? run_block_bwd<DIM, true>(d, g, p, ws, mp, s) : run_block_bwd<DIM, false>(d, g, p, ws, NoMetric{}, s);
   if (st) return st;
+  // fixed-order sum of the per-CTA partials into the parameter gradients (one launch: 10 jobs)
   const int small_words = c * (P + 3 * G + 3);
-  FinalSegs fs;
+  FinalJob jobs[10];
+  memset(jobs, 0, sizeof(jobs));
   int k = 0;
   auto add = [&](const float* in, float* out, int n, int parts, int64_t stride) {
-    fs.s[k].in = in; fs.s[k].out = out; fs.s[k].n = n; fs.s[k].parts = parts; fs.s[k].stride = stride; ++k;
+    jobs[k].in = in; jobs[k].out = out; jobs[k].n = n; jobs[k].parts = parts; jobs[k].stride = stride; ++k;  // kind 0
   };
   add(ws.dw1, g.g_w1, c * cin * G, (int)slots, (int64_t)c * cin * G);
   add(ws.dwr, g.g_wr, c * c * G, (int)slots, (int64_t)c * c * G);
@@ -1050,12 +1018,7 @@ int launch_block_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void
   add(sm, g.g_la, c, p.grid, small_words); sm += c;
   add(sm, d.has_b1 ? g.g_b1 : nullptr, c, p.grid, small_words); sm += c;
   add(sm, g.g_bl, c, p.grid, small_words);
-  fs.count = k;
-  fs.total = 0;
-  for (int i = 0; i < k; ++i) fs.total += fs.s[i].n;
-  block_bwd_final_kernel<<<(unsigned)((fs.total + 15) / 16), 256, 0, s>>>(fs);
-  CSMPN_LAUNCH_CHECK("block_bwd_final");
-  return CSMPN_OK;
+  return launch_final_reduce(jobs, k, s);
 }
 
 inline int check_desc(int dim, const csmpn_block_desc* d) {

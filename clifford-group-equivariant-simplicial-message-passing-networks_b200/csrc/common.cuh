@@ -176,6 +176,23 @@ __device__ __forceinline__ void grade_q(const float* x, const float* qs, float* 
   for (int i = 0; i < A::B; ++i) q[A::grade_of(i)] = fmaf(qs[i] * x[i], x[i], q[A::grade_of(i)]);
 }
 
+// ---------------------------------------------------------------- fixed-order reduction of per-CTA partials
+// One job of final_reduce_kernel (tc_block_bwd.cu), the last kernel of both block engines' backward; a job with out =
+// NULL is skipped (a gradient the caller does not want).
+struct FinalJob {
+  const float* in;   // partials
+  float* out;
+  int parts;         // number of partials
+  int64_t stride;    // floats between partials
+  int kind;          // 0: out[i] = sum in[p][i] (n = count);  1: weight gradient from [G][M][N] partials
+  int n;             // kind 0: element count; kind 1: c_out * c_in * G
+  int G, M, N, m0, co, ci;  // kind 1: out[((o0 + o)*ci_tot + i0 + i)*G + g] = sum_p in[p][(g*M + m0 + o)*N + i], i < ci
+  int ci_tot, i0, o0;
+};
+
+// final_reduce_kernel over jobs[0, count), split into launches of at most kFinalJobs jobs each
+int launch_final_reduce(const FinalJob* jobs, size_t count, cudaStream_t stream);
+
 inline int sm_count_cached() {
   static int n = 0;
   if (n == 0) {

@@ -11,7 +11,8 @@
 //   tc_bgemm      (tensor pipe) grad_x = dy1 * W1                                    (BPT or reference layout)
 //   tc_dw_kernel  (tensor pipe) weight gradients [d | dxr]^T y2 and dy1^T x0: MN-major TF32 operands, K = rows,
 //                               accumulated over blades of a grade and over all tiles of a CTA in TMEM
-//   tc_final_kernel             fixed-order sum of the per-CTA partials -> reference parameter layouts
+//   final_reduce_kernel         fixed-order sum of the per-CTA partials -> reference parameter layouts (also the last
+//                               kernel of the FP32 SIMT engine's backward, block_fused.cu)
 //
 // The elementwise kernels keep one channel per thread for the whole kernel (warp = 4 channels x 8 rows), so every
 // per-channel parameter gradient is a register accumulator and every BPT access of a warp is one 128-byte line.
@@ -21,6 +22,67 @@
 #include "tc_block.cuh"
 
 namespace csmpn {
+
+// =====================================================================================================================
+// fixed-order reduction of per-CTA partials (both block engines)
+constexpr int kFinalJobs = 14;
+struct FinalJobs { FinalJob j[kFinalJobs]; int count; };
+
+// 16 consecutive elements per CTA x 16 partial groups: thread (e, pg) sums partials pg, pg+16, ... in order (independent
+// loads, 64 contiguous bytes per partial row), then the 16 group sums are combined in a fixed order (bit-reproducible).
+// Elements are enumerated in SOURCE order (i fastest).
+__global__ void __launch_bounds__(256) final_reduce_kernel(FinalJobs jobs) {
+  __shared__ float red[16][17];
+  const int e = threadIdx.x & 15, pg = threadIdx.x >> 4;
+  int64_t idx = (int64_t)blockIdx.x * 16 + e;
+  float s = 0.f;
+  float* outp = nullptr;
+  for (int k = 0; k < jobs.count; ++k) {
+    const FinalJob& jb = jobs.j[k];
+    if (idx < jb.n) {
+      if (jb.out) {
+        size_t src, dst;
+        if (jb.kind == 0) {
+          src = dst = (size_t)idx;
+        } else {
+          const int i = (int)(idx % jb.ci), o = (int)((idx / jb.ci) % jb.co), g = (int)(idx / ((int64_t)jb.ci * jb.co));
+          src = ((size_t)g * jb.M + jb.m0 + o) * jb.N + i;
+          dst = ((size_t)(jb.o0 + o) * jb.ci_tot + jb.i0 + i) * jb.G + g;
+        }
+        const float* in = jb.in + src;
+#pragma unroll 4
+        for (int p = pg; p < jb.parts; p += 16) s += in[(size_t)p * jb.stride];
+        outp = jb.out + dst;
+      }
+      break;
+    }
+    idx -= jb.n;
+  }
+  red[pg][e] = s;
+  __syncthreads();
+  if (pg == 0 && outp) {
+    float t = 0.f;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) t += red[i][e];
+    *outp = t;
+  }
+}
+
+int launch_final_reduce(const FinalJob* jobs, size_t count, cudaStream_t stream) {
+  for (size_t j0 = 0; j0 < count; j0 += kFinalJobs) {  // wide blocks have more jobs than one launch takes
+    FinalJobs fj;
+    memset(&fj, 0, sizeof(fj));
+    int64_t total = 0;
+    for (size_t k = j0; k < count && k < j0 + kFinalJobs; ++k) {
+      fj.j[fj.count++] = jobs[k];
+      total += jobs[k].n;
+    }
+    final_reduce_kernel<<<(unsigned)((total + 15) / 16), 256, 0, stream>>>(fj);
+    CSMPN_LAUNCH_CHECK("final_reduce_kernel");
+  }
+  return CSMPN_OK;
+}
+
 namespace tcb {
 
 // =====================================================================================================================
@@ -799,61 +861,6 @@ __global__ void __launch_bounds__(256, 1) tc_dw_kernel(DwArgs a) {
 }
 
 // =====================================================================================================================
-// fixed-order reduction of per-CTA partials
-struct FinalJob {
-  const float* in;   // partials
-  float* out;
-  int parts;         // number of partials
-  int64_t stride;    // floats between partials
-  int kind;          // 0: out[i] = sum in[p][i] (n = count);  1: weight gradient from [G][M][N] partials
-  int n;             // kind 0: element count; kind 1: c_out * c_in * G
-  int G, M, N, m0, co, ci;  // kind 1: out[((o0 + o)*ci_tot + i0 + i)*G + g] = sum_p in[p][(g*M + m0 + o)*N + i], i < ci
-  int ci_tot, i0, o0;
-};
-constexpr int kFinalJobs = 14;
-struct FinalJobs { FinalJob j[kFinalJobs]; int count; };
-
-// 16 consecutive elements per CTA x 16 partial groups: thread (e, pg) sums partials pg, pg+16, ... in order (independent
-// loads, 64 contiguous bytes per partial row), then the 16 group sums are combined in a fixed order (bit-reproducible).
-// Elements are enumerated in SOURCE order (i fastest).
-__global__ void __launch_bounds__(256) tc_final_kernel(FinalJobs jobs) {
-  __shared__ float red[16][17];
-  const int e = threadIdx.x & 15, pg = threadIdx.x >> 4;
-  int64_t idx = (int64_t)blockIdx.x * 16 + e;
-  float s = 0.f;
-  float* outp = nullptr;
-  for (int k = 0; k < jobs.count; ++k) {
-    const FinalJob& jb = jobs.j[k];
-    if (idx < jb.n) {
-      if (jb.out) {
-        size_t src, dst;
-        if (jb.kind == 0) {
-          src = dst = (size_t)idx;
-        } else {
-          const int i = (int)(idx % jb.ci), o = (int)((idx / jb.ci) % jb.co), g = (int)(idx / ((int64_t)jb.ci * jb.co));
-          src = ((size_t)g * jb.M + jb.m0 + o) * jb.N + i;
-          dst = ((size_t)(jb.o0 + o) * jb.ci_tot + jb.i0 + i) * jb.G + g;
-        }
-        const float* in = jb.in + src;
-#pragma unroll 4
-        for (int p = pg; p < jb.parts; p += 16) s += in[(size_t)p * jb.stride];
-        outp = jb.out + dst;
-      }
-      break;
-    }
-    idx -= jb.n;
-  }
-  red[pg][e] = s;
-  __syncthreads();
-  if (pg == 0 && outp) {
-    float t = 0.f;
-#pragma unroll
-    for (int i = 0; i < 16; ++i) t += red[i][e];
-    *outp = t;
-  }
-}
-
-// =====================================================================================================================
 // host side
 template <int DIM>
 size_t gemm_smem(int nsets, int n16, int kmax, int nimg = 2) {
@@ -1181,19 +1188,7 @@ int launch_bwd(const csmpn_block_desc& d, const csmpn_block_grads& g, void* work
   cjob(ws + p.o_p3, g.g_sa, p.grid_ew, NP3, 0, G);
   cjob(ws + p.o_p3, g.g_sb, p.grid_ew, NP3, G, G);
   cjob(ws + p.o_p3, d.has_b1 ? g.g_b1 : nullptr, p.grid_ew, NP3, 2 * G, 1);
-  if (mask & 64) {
-    for (size_t j0 = 0; j0 < jobs.size(); j0 += kFinalJobs) {  // wide blocks have more jobs than one launch takes
-      FinalJobs fj;
-      memset(&fj, 0, sizeof(fj));
-      int64_t total = 0;
-      for (size_t k = j0; k < jobs.size() && k < j0 + kFinalJobs; ++k) {
-        fj.j[fj.count++] = jobs[k];
-        total += jobs[k].n;
-      }
-      tc_final_kernel<<<(unsigned)((total + 15) / 16), 256, 0, stream>>>(fj);
-      CSMPN_LAUNCH_CHECK("tc_final_kernel");
-    }
-  }
+  if (mask & 64) return launch_final_reduce(jobs.data(), jobs.size(), stream);
   return CSMPN_OK;
 }
 

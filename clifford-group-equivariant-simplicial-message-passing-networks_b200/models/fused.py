@@ -755,7 +755,7 @@ def _kernel_stages(d: BlockDesc, g, B: int):
             ("tc_bgemm", "grad_x = dy1 W1", 8, T + gx, k * rows * 2 * B * C * cin),
             ("tc_dw", "dWL, dWR = [d|dxr]^T y2", 16, 3 * T, k * rows * 4 * B * C * C),
             ("tc_dw", "dW1 = dy1^T x0", 32, T + Tin, k * rows * 2 * B * C * cin),
-            ("tc_final", "fixed-order reduction of per-CTA partials", 64, 0, 0)]
+            ("final_reduce (both engines)", "fixed-order reduction of per-CTA partials", 64, 0, 0)]
 
 
 def bench_layer_kernels(layer, d, graph, hbm_peak, peak_src, traffic=None, iters=8):

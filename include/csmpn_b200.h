@@ -256,7 +256,7 @@ int csmpn_block_tc_plan(int dim, int c_in, int c);
  * backward GEMMs of the wide plan (np; 0 for the resident backward); 0 if engine 1 does not handle the shape */
 int csmpn_block_tc_passes(int dim, int c_in, int c);
 /* > 0 (the rows per shared-memory tile) if engine 0 keeps the block's weights resident in shared memory (forward and
- * backward), 0 if it would stage them per GEMM; with fewer than 8 rows per tile or staged weights the unit kernels
+ * backward), 0 if it would stage them per GEMM; with fewer than 4 rows per tile or staged weights the unit kernels
  * (csmpn_mvlinear_*, csmpn_mvsilu_*, csmpn_wgp_*, ...) composed by the host are the faster path for that shape */
 int csmpn_block_simt_resident(int dim, int c_in, int c);
 /* number of floats of a BPT tensor with `rows` rows and `channels` channels (padded to a multiple of 16) */

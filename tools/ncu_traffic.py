@@ -16,7 +16,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CLASSES = (("tc_f1", "tc_f1"), ("tc_f2", "tc_f2"), ("tc_b1", "tc_b1"), ("tc_bgemm", "tc_bgemm"),
-           ("tc_b3", "tc_b3"), ("tc_dw", "tc_dw"), ("tc_final", "tc_final"), ("tc_weight_images", "tc_weight_images"),
+           ("tc_b3", "tc_b3"), ("tc_dw", "tc_dw"), ("final_reduce", "final_reduce (both engines)"), ("tc_weight_images", "tc_weight_images"),
            ("block_fwd_kernel", "block_fwd (fp32 simt)"), ("block_bwd", "block_bwd (fp32 simt)"), ("segment_", "segment reduce / expand"),
            ("scatter_", "scatter (grad_h, table grads)"), ("add3_rows", "add3_rows"))
 
